@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the wav2sleep forward hot path on B200 (BASELINE.json metric: recording-hours/sec, forward).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]                    # this repo's CUDA path
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path
     python bench.py --impl reference [--steps K] [--warmup W]              # reference algorithm on host CPU cores
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N   # N > 1, one rank per GPU
 
@@ -144,6 +144,16 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: the tensors the timed path handed back in its last step, as <out_dir>/<name>.npy (float32), so
+    that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output."""
+    import numpy as np
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(d / f"{name}.npy", t.detach().to("cpu", torch.float32).numpy())
+
+
 def collect_profile(lib):
     n = lib.w2s_profile_count()
     recs = []
@@ -239,6 +249,8 @@ def run_cuda(args):
         barrier()
         launches = lib.w2s_launch_count() - l0 + model._get_engine().replayed_launches
         ms_dev = max_over_ranks(e0.elapsed_time(e1))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"predictions" if world == 1 else f"predictions_rank{rank}": pred})
 
         # ---------------- end-to-end timing: pinned host inputs -> predictions on host ----------------
         copy_stream = torch.cuda.Stream(device=dev)
@@ -587,7 +599,14 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the secondary train-step timings")
     ap.add_argument("--no-eog", action="store_true", help="skip the secondary EOG-model timing (BASELINE configs[1])")
     ap.add_argument("--kernels-out", default=None, help="also write the full per-kernel profile (JSON list) to this file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the int64 [16, 1200] predictions of the last timed step (as float32) to DIR/predictions.npy"
+                         " (DIR/predictions_rank<r>.npy for N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs applies to the CUDA path only")
     args.warmup = max(args.warmup, 3) if args.impl == "cuda" else max(args.warmup, 1)
     if args.impl == "reference":
         run_reference(args)
