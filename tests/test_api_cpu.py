@@ -141,7 +141,6 @@ def test_encoder_pairing_rules():
     assert groups(stub(smap, descs, 1), names, xs, True) == [("ECG", "PPG"), ("ABD", "THX")]
     assert groups(stub(smap, descs, 0), names, xs, True) == [("ECG",), ("PPG",), ("ABD",), ("THX",)]
     assert groups(stub(smap, descs, 1), names, xs, False) == [("ECG",), ("PPG",), ("ABD",), ("THX",)]
-    assert groups(stub(smap, descs, 3), names, xs, True) == [("ECG",), ("PPG",), ("ABD", "THX")]
     # a different architecture (wide storage) or input length is never paired
     odd = dict(descs, PPG=desc(hi, wide=2))
     assert groups(stub(smap, odd, 1), names, xs, True) == [("ECG",), ("PPG",), ("ABD", "THX")]

@@ -347,14 +347,14 @@ def test_fp32_check_mode_on_full_nights(cuda_device):
 
 
 def test_predict_async_lanes_match_predict(cuda_device):
-    """Throughput API: several batches in flight on alternating lanes give exactly the predictions of the blocking call,
-    in order, also when the lane buffers are re-used and when the shape changes in between."""
+    """Throughput API: several batches in flight give exactly the predictions of the blocking call, in order, also when
+    the engine's asynchronous buffers are re-used and when the shape changes in between."""
     model = build_default(CARDIO, 4, seed=0).to(cuda_device).eval()
     batches = [{k: v.to(cuda_device) for k, v in make_inputs(CARDIO, 3, 16, seed=s).items()} for s in range(5)]
     batches[3]["THX"][1] = float("-inf")
     with torch.inference_mode():
         ref = [model.predict(b).clone() for b in batches]
-        pend = [model.predict_async(b) for b in batches]           # 5 batches over 2 lanes: buffers re-used
+        pend = [model.predict_async(b) for b in batches]           # 5 batches on one set of buffers: re-used
         other = model.predict_async({k: v[:, : v.size(1) // 2] for k, v in batches[0].items()})  # new shape
         outs = [p.wait() for p in pend]
         half = other.wait()

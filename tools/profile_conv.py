@@ -86,9 +86,9 @@ if int(os.environ.get("W2S_DEBUG_FLAGS", "0")) & 64:
     names = ["entry", "tmem_alloc", "setup_done", "xform_start", "xform_raw_ready", "xform_first_done", "epi_first_full",
              "epi_loop_done", "epi_flushed", "teardown_sync"]
     tot = max(buf[15], 1)
-    print("blocked in mbarrier waits (%% of the CTA's %d cycles): producer(raw_empty) %.0f%%, MMA(a_full+t_empty) %.0f%%, "
+    print("blocked in mbarrier waits (%% of the CTA's %d cycles): MMA(t_empty) %.0f%%, "
           "epilogue(t_full) %.0f%%, transform: raw_full %.0f%% + a_empty %.0f%%"
-          % (tot, 100 * buf[11] / tot, 100 * buf[12] / tot, 100 * buf[13] / tot, 100 * buf[10] / tot, 100 * buf[14] / tot))
+          % (tot, 100 * buf[12] / tot, 100 * buf[13] / tot, 100 * buf[10] / tot, 100 * buf[14] / tot))
     base = buf[0]
     print("event-timed %.1f us; CTA0 milestones (us since entry): " % (t0.elapsed_time(t1) * 1e3)
           + ", ".join(f"{n}={(buf[i] - base) / 1e3:.1f}" for i, n in enumerate(names)))

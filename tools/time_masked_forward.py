@@ -1,7 +1,7 @@
 """Forward time of the cardio model when signals are missing on some nights (rows of -inf, data/dataset.py:170-173):
-16 synthetic 10-h nights, PPG missing on 12 of them, THX on 8.  Compares the launch policies through the environment:
-W2S_ENC_PAIRS=0 (one launch chain per signal), W2S_LIB_VARIANT=equal (paired, grid split in halves), default (paired,
-grid split in proportion to the live samples of the two encoders)."""
+16 synthetic 10-h nights, PPG missing on 12 of them, THX on 8.  Compares the engine's launch policies, set through
+its ``enc_pairs`` attribute: 0 (one launch chain per signal) against the default 1 (paired launches, the grid split
+in proportion to the live samples of the two encoders)."""
 import sys
 from pathlib import Path
 
@@ -20,19 +20,29 @@ for seed in (42, 43):
     x["PPG"][:12] = float("-inf")
     x["THX"][:8] = float("-inf")
     xs.append(x)
-with torch.inference_mode():
-    for i in range(4):
-        model.predict(xs[i % 2])
-    torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    pend = []
-    for i in range(30):
-        pend.append(model.predict_async(xs[i % 2]))
-        if len(pend) > 1:
-            pend.pop(0).wait()
-    for q in pend:
-        q.wait()
-    e1.record()
-    torch.cuda.synchronize()
-print(f"masked forward (PPG 4/16, THX 8/16 nights live): {e0.elapsed_time(e1) / 30:.3f} ms/step")
+eng = model._get_engine()
+
+
+def time_forward(enc_pairs):
+    eng.enc_pairs = enc_pairs
+    with torch.inference_mode():
+        for i in range(4):
+            model.predict(xs[i % 2])
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        pend = []
+        for i in range(30):
+            pend.append(model.predict_async(xs[i % 2]))
+            if len(pend) > 1:
+                pend.pop(0).wait()
+        for q in pend:
+            q.wait()
+        e1.record()
+        torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / 30
+
+
+for enc_pairs in (0, 1):
+    ms = time_forward(enc_pairs)
+    print(f"masked forward (PPG 4/16, THX 8/16 nights live), enc_pairs={enc_pairs}: {ms:.3f} ms/step")

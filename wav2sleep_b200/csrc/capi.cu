@@ -303,8 +303,7 @@ int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* 
   const bool linear_shape = c.epilogue == W2S_EPI_BIAS_GELU && c.taps == 4 && c.stride == 4 && c.dilation == 1 && c.pad == 0 &&
                             c.prologue == W2S_PRO_NORM_RES && !c.has_ds && impl == 0 && c.cout == 128 &&
                             (c.cin == 64 || c.cin == 128) && !c.in_wide && !c.out_wide && !c.force_split;
-  static const bool pair_linear = [] { const char* e = getenv("W2S_PAIR_LINEAR"); return !e || atoi(e) != 0; }();
-  if (c2 != nullptr && !((stream_shape && stream_pairable(c.cout, c.has_ds != 0)) || (linear_shape && pair_linear)))
+  if (c2 != nullptr && !((stream_shape && stream_pairable(c.cout, c.has_ds != 0)) || linear_shape))
     return kNotPaired;
   LaunchScope scope(st, label, npair * (in_b + out_b + ab_b), npair * fl);
   if (stream_shape) {
@@ -320,40 +319,28 @@ int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* 
   W2S_STREAMX(CIN, COUT, STRIDE, PRO, DS, MT, NR, NA, NTW, WIN, WOUT, (CIN <= 16 && COUT <= 16))
 #define W2S_STREAM(CIN, COUT, STRIDE, PRO, DS, MT, NR, NA, NTW) \
   W2S_STREAMW(CIN, COUT, STRIDE, PRO, DS, MT, NR, NA, NTW, false, false)
-    // W2S_STREAMD: kernels with CIN >= W2S_DIRECT_MIN_CIN drop the raw ring (NR = 0: the transform warps read global
-    // memory directly through a register prefetch ring, conv_stream.cuh) and use NAD A stages instead of NA.  Default
-    // 128: only the 128-channel kernels, whose weights left room for a single A stage next to a raw ring.
-#ifndef W2S_DIRECT_MIN_CIN
-#define W2S_DIRECT_MIN_CIN 128
-#endif
-#define W2S_STREAMD(CIN, COUT, STRIDE, PRO, DS, MT, NR, NA, NTW, NAD) \
-  W2S_STREAM(CIN, COUT, STRIDE, PRO, DS, MT, (CIN >= W2S_DIRECT_MIN_CIN ? 0 : NR), (CIN >= W2S_DIRECT_MIN_CIN ? NAD : NA), NTW)
-    //          cin cout s  prologue      ds    MT NR NA NTW [NA direct]
+    //          cin cout s  prologue      ds    MT NR NA NTW
     W2S_STREAM(16, 16, 1, PRO_FIR, false, 8, 3, 2, 18)
     W2S_STREAM(16, 16, 1, PRO_NORM_RES_X, true, 8, 2, 2, 14)
-    W2S_STREAMD(16, 16, 1, PRO_NORM, false, 8, 2, 2, 18, 3)
-    W2S_STREAMD(16, 16, 2, PRO_NORM, false, 4, 2, 2, 18, 3)
-    W2S_STREAMD(16, 16, 1, PRO_NORM_RES, true, 4, 3, 2, 14, 3)
+    W2S_STREAM(16, 16, 1, PRO_NORM, false, 8, 2, 2, 18)
+    W2S_STREAM(16, 16, 2, PRO_NORM, false, 4, 2, 2, 18)
+    W2S_STREAM(16, 16, 1, PRO_NORM_RES, true, 4, 3, 2, 14)
     // (10 transform warps at 120 registers; 12 / 14 warps cap the kernel at 96 registers and spill: 16 -> 32 conv1
     //  265 -> 339 / 361 us per paired launch, 32 -> 32 conv1 227 -> 214 / 241 us, step +2-3 %)
-    W2S_STREAMD(16, 32, 1, PRO_NORM_RES, true, 4, 3, 2, 10, 3)
-    W2S_STREAMD(32, 32, 1, PRO_NORM, false, 4, 2, 2, 14, 3)
-    W2S_STREAMD(32, 32, 2, PRO_NORM, false, 2, 2, 2, 14, 3)
-    W2S_STREAMD(32, 32, 1, PRO_NORM_RES, true, 2, 3, 2, 10, 3)
-    W2S_STREAMD(32, 64, 1, PRO_NORM_RES, true, 2, 3, 2, 14, 3)
-    W2S_STREAMD(64, 64, 1, PRO_NORM, false, 2, 2, 2, 14, 3)
-    W2S_STREAMD(64, 64, 2, PRO_NORM, false, 1, 3, 2, 14, 3)
-    W2S_STREAMD(64, 64, 1, PRO_NORM_RES, true, 1, 3, 2, 14, 3)
+    W2S_STREAM(16, 32, 1, PRO_NORM_RES, true, 4, 3, 2, 10)
+    W2S_STREAM(32, 32, 1, PRO_NORM, false, 4, 2, 2, 14)
+    W2S_STREAM(32, 32, 2, PRO_NORM, false, 2, 2, 2, 14)
+    W2S_STREAM(32, 32, 1, PRO_NORM_RES, true, 2, 3, 2, 10)
+    W2S_STREAM(32, 64, 1, PRO_NORM_RES, true, 2, 3, 2, 14)
+    W2S_STREAM(64, 64, 1, PRO_NORM, false, 2, 2, 2, 14)
+    W2S_STREAM(64, 64, 2, PRO_NORM, false, 1, 3, 2, 14)
+    W2S_STREAM(64, 64, 1, PRO_NORM_RES, true, 1, 3, 2, 14)
     W2S_STREAM(64, 128, 1, PRO_NORM_RES, true, 1, 0, 3, 14)  // direct: 68 vs 75 us (the 64 -> 64 kernels lose 12-20 %)
-#ifdef W2S_C128_RING  // A/B build: raw ring + ONE A stage (round-1 / early round-2 configuration)
-    W2S_STREAM(128, 128, 1, PRO_NORM, false, 1, 2, 1, 14)
-    W2S_STREAM(128, 128, 2, PRO_NORM, false, 1, 1, 1, 14)
-    W2S_STREAM(128, 128, 1, PRO_NORM_RES, true, 1, 1, 1, 14)
-#else  // NR = 0, 2-3 A stages
+    // NR = 0 (direct from global, conv_stream.cuh): the 128-channel weights leave room for one A stage next to a raw
+    // ring, and two or three without one
     W2S_STREAM(128, 128, 1, PRO_NORM, false, 1, 0, 3, 14)
     W2S_STREAM(128, 128, 2, PRO_NORM, false, 1, 0, 2, 14)
     W2S_STREAM(128, 128, 1, PRO_NORM_RES, true, 1, 0, 2, 14)
-#endif
     // wide (fp32) storage of the leading <= 32-channel blocks            MT NR NA NTW  in     out
     W2S_STREAMW(16, 16, 1, PRO_FIR, false, 8, 3, 2, 18, false, true)
     W2S_STREAMW(16, 16, 1, PRO_NORM_RES_X, true, 4, 3, 2, 14, true, true)
@@ -373,7 +360,6 @@ int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* 
     W2S_STREAMX(64, 64, 1, PRO_NORM_RES, true, 1, 1, 2, 14, true, true, true)
     W2S_STREAMX(64, 128, 1, PRO_NORM_RES, true, 1, 1, 2, 14, true, false, false)
 #undef W2S_STREAM
-#undef W2S_STREAMD
 #undef W2S_STREAMW
 #undef W2S_STREAMX
     if (!found && (c.in_wide || c.out_wide || c.force_split))
@@ -384,7 +370,7 @@ int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* 
       return 0;
     }
   }
-  if (c2 != nullptr && linear_shape && pair_linear) {
+  if (c2 != nullptr && linear_shape) {
     e = c.cin == 64 ? launch_conv_igemm_pair<64, 128, 4, 4, PRO_NORM_RES, EPI_BIAS_GELU, false>(a, a2s, c.B, st)
                     : launch_conv_igemm_pair<128, 128, 4, 2, PRO_NORM_RES, EPI_BIAS_GELU, false>(a, a2s, c.B, st);
     return e == cudaSuccess ? 0 : cuda_fail(e, "conv_igemm pair launch");
@@ -892,8 +878,7 @@ int w2s_encoder_fwd_pair(const w2s_encoder_desc* d0, const float* x0, void* work
       if (rc == 0) continue;
       if (rc != kNotPaired) return 1;
     }
-    static const bool pair_xstats = [] { const char* e = getenv("W2S_PAIR_XSTATS"); return !e || atoi(e) != 0; }();
-    if (pair_xstats && p0[i].kind == EncStep::XSTATS && p0[i].B == p1[i].B && p0[i].L == p1[i].L) {
+    if (p0[i].kind == EncStep::XSTATS && p0[i].B == p1[i].B && p0[i].L == p1[i].L) {
       if (run_x_stats(p0[i], &p1[i], st) != 0) return 1;
       continue;
     }
@@ -954,16 +939,6 @@ size_t w2s_seqmixer_workspace_bytes(const w2s_seq_desc* d, int B, int S, int kee
   return t * 4 > fused ? t * 4 : fused;
 }
 
-// W2S_SEQ_FUSED=0 in the environment selects the layer-per-launch sequence mixer (A/B measurements).
-static bool seq_fused_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("W2S_SEQ_FUSED");
-    on = (e != nullptr && e[0] == '0') ? 0 : 1;
-  }
-  return on == 1;
-}
-
 int w2s_seqmixer_head_fwd(const w2s_seq_desc* d, const void* x, int B, int S, void* workspace, size_t ws_bytes,
                           int keep, void* feat_out, float* logits, void* stream) {
   if (d == nullptr || x == nullptr || workspace == nullptr || logits == nullptr) return fail("seqmixer: null pointer");
@@ -975,9 +950,7 @@ int w2s_seqmixer_head_fwd(const w2s_seq_desc* d, const void* x, int B, int S, vo
   const size_t t = align_up((size_t)B * S * 128 * sizeof(__half), 256);
   uint8_t* ws = (uint8_t*)workspace;
   SeqGeom geom;
-  static const int nc_force = getenv("W2S_SEQ_NC") ? atoi(getenv("W2S_SEQ_NC")) : 0;  // A/B: pin the cluster size
-  if (!keep && seq_fused_enabled() && d->n_blocks * d->n_dilations <= kSeqMaxLayers &&
-      seq_fused_geometry(B, S, d->n_dilations, geom, nc_force)) {
+  if (!keep && d->n_blocks * d->n_dilations <= kSeqMaxLayers && seq_fused_geometry(B, S, d->n_dilations, geom)) {
     // inference: all layers of a night inside one thread-block cluster (seq_mixer.cuh)
     SeqArgs a;
     memset(&a, 0, sizeof(a));

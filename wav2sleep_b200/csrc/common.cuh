@@ -58,15 +58,9 @@ W2S_DEVINL bool mbar_try_wait_hint(uint64_t* bar, uint32_t parity, uint32_t ns) 
 W2S_DEVINL void mbar_wait(uint64_t* bar, uint32_t parity) {
   if (mbar_try_wait(bar, parity)) return;
   uint32_t it = 0;
-#ifdef W2S_WAIT_PLAIN  // A/B build: plain try_wait polling (hardware-default suspend window), no NANOSLEEP
-  while (!mbar_try_wait(bar, parity)) {
-    if (++it > (1u << 28)) __trap();
-  }
-#else
   while (!mbar_try_wait_hint(bar, parity, 20000u)) {
     if (++it > (1u << 22)) __trap();
   }
-#endif
 }
 
 // One lane of a fully converged warp (warp-uniform code keeps operands in uniform registers, so single-thread
@@ -211,11 +205,10 @@ W2S_DEVINL float gelu_fast(float x) {
   return __fdividef(x, 1.0f + e);
 }
 // Two elements at once on the packed-fp32 pipe (FFMA2/FMUL2/FADD2, sm_100): ~half the issue slots of gelu_fast.
-// Clamping t = x^2 (not x) keeps the exponent monotone for |x| > 5: u = x * q(25), |u| >= 21.7, Phi saturates.
-#ifndef W2S_GELU_EX2
-// Default: 0.5 x (1 + tanh(x p(min(x^2,25)))) with ONE MUFU.TANH per element (tanh.approx.f32, 2^-11 relative error:
-// below fp16 rounding of the result).  Measured against the ex2+rcp form below: same logit parity (cardio 9e-3 /
-// 100 %, EOG 2.2e-2 / 99.7 %), 10 % faster step.  -DW2S_GELU_EX2 selects the 2.5e-5-accurate variant.
+// 0.5 x (1 + tanh(x p(min(x^2,25)))) with ONE MUFU.TANH per element (tanh.approx.f32, 2^-11 relative error: below
+// fp16 rounding of the result).  Clamping t = x^2 (not x) keeps the argument monotone for |x| > 5: u = x * p(25),
+// |u| >= 7.5, tanh saturates.  Measured against a packed ex2+rcp form of gelu_fast: same logit parity (cardio 9e-3 /
+// 100 %, EOG 2.2e-2 / 99.7 %), 10 % faster step.
 W2S_DEVINL float2 gelu_fast2(float2 x) {
   float2 t = __fmul2_rn(x, x);
   t.x = fminf(t.x, 25.0f);
@@ -229,24 +222,6 @@ W2S_DEVINL float2 gelu_fast2(float2 x) {
   const float2 h = __fmul2_rn(x, make_float2(0.5f, 0.5f));
   return __ffma2_rn(h, th, h);
 }
-#else
-W2S_DEVINL float2 gelu_fast2(float2 x) {
-  float2 t = __fmul2_rn(x, x);
-  t.x = fminf(t.x, 25.0f);
-  t.y = fminf(t.y, 25.0f);
-  float2 q = __ffma2_rn(t, make_float2(1.01448193e-3f, 1.01448193e-3f), make_float2(-0.10677673f, -0.10677673f));
-  q = __ffma2_rn(q, t, make_float2(-2.30112048f, -2.30112048f));
-  const float2 u = __fmul2_rn(x, q);
-  float2 e;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e.x) : "f"(u.x));
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e.y) : "f"(u.y));
-  const float2 d = __fadd2_rn(e, make_float2(1.0f, 1.0f));
-  float2 r;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r.x) : "f"(d.x));
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r.y) : "f"(d.y));
-  return __fmul2_rn(x, r);
-}
-#endif
 W2S_DEVINL uint4 lds128(uint32_t addr) {
   uint4 v;
   asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));

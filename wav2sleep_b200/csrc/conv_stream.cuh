@@ -11,7 +11,8 @@
 //   warp 1 (1 lane)  : MMA issuer - tcgen05.mma per 128-row sub-tile and tap into a double-buffered TMEM stage
 //   warps 2..5       : epilogue   - tcgen05.ld, fp16 store, sum / sum-of-squares kept in registers across tiles and
 //                                   flushed with fp64 atomics only when the sample changes
-// Stages hand over through mbarriers (raw full/empty, A full/empty, TMEM full/empty); weights are loaded once.
+// Stages hand over through mbarriers (raw full, A empty, TMEM full/empty) and named barriers (transform -> producer
+// "raw stage read", transform -> MMA issuer "A stage written"); weights are loaded once.
 // Variants: NR = 0 (StreamCfg::DIRECT) drops the raw ring - the transform warps read global memory directly through a
 // register prefetch ring (128-channel kernels); a paired launch (ConvGroup2) runs the same layer of two encoders of
 // identical architecture in one grid, split in proportion to the encoders' live samples.
@@ -41,8 +42,8 @@ W2S_DEVINL void dbg_ts(const ConvArgs& p, int slot) {
   }
 }
 
-// debug_flags & 64: cycles a role spends blocked in mbarrier waits (slot 11 producer, 12 MMA, 13 epilogue warp 2,
-// 14 transform warp 0, 15 = total cycles of the CTA), to see which stage the pipeline is waiting for.
+// debug_flags & 64: cycles a role spends blocked in mbarrier waits (slot 12 MMA, 13 epilogue warp 2, 14 transform
+// warp 0, 15 = total cycles of the CTA), to see which stage the pipeline is waiting for.
 struct WaitClock {
   long long acc = 0;
   W2S_DEVINL void wait(const ConvArgs& p, uint64_t* bar, uint32_t parity) {
@@ -74,10 +75,7 @@ constexpr int stream_threads(int ntw, int cout) { return 32 * (stream_first_tran
 // bar.sync parks the waiting warp in hardware until the count is reached - no polling.  ncu source view of the round-2
 // kernels: 15 % of the executed warp instructions were still mbarrier polls of waiting roles (SYNCS 6.4 %, NANOSLEEP 2.9 %
 // and their branches), because a parked try_wait is woken by every mbarrier event of the CTA and the transform warps
-// produced 36 such events per tile.  -DW2S_NAMED_BARS=0 restores the mbarrier hand-over (A/B).
-#ifndef W2S_NAMED_BARS
-#define W2S_NAMED_BARS 1
-#endif
+// produced 36 such events per tile.
 W2S_DEVINL void named_arrive(int id, int nthreads) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 W2S_DEVINL void named_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 
@@ -198,18 +196,8 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
   constexpr uint32_t IDESC = umma_idesc_f16(128, COUT, false);
   constexpr bool REG_STATS = Cfg::REG_STATS;
   constexpr bool STAGED = Cfg::STAGED;
-  // Transform -> MMA / producer hand-over: one mbarrier arrive per transform warp.  The alternative (-DW2S_TILE_ARRIVE:
-  // the transform warps meet at a named barrier and one thread arrives, 2 instead of 36 mbarrier events per tile, so the
-  // parked waiters of the CTA are woken less often) was measured on one box against this build: 1.3 % SLOWER per step,
-  // 2 % slower summed kernel time - the lock-step of 14-18 warps costs more than the spurious wake-ups.
-#ifdef W2S_TILE_ARRIVE
-  constexpr int kTransformArrives = 1;
-#else
-  constexpr int kTransformArrives = NTW;
-#endif
   // named barriers: ids 1 .. NA = "A stage written" (transform -> MMA issuer), NA+1 .. NA+NR = "raw stage read"
   // (transform -> producer); each is joined by the NTW transform warps (bar.arrive) and the one waiting warp (bar.sync)
-  constexpr bool NAMED = W2S_NAMED_BARS != 0;
   constexpr int kNamedCount = 32 * (NTW + 1);
   static_assert(NA + NR < 16, "named barrier ids");
 
@@ -219,9 +207,7 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
   uint8_t* sB = sA + NA * Cfg::A_BYTES;
   uint8_t* sCtl = sB + Cfg::B_BYTES;
   uint64_t* raw_full = reinterpret_cast<uint64_t*>(sCtl);
-  uint64_t* raw_empty = raw_full + NR;
-  uint64_t* a_full = raw_empty + NR;
-  uint64_t* a_empty = a_full + NA;
+  uint64_t* a_empty = raw_full + NR;
   uint64_t* t_full = a_empty + NA;
   uint64_t* t_empty = t_full + 2;
   uint64_t* w_full = t_empty + 2;  // weights landed in sB (one bulk-copy transaction group per CTA)
@@ -251,14 +237,8 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
   if (warp == 0) tmem_alloc(tmem_slot, Cfg::TMEM_COLS);
   if (tid == 0) dbg_ts(p, 1);
   if (tid == 32) {
-    for (int s = 0; s < NR; ++s) {
-      mbar_init(&raw_full[s], 1);
-      mbar_init(&raw_empty[s], kTransformArrives);
-    }
-    for (int s = 0; s < NA; ++s) {
-      mbar_init(&a_full[s], kTransformArrives);
-      mbar_init(&a_empty[s], 1);
-    }
+    for (int s = 0; s < NR; ++s) mbar_init(&raw_full[s], 1);
+    for (int s = 0; s < NA; ++s) mbar_init(&a_empty[s], 1);
     for (int s = 0; s < 2; ++s) {
       mbar_init(&t_full[s], 1);
       mbar_init(&t_empty[s], Cfg::EPI_WARPS);
@@ -266,27 +246,10 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
     mbar_init(w_full, 1);
     fence_mbar_init();
   }
-  // Programmatic dependent launch (only with W2S_PDL=1, see launch_conv_stream; both instructions are no-ops for a
-  // normally launched grid): the next stream kernel of this CUDA stream may be scheduled onto SMs as this grid's CTAs
-  // exit (launch latency, TMEM allocation and barrier set-up then overlap this grid's tail); everything that reads or
-  // writes global memory comes after the wait, which returns when the preceding grid has completed and flushed.
-#ifndef W2S_PDL_LATE_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-#ifdef W2S_SERIAL_LIVE  // A/B build: one thread scans the mask (one dependent global load per sample)
-  if (compact && tid == 64) {
-    int n = 0;
-    for (int b = 0; b < n_samples; ++b)
-      if (!pa.row_mask[b]) sLive0[n++] = (uint16_t)b;
-    *sNLive = n;
-  }
-#else
   if (compact && warp == 2) {
     const int n = build_live_list(pa.row_mask, n_samples, sLive0, lane);
     if (lane == 0) *sNLive = n;
   }
-#endif
   if (compact && paired && warp == 3) {
     const int n = build_live_list(pb.row_mask, n_samples, sLive1, lane);
     if (lane == 0) *sNLive1 = n;
@@ -302,7 +265,6 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
   int ctas0 = (int)gridDim.x;
   if (paired) {
     ctas0 = (int)gridDim.x >> 1;
-#ifndef W2S_EQUAL_SPLIT  // (A/B build: always half of the grid per group)
     if (compact) {
       const int n0 = *sNLive, n1 = *sNLive1;
       if (n0 != n1) {  // (equal counts: half each, nothing to compute; 32-bit: gridDim.x * n0 <= 296 * 120)
@@ -311,7 +273,6 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
         if (n1 > 0 && ctas0 > (int)gridDim.x - 1) ctas0 = (int)gridDim.x - 1;
       }
     }
-#endif
   }
   const bool grp1 = paired && (int)blockIdx.x >= ctas0;
   const int cta = grp1 ? (int)blockIdx.x - ctas0 : (int)blockIdx.x;
@@ -362,8 +323,6 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
       }
       __syncwarp();
       int s = 0, n_issued = 0;
-      uint32_t ph = 0;
-      WaitClock wc;
       const long long cta_t0 = clock64();
       TilePos tp = pos0;
       for (int tile = tile_begin; tile < (Cfg::DIRECT ? tile_begin : tile_end); ++tile, advance(tp)) {
@@ -382,12 +341,8 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
         int xhi = xs0 + Cfg::XN;
         xhi = (xhi > p.T_raw ? p.T_raw : xhi) & ~3;
         const uint32_t xbytes = (Cfg::XN > 0 && xhi > xlo) ? (uint32_t)(xhi - xlo) * 4 : 0u;
-        if (NAMED) {
-          if (n_issued >= NR) named_sync(1 + NA + s, kNamedCount);  // (the first NR fills find the ring empty)
-          ++n_issued;
-        } else {
-          wc.wait(p, &raw_empty[s], ph ^ 1);
-        }
+        if (n_issued >= NR) named_sync(1 + NA + s, kNamedCount);  // (the first NR fills find the ring empty)
+        ++n_issued;
         uint8_t* dst = sRaw + s * Cfg::RAW_BYTES + (size_t)(lo - i0) * CIN * ESZ;
         const size_t goff = ((size_t)b * p.L_in + lo) * CIN * ESZ;  // byte offset
         if (elect_one()) {
@@ -400,21 +355,15 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
                      p.x_raw + (size_t)b * p.T_raw + xlo, xbytes, &raw_full[s]);
         }
         __syncwarp();
-        if (++s == NR) {
-          s = 0;
-          ph ^= 1;
-        }
+        if (++s == NR) s = 0;
       }
-      if (lane == 0) {
-        wc.publish(p, 11);
-        if (W2S_DBG(p, 64) && blockIdx.x == 0) g_stream_ts[15] = (unsigned long long)(clock64() - cta_t0);
-      }
+      if (lane == 0 && W2S_DBG(p, 64) && blockIdx.x == 0) g_stream_ts[15] = (unsigned long long)(clock64() - cta_t0);
     }
   } else if (warp == 1) {
     // ---------------- MMA issuer (warp-uniform loop; one elected lane issues) ----------------
     {
       int as = 0, ts = 0;
-      uint32_t aph = 0, tph = 0;
+      uint32_t tph = 0;
       WaitClock wc;
       constexpr uint32_t lbo_a = RP * 16, lbo_b = COUT * 16;
       // descriptors = (stage / operand base) + compile-time offset: one integer add per operand on the issuing thread
@@ -427,8 +376,7 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
       for (int tile = tile_begin; tile < tile_end; ++tile, advance(tp)) {
         int b;
         if (!sample_of(tp, b)) continue;
-        if (NAMED) named_sync(1 + as, kNamedCount);
-        else wc.wait(p, &a_full[as], aph);
+        named_sync(1 + as, kNamedCount);
         wc.wait(p, &t_empty[ts], tph ^ 1);
         tc_fence_after_sync();
         const uint32_t d_base = tmem_base + ts * Cfg::STAGE_COLS;
@@ -479,7 +427,6 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
         a_lo0 += Cfg::A_BYTES >> 4;
         if (++as == NA) {
           as = 0;
-          aph ^= 1;
           a_lo0 = a_lo_first;
         }
         if (++ts == 2) {
@@ -543,17 +490,6 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
       // issued before the single tcgen05.wait::ld: the round trip of a TMEM load while the MMA unit is accumulating
       // into the other stage is several hundred cycles, and it used to be paid once per 16 columns.
       auto stage_in = [&](uint32_t taddr) {
-#ifdef W2S_EPI_LD16  // A/B build: one wait per 16 columns (round-2 first version)
-#pragma unroll
-        for (int q = 0; q < SEG / 16; ++q) {
-          float v[16];
-          tmem_ld16(taddr + q * 16, v);
-          const uint4 lo = make_uint4(pack_h2(v[0], v[1]), pack_h2(v[2], v[3]), pack_h2(v[4], v[5]), pack_h2(v[6], v[7]));
-          const uint4 hi = make_uint4(pack_h2(v[8], v[9]), pack_h2(v[10], v[11]), pack_h2(v[12], v[13]), pack_h2(v[14], v[15]));
-          sts128(stg + lane * SEGB + (((2 * q) ^ swz(lane)) * 16), lo);
-          sts128(stg + lane * SEGB + (((2 * q + 1) ^ swz(lane)) * 16), hi);
-        }
-#else
         uint32_t r[SEG];
 #pragma unroll
         for (int q = 0; q < SEG / 32; ++q) tmem_ld32(taddr + q * 32, r + q * 32);
@@ -566,7 +502,6 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
                                      pack_h2(__uint_as_float(r[8 * c + 6]), __uint_as_float(r[8 * c + 7])));
           sts128(stg + lane * SEGB + ((c ^ swz(lane)) * 16), w);
         }
-#endif
       };
       TilePos tp = pos0;
       for (int tile = tile_begin; tile < tile_end; ++tile, advance(tp)) {
@@ -883,27 +818,11 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
       sts128(adst + soff, o);
       if (SPLIT) sts128(adst + Cfg::A_ONE + soff, olo);
     };
-    // Hand-over: every transform thread publishes its shared-memory writes to the async proxy, then each warp signals
+    // Hand-over: every transform thread publishes its shared-memory writes to the async proxy, then arrives
     auto hand_over = [&]() {
       fence_proxy_async_smem();
-#ifdef W2S_TILE_ARRIVE
-      asm volatile("bar.sync 1, %0;" ::"n"(NTT) : "memory");
-      if (tt == 0) {
-        mbar_arrive(&a_full[as]);
-        if (!Cfg::DIRECT) mbar_arrive(&raw_empty[rs]);
-      }
-#else
-      if (NAMED) {
-        named_arrive(1 + as, kNamedCount);
-        if (!Cfg::DIRECT) named_arrive(1 + NA + rs, kNamedCount);
-      } else {
-        __syncwarp();
-        if (lane == 0) {
-          mbar_arrive(&a_full[as]);
-          if (!Cfg::DIRECT) mbar_arrive(&raw_empty[rs]);
-        }
-      }
-#endif
+      named_arrive(1 + as, kNamedCount);
+      if (!Cfg::DIRECT) named_arrive(1 + NA + rs, kNamedCount);
       if (!Cfg::DIRECT && ++rs == NR) {
         rs = 0;
         rph ^= 1;
@@ -1057,9 +976,6 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
   }
 
   // ---------------- teardown ----------------
-#ifdef W2S_PDL_LATE_TRIGGER  // A/B build: dependents may be scheduled only when this CTA is done with its tiles
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
   tc_fence_before_sync();
   __syncthreads();
   if (tid == 0) dbg_ts(p, 9);
@@ -1094,26 +1010,8 @@ inline cudaError_t launch_conv_stream(const ConvArgs& a, const ConvArgs* a2, int
     grid = 2 * per;
   }
   const ConvGroup2 g2 = conv_group2(a2);
-  // W2S_PDL=1 launches with programmatic stream serialization (never while the stream is being captured).  Measured
-  // (3 alternating rounds, one box): the serialised kernel sum drops 1 % (7.40 vs 7.49 ms) but the step gets 2.4 % SLOWER
-  // (6.72 vs 6.55 ms): the four encoder streams fill each other's tails with useful CTAs, and an early-scheduled
-  // dependent CTA holds its SM idle at griddepcontrol.wait instead.  Re-measured on top of the paired launches (two
-  // streams): 6.73 / 6.70 vs 6.55 / 6.62 ms; with the trigger moved to the end of each CTA's work (-DW2S_PDL_LATE_TRIGGER)
-  // 6.58 / 6.57 / 6.57 vs 6.56 / 6.61 / 6.56 ms - neutral.  Off by default.
-  static const bool pdl_enabled = [] { const char* e = getenv("W2S_PDL"); return e && atoi(e) != 0; }();
-  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-  if (pdl_enabled) cudaStreamIsCapturing(stream, &cap);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(Cfg::THREADS);
-  cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = (pdl_enabled && cap == cudaStreamCaptureStatusNone) ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, a, g2, tiles_per_sample, (int)total);
+  kern<<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, stream>>>(a, g2, tiles_per_sample, (int)total);
+  return cudaGetLastError();
 }
 
 }  // namespace w2s

@@ -22,10 +22,7 @@ constexpr int kMixHeads = 8;     // nhead
 constexpr int kMixHd = 16;       // head dim
 constexpr int kMixFF = 512;      // dim_feedforward
 constexpr int kMixEp = 16;       // epochs per tile
-#ifndef W2S_MIX_THREADS
-#define W2S_MIX_THREADS 256  // measured on B200: 512 threads (16 warps) give the same 395 us per 19200 epochs
-#endif
-constexpr int kMixThreads = W2S_MIX_THREADS;
+constexpr int kMixThreads = 256;  // measured on B200: 512 threads (16 warps) give the same 395 us per 19200 epochs
 constexpr int kMixWarps = kMixThreads / 32;
 constexpr int kMixMaxLayers = 8;
 constexpr int kMixMaxSig = 4;

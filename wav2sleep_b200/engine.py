@@ -161,25 +161,21 @@ class ForwardEngine:
         # One CUDA stream per signal encoder: the encoders are independent chains of ~25 persistent kernels, each of
         # which ends with a tail (CTAs finish 3-20 % apart) and starts with a ~5 us pipeline fill.  On separate
         # streams the next chain's CTAs take over the SMs the moment a kernel's early finishers release them, so
-        # fill and tail of one encoder are covered by the other encoders' work.  W2S_ENC_STREAMS=0 serialises them.
-        import os
-        self.enc_streams = os.environ.get("W2S_ENC_STREAMS", "1") != "0"
+        # fill and tail of one encoder are covered by the other encoders' work.  False serialises them.
+        self.enc_streams = True
         # encoders of identical architecture on inputs of equal length (ECG + PPG, ABD + THX) share their conv launches
-        # (w2s_encoder_fwd_pair); W2S_ENC_PAIRS=0: one launch chain per signal (A/B).
-        # 1 (default): only while at least two launch chains remain to overlap each other's kernel tails - the two-signal
-        # EOG model keeps one chain per signal (paired: 44.4 vs 42.3 ms per 16 x 14-h nights); 2: always
-        self.enc_pairs = int(os.environ.get("W2S_ENC_PAIRS", "1"))
+        # (w2s_encoder_fwd_pair).  0: one launch chain per signal; 1 (default): only while at least two launch chains
+        # remain to overlap each other's kernel tails - the two-signal EOG model keeps one chain per signal (paired: 44.4
+        # vs 42.3 ms per 16 x 14-h nights); 2: always
+        self.enc_pairs = 1
         # measurement mode: the encoder streams run one after the other (isolated per-kernel durations of exactly the
         # launches of a normal step, paired launches included)
         self.serial_groups = False
-        # Asynchronous forwards (forward_async / predict_async) run on the engine's own streams (the current stream only
-        # records the fork event), alternating between n_lanes independent sets of streams and workspaces.  One lane is
-        # the default: with two, consecutive batches could overlap, but measured on B200 it buys nothing (6.91 vs 6.89 ms
-        # per step) - every kernel of the forward claims 150-230 KB of shared memory, so the mixer tail of one batch and
-        # the encoder kernels of the next cannot be co-resident on an SM - and it doubles the workspaces (EOG: 70 GB).
-        self.n_lanes = int(os.environ.get("W2S_LANES", "1"))
-        self.seq_groups = int(os.environ.get("W2S_SEQ_GROUPS", "1"))  # night groups of the sequence mixer (see _seq_head)
-        self._lane = 0
+        # Asynchronous forwards (forward_async / predict_async) run on the engine's own streams and workspaces (the
+        # current stream only records the fork event); a batch starts once the previous one has finished with them.
+        # One set: two alternating sets, which would let consecutive batches overlap, buy nothing on B200 (6.91 vs 6.89
+        # ms per step) - every kernel of the forward claims 150-230 KB of shared memory, so the mixer tail of one batch
+        # and the encoder kernels of the next cannot be co-resident on an SM - and double the workspaces.
 
     # ------------------------------------------------------------------ weights
     def _params_key(self, device):
@@ -246,15 +242,16 @@ class ForwardEngine:
 
     # ------------------------------------------------------------------ buffers
     def _release_buffers(self) -> None:
-        """Drop every workspace.  Batches still in flight on the lanes' own streams must finish before their memory goes
-        back to the allocator of the current stream."""
+        """Drop every workspace.  Batches still in flight on the engine's own streams must finish before their memory
+        goes back to the allocator of the current stream."""
         for old in self._ws.values():
             if old.get("tail_done") is not None:
                 torch.cuda.current_stream(old["mix"].device).wait_event(old["tail_done"])
         self._ws.clear()
 
-    def _buffers(self, device, names, B, S, lane: int = -1):
-        key = (str(device), tuple(names), B, S, self.enc_streams, lane)
+    def _buffers(self, device, names, B, S, detached: bool = False):
+        """Workspaces of one shape; detached: the set of the asynchronous forwards, with their own tail stream."""
+        key = (str(device), tuple(names), B, S, self.enc_streams, detached)
         buf = self._ws.get(key)
         if buf is not None:
             return buf
@@ -265,11 +262,8 @@ class ForwardEngine:
         for n in names:
             pe = self.enc[self.model.signal_encoders.signal_map[n]]
             sizes[n] = lib.w2s_encoder_workspace_bytes(C.byref(pe.desc), B, S * pe.samples_per_epoch, 0)
-        G = max(1, min(self.seq_groups, B))
-        per = (B + G - 1) // G
-        seq_ws = max(lib.w2s_seqmixer_workspace_bytes(C.byref(self.seq_desc), B, S, 0),
-                     G * lib.w2s_seqmixer_workspace_bytes(C.byref(self.seq_desc), per, S, 0))
-        concurrent = (self.enc_streams and len(names) > 1) or lane >= 0
+        seq_ws = lib.w2s_seqmixer_workspace_bytes(C.byref(self.seq_desc), B, S, 0)
+        concurrent = (self.enc_streams and len(names) > 1) or detached
         if concurrent:  # encoders run side by side: one workspace each
             enc_ws = {n: torch.empty(sizes[n], dtype=torch.uint8, device=device) for n in names}
         else:           # encoders run back to back: one workspace of the largest size
@@ -278,8 +272,7 @@ class ForwardEngine:
         buf = {
             "enc_ws": enc_ws,
             "streams": [torch.cuda.Stream(device=device) for _ in names] if concurrent else None,
-            "tail": torch.cuda.Stream(device=device) if lane >= 0 else None,   # mixer + sequence mixer + head of a lane
-            "seq_streams": [torch.cuda.Stream(device=device) for _ in range(G)] if (G > 1 and self.enc_streams) else None,
+            "tail": torch.cuda.Stream(device=device) if detached else None,   # mixer + sequence mixer + head
             "tail_done": None,
             "seq_ws": torch.empty(seq_ws, dtype=torch.uint8, device=device),
             "z": {n: torch.empty(B, S, 128, dtype=torch.float16, device=device) for n in names},
@@ -316,33 +309,10 @@ class ForwardEngine:
         return B, S, device
 
     def _seq_head(self, buf, B: int, S: int, logits: Tensor, stream: "torch.cuda.Stream") -> None:
-        """Sequence mixer + classifier on `stream`, the nights split into groups that run on side streams: each of the 12
-        dependent layer launches is 10 one-tile CTAs per night (160 for 16 nights = two waves on 148 SMs, the second one
-        12 CTAs wide); independent groups make the schedule work-conserving - a group's next layer starts as soon as
-        its own CTAs are done."""
-        lib = self.lib
-        G = min(self.seq_groups, B)
-        if G <= 1 or buf.get("seq_streams") is None:
-            _lib.check(lib.w2s_seqmixer_head_fwd(C.byref(self.seq_desc), buf["mix"].data_ptr(), B, S, buf["seq_ws"].data_ptr(),
-                                                 buf["seq_ws"].numel(), 0, None, logits.data_ptr(), stream.cuda_stream))
-            return
-        fork = torch.cuda.Event()
-        fork.record(stream)
-        per = (B + G - 1) // G
-        ws_per = lib.w2s_seqmixer_workspace_bytes(C.byref(self.seq_desc), per, S, 0)
-        ncls = self.model.num_classes
-        for g in range(G):
-            b0, nb = g * per, min(per, B - g * per)
-            if nb <= 0:
-                break
-            st = buf["seq_streams"][g]
-            st.wait_event(fork)
-            _lib.check(lib.w2s_seqmixer_head_fwd(C.byref(self.seq_desc), buf["mix"].data_ptr() + b0 * S * 128 * 2, nb, S,
-                                                 buf["seq_ws"].data_ptr() + g * ws_per, ws_per, 0, None,
-                                                 logits.data_ptr() + b0 * S * ncls * 4, st.cuda_stream))
-            join = torch.cuda.Event()
-            join.record(st)
-            stream.wait_event(join)
+        """Sequence mixer + classifier on `stream`."""
+        ws = buf["seq_ws"]
+        _lib.check(self.lib.w2s_seqmixer_head_fwd(C.byref(self.seq_desc), buf["mix"].data_ptr(), B, S, ws.data_ptr(),
+                                                  ws.numel(), 0, None, logits.data_ptr(), stream.cuda_stream))
 
     def _enc_groups(self, names, xs, paired: bool):
         """Signals in launch order (longest chains first - they set the critical path when the encoders overlap), grouped
@@ -369,9 +339,6 @@ class ForwardEngine:
                 groups.append((n, mate))
         if len(groups) < 2 and self.enc_pairs < 2:
             return [(n,) for n in order]
-        if self.enc_pairs == 3:  # A/B: pair only the shorter signals, the longest ones keep one chain each
-            tmax = max(xs[n].size(1) for n in order)
-            groups = [g2 for g in groups for g2 in ([(n,) for n in g] if xs[g[0]].size(1) == tmax else [g])]
         return groups
 
     def _encode(self, buf, xs, grp, B: int, stream_ptr) -> None:
@@ -421,7 +388,7 @@ class ForwardEngine:
         self._seq_head(buf, B, S, logits, torch.cuda.current_stream())
 
     def _launch_async(self, buf, xs: dict[str, Tensor], names, B: int, S: int, argmax: bool, ready=None) -> Pending:
-        """The whole forward on the lane's own streams: nothing is enqueued on the current stream except the fork event.
+        """The whole forward on the engine's own streams: nothing is enqueued on the current stream except the fork event.
         ready: optional {signal: event} - the signal's encoder additionally waits for its event (e.g. the end of that
         signal's host -> device copy on another stream), so the first encoders start while the other signals still
         arrive."""
@@ -439,7 +406,7 @@ class ForwardEngine:
                     st.wait_event(ready[n])
                 xs[n].record_stream(st)
             if buf["tail_done"] is not None:
-                st.wait_event(buf["tail_done"])  # the lane's previous batch has finished reading z / masks
+                st.wait_event(buf["tail_done"])  # the previous batch has finished reading z / masks
             self._encode(buf, xs, grp, B, st.cuda_stream)
             ev = torch.cuda.Event()
             ev.record(st)
@@ -462,15 +429,13 @@ class ForwardEngine:
 
     @torch.no_grad()
     def forward_async(self, x: dict[str, Tensor], argmax: bool = False, ready=None) -> Pending:
-        """Enqueue a forward on the next lane and return at once; ``.wait()`` on the result orders the current stream
-        after it.  Up to ``n_lanes`` batches are in flight on the GPU; inputs must stay untouched until then."""
+        """Enqueue a forward on the engine's own streams and return at once; ``.wait()`` on the result orders the current
+        stream after it.  Inputs must stay untouched until then."""
         B, S, device = self._check_inputs(x)
         with torch.cuda.device(device):
             self._ensure_packed(device)
             names = sorted(x.keys())
-            lane = self._lane
-            self._lane = (lane + 1) % max(self.n_lanes, 1)
-            buf = self._buffers(device, names, B, S, lane)
+            buf = self._buffers(device, names, B, S, detached=True)
             xs = {}
             for n in names:
                 t = x[n].detach()

@@ -397,8 +397,8 @@ class Wav2Sleep(nn.Module):
 
     def predict_async(self, x: dict[str, Tensor], ready=None):
         """``predict`` without ordering the current stream after it: returns a handle whose ``wait()`` does (and hands
-        back the int64 [B, S] tensor).  Consecutive calls alternate between two sets of streams and workspaces, so the
-        latency-bound tail of one batch overlaps the encoders of the next (throughput mode for loops over batches).
+        back the int64 [B, S] tensor).  The host can enqueue the next batches while the GPU works (throughput mode for
+        loops over batches); each batch runs on the engine's own streams and starts once the previous one is done.
         ``ready``: optional ``{signal: torch.cuda.Event}``; a signal's encoder starts once its event has completed (e.g.
         that signal's host -> device copy on a copy stream), so a batch need not be fully uploaded before work begins."""
         if not self.fast_path:

@@ -12,8 +12,6 @@ the encoder backward, which is >90 % of the step.
 """
 from __future__ import annotations
 
-import os
-
 from typing import Callable, Iterable, Optional
 
 import torch
@@ -129,14 +127,12 @@ def sum_if_distributed(t: Tensor) -> Tensor:
 class GradReducer:
     """Bucketed SUM all-reduce of a flat gradient buffer, fired from the backward's bucket hooks."""
 
-    def __init__(self, flat_grad: Tensor, segments: dict[str, tuple[int, int]], process_group=None, use_stream=True,
-                 overlap: bool = True):
-        """overlap=True: each bucket is reduced on a side stream as soon as the backward has finished it.
-        overlap=False: one all-reduce of the whole flat gradient in ``wait()`` (after the backward).  Measured on 2 x B200
-        both take the same step time (55.5 ms): the exchange is only 11.8 MB; the multi-GPU step is longer than the
-        single-GPU one because each rank draws its own modality masks and the slowest rank sets the pace."""
+    def __init__(self, flat_grad: Tensor, segments: dict[str, tuple[int, int]], process_group=None, use_stream=True):
+        """Each bucket is reduced on a side stream as soon as the backward has finished it.  Measured on 2 x B200, one
+        all-reduce of the whole flat gradient after the backward takes the same step time (55.5 ms): the exchange is
+        only 11.8 MB; the multi-GPU step is longer than the single-GPU one because each rank draws its own modality
+        masks and the slowest rank sets the pace."""
         self.flat_grad, self.segments, self.group = flat_grad, segments, process_group
-        self.overlap = overlap
         self.use_stream = use_stream and flat_grad.is_cuda
         self.comm = torch.cuda.Stream(device=flat_grad.device) if self.use_stream else None
         self.done = []
@@ -148,7 +144,7 @@ class GradReducer:
 
     def __call__(self, bucket: str) -> None:
         self.fired.append(bucket)
-        if self.world_size == 1 or bucket not in self.segments or not self.overlap:
+        if self.world_size == 1 or bucket not in self.segments:
             return
         a, b = self.segments[bucket]
         seg = self.flat_grad[a:b]
@@ -166,8 +162,6 @@ class GradReducer:
 
     def wait(self) -> None:
         """Make the current stream wait for every bucket issued since the last call (before the optimizer step)."""
-        if not self.overlap and self.world_size > 1:
-            dist.all_reduce(self.flat_grad, op=dist.ReduceOp.SUM, group=self.group)
         for ev in self.done:
             torch.cuda.current_stream().wait_event(ev)
         self.done.clear()
@@ -328,8 +322,7 @@ class SleepLightningModule(nn.Module):
             covered = sum(b - a for a, b in segs.values())
             if covered != self._opt.flat_grad.numel():  # e.g. a parameter outside encoders / tail: one late bucket
                 segs = {"tail": segs["tail"], "encoders": self._opt.segment(enc)}
-            self._reducer = GradReducer(self._opt.flat_grad, segs, process_group,
-                                        overlap=os.environ.get("W2S_DDP_OVERLAP", "1") != "0")
+            self._reducer = GradReducer(self._opt.flat_grad, segs, process_group)
             self._opt.grad_scale = 1.0 / self._reducer.world_size
             if self._reducer.world_size > 1:
                 # what Lightning's DDP strategy does at start-up: every replica begins from rank 0's parameters

@@ -24,7 +24,6 @@ exactly (powers of two), and nothing outside this file sees the scale.
 from __future__ import annotations
 
 import contextlib
-import os
 import ctypes as C
 
 import torch
@@ -59,10 +58,8 @@ class TrainEngine(ForwardEngine):
         self.last_dropout_seed = 0
         self._side_streams = {}   # device -> per-encoder CUDA streams (same overlap of kernel tails as in inference)
         # InstanceNorm backward of a layer's gradient inside the prologue of the data-gradient conv that consumes it
-        # (W2S_PRO_DNORM) instead of a separate enc_norm_bwd pass; W2S_FUSE_NORM_BWD=0 keeps the separate kernels (A/B)
-        self.fuse_norm_bwd = os.environ.get("W2S_FUSE_NORM_BWD", "1") != "0"
-        # weight gradients of the classifier / mixer backward on a side stream (W2S_WGRAD_STREAM=0: in stream order, A/B)
-        self.wgrad_stream = os.environ.get("W2S_WGRAD_STREAM", "1") != "0"
+        # (W2S_PRO_DNORM) instead of a separate enc_norm_bwd pass; False keeps the separate kernels
+        self.fuse_norm_bwd = True
         self._wg = None
         self._wg_streams = {}
         self.loss_scale = None    # power of two applied to the fp16 activation gradients; None = from B*S (see below)
@@ -450,8 +447,7 @@ class TrainEngine(ForwardEngine):
             st = _stream()
             G = self._grad
             dlogits = dlogits.detach().to(torch.float32).contiguous()
-            if self.wgrad_stream:
-                self._wg = self._wg_streams.setdefault(str(device), torch.cuda.Stream(device=device))
+            self._wg = self._wg_streams.setdefault(str(device), torch.cuda.Stream(device=device))
             # ---- classifier ----
             dfeat = torch.empty(N, 128, dtype=F16, device=device)
             _lib.check(lib.w2s_head_bwd(sv["feat"].data_ptr(), sv["wc"].data_ptr(), dlogits.data_ptr(), dfeat.data_ptr(),
