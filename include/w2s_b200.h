@@ -379,9 +379,51 @@ int w2s_gen_affine_act(const float* in, const float* scale, const float* shift, 
 /* per-row LayerNorm (rms = 0) / RMSNorm (rms = 1) over C features, affine weight (+ bias), activation. */
 int w2s_gen_rownorm(const float* x, const float* weight, const float* bias, float* out, long long rows, int C, int rms, int act,
                     float eps, void* stream);
-/* H-head attention over the D tokens of each of N epochs; q, k, v, o: [N, D, H*hd]; key_mask [N, D] (1 = masked). */
+/* H-head attention over the D tokens of each of N epochs; q, k, v: rows of ld >= H*hd floats ([N, D, ld], e.g. ld = 3*H*hd
+ * for column slices of one fused in-projection), o: [N, D, H*hd]; key_mask [N, D] (1 = masked).  drop_p > 0: dropout on
+ * the attention weights (nn.MultiheadAttention in training), keep decision of element ((n*H + h)*D + query)*D + key of
+ * dropout site `site` (the generator of w2s_dropout).  drop_p = 0: no dropout.  (ABI v5: ld, drop_p, seed, site) */
 int w2s_gen_attn(const float* q, const float* k, const float* v, float* o, const uint8_t* key_mask, int N, int D, int H, int hd,
-                 void* stream);
+                 int ld, float drop_p, uint64_t seed, uint32_t site, void* stream);
+
+/* Backward of the general path (training of the non-default options; ABI v5).  Same conventions as the forward entry
+ * points; rows of samples with row_mask[b] != 0 are skipped (their gradients stay as the caller initialised them, and they
+ * add nothing to any reduction).  Parameter gradients are written (not accumulated).  The fp64 workspaces `ws` / `sums`
+ * are zeroed by the call itself. */
+/* din[b, li, ci] = sum over (lo, t) with lo*stride - pad_left + t*dil = li of dout[b, lo, co] * w[co, ci, t]  (gather, no
+ * atomics; every case of w2s_gen_conv incl. taps_major). */
+int w2s_gen_conv_dgrad(const float* dout, const float* w, float* din, const uint8_t* row_mask, int B, int L_in, int L_out, int cin,
+                       int cout, int taps, int stride, int dil, int pad_left, int taps_major, void* stream);
+/* dw[co, ci, t] = sum_{b, lo} dout * in (layout of w2s_gen_conv's w), dbias[co] = sum dout; non-finite raw samples read as 0
+ * (raw_inf_to_zero).  dw or dbias may be NULL.  ws: taps*cin*cout + cout doubles. */
+int w2s_gen_conv_wgrad(const float* in, const float* dout, float* dw, float* dbias, double* ws, const uint8_t* row_mask, int B,
+                       int L_in, int L_out, int cin, int cout, int taps, int stride, int dil, int pad_left, int taps_major,
+                       int raw_inf_to_zero, void* stream);
+/* Backward of w2s_gen_affine_act: dpre = dout * act'(in * scale + shift + res); din = dpre * scale (NULL: skipped); dpre (the
+ * residual gradient; NULL: skipped); sums (NULL: skipped) = fp64 (sum dpre, sum dpre * in) per [b, c] (per [c] when
+ * per_channel), i.e. the shift and scale gradients. */
+int w2s_gen_affine_act_bwd(const float* in, const float* scale, const float* shift, const float* res, const float* dout, float* din,
+                           float* dpre, double* sums, const uint8_t* row_mask, int B, int L, int C, int act, int per_channel,
+                           void* stream);
+/* InstanceNorm (groups = C) / GroupNorm backward: from the forward's stats and the sums of w2s_gen_affine_act_bwd over
+ * the conv output x, dx = alpha * dpre + beta * x + gamma per [b, c] (coef: workspace of B*C*3 floats); dweight / dbias
+ * (NULL: skipped) of the affine GroupNorm. */
+int w2s_gen_norm_bwd(const float* x, const float* dpre, const double* stats, const double* sums, const float* weight, float* coef,
+                     float* dx, float* dweight, float* dbias, const uint8_t* row_mask, int B, int L, int C, int groups, float eps,
+                     void* stream);
+/* Backward of w2s_gen_rownorm (fused activation included): dx, and dweight / dbias (NULL: skipped) as fp64 column sums over
+ * the rows (ws: 2*C doubles, needed when either is requested).  C <= 2048. */
+int w2s_gen_rownorm_bwd(const float* x, const float* weight, const float* bias, const float* dout, float* dx, float* dweight,
+                        float* dbias, double* ws, long long rows, int C, int rms, int act, float eps, void* stream);
+/* Backward of w2s_gen_attn (same key mask, same dropout decisions): dq, dk, dv with the row stride ld of q, k, v; dout has
+ * rows of H*hd.  Masked keys get dk = dv = 0. */
+int w2s_gen_attn_bwd(const float* q, const float* k, const float* v, const float* dout, float* dq, float* dk, float* dv,
+                     const uint8_t* key_mask, int N, int D, int H, int hd, int ld, float drop_p, uint64_t seed, uint32_t site,
+                     void* stream);
+/* fp32 dropout over any n < 2^32 elements: out[i] = keep(seed, site, i) ? x[i] / (1 - p) : 0, the decisions of w2s_dropout;
+ * applied to the gradient it is the backward.  mask_out != NULL: only write the n keep decisions (0/1) there (test hook). */
+int w2s_gen_dropout(const float* x, float* out, uint8_t* mask_out, long long n, float p, uint64_t seed, uint32_t site,
+                    void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
  * Measurement hooks (bench.py).  Not part of the data path.

@@ -23,7 +23,7 @@ MAX_MIXER_LAYERS = 8
 MAX_SIGNALS = 4
 MAX_SEQ_BLOCKS = 4
 MAX_DILATIONS = 8
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 PRO_NONE, PRO_NORM, PRO_NORM_RES, PRO_FIR, PRO_NORM_RES_X, PRO_DNORM = 0, 1, 2, 3, 4, 5
 EPI_STATS, EPI_BIAS_GELU, EPI_LN_GELU, EPI_LN_GELU_RES, EPI_PLAIN, EPI_ACT_BWD = 0, 1, 2, 3, 4, 5
@@ -183,7 +183,14 @@ SYMBOLS = {
     "w2s_gen_norm_consts": (C.c_int, [C.c_void_p] * 7 + [C.c_int] * 5 + [C.c_float, C.c_void_p]),
     "w2s_gen_affine_act": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 5 + [C.c_void_p]),
     "w2s_gen_rownorm": (C.c_int, [C.c_void_p] * 4 + [C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p]),
-    "w2s_gen_attn": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 4 + [C.c_void_p]),
+    "w2s_gen_attn": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 5 + [C.c_float, C.c_uint64, C.c_uint32, C.c_void_p]),
+    "w2s_gen_conv_dgrad": (C.c_int, [C.c_void_p] * 4 + [C.c_int] * 10 + [C.c_void_p]),
+    "w2s_gen_conv_wgrad": (C.c_int, [C.c_void_p] * 6 + [C.c_int] * 11 + [C.c_void_p]),
+    "w2s_gen_affine_act_bwd": (C.c_int, [C.c_void_p] * 9 + [C.c_int] * 5 + [C.c_void_p]),
+    "w2s_gen_norm_bwd": (C.c_int, [C.c_void_p] * 10 + [C.c_int] * 4 + [C.c_float, C.c_void_p]),
+    "w2s_gen_rownorm_bwd": (C.c_int, [C.c_void_p] * 8 + [C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p]),
+    "w2s_gen_attn_bwd": (C.c_int, [C.c_void_p] * 8 + [C.c_int] * 5 + [C.c_float, C.c_uint64, C.c_uint32, C.c_void_p]),
+    "w2s_gen_dropout": (C.c_int, [C.c_void_p] * 3 + [C.c_longlong, C.c_float, C.c_uint64, C.c_uint32, C.c_void_p]),
     "w2s_launch_count": (C.c_longlong, []),
     "w2s_profile_enable": (C.c_int, [C.c_int]),
     "w2s_profile_count": (C.c_int, []),

@@ -22,6 +22,7 @@
 #include "train_kernels.cuh"
 #include "check_fp32.cuh"
 #include "general.cuh"
+#include "general_bwd.cuh"
 #include "staging.cuh"
 #include "seq_mixer.cuh"
 
@@ -506,7 +507,7 @@ int check_encoder_desc(const w2s_encoder_desc* d) {
 
 extern "C" {
 
-int w2s_abi_version(void) { return 4; }
+int w2s_abi_version(void) { return 5; }
 const char* w2s_last_error(void) { return g_err.c_str(); }
 
 int w2s_conv_uses_split(int cin, int cout) { return (cin <= 16 && cout <= 16) ? 1 : 0; }
@@ -1368,12 +1369,126 @@ int w2s_gen_rownorm(const float* x, const float* weight, const float* bias, floa
   W2S_LAUNCH_CHECK("gen_rownorm");
 }
 int w2s_gen_attn(const float* q, const float* k, const float* v, float* o, const uint8_t* key_mask, int N, int D, int H, int hd,
-                 void* stream) {
-  if (!q || !k || !v || !o || N <= 0 || D < 1 || H < 1 || hd < 1) return fail("gen_attn: bad arguments");
-  gen::AttnArgs a{q, k, v, o, key_mask, N, D, H, hd};
+                 int ld, float drop_p, uint64_t seed, uint32_t site, void* stream) {
+  if (!q || !k || !v || !o || N <= 0 || D < 1 || H < 1 || hd < 1 || ld < H * hd) return fail("gen_attn: bad arguments");
+  if (!(drop_p >= 0.0f && drop_p < 1.0f)) return fail("gen_attn: dropout p=%g outside [0, 1)", drop_p);
+  gen::AttnArgs a{q, k, v, o, key_mask, N, D, H, hd, ld, drop_p, seed, site};
   LaunchScope scope((cudaStream_t)stream, "gen_attn", (double)N * D * H * hd * 16.0, 0);
   gen::attn_kernel<<<ew_grid((long long)N * D * H, 128), 128, 0, (cudaStream_t)stream>>>(a);
   W2S_LAUNCH_CHECK("gen_attn");
+}
+
+// ---- backward of the general path ----
+static bool gen_conv_shape_ok(int B, int L_in, int L_out, int cin, int cout, int taps, int stride, int dil) {
+  return B > 0 && B <= 65535 && L_in > 0 && L_out > 0 && cin >= 1 && cout >= 1 && taps >= 1 && stride >= 1 && dil >= 1;
+}
+int w2s_gen_conv_dgrad(const float* dout, const float* w, float* din, const uint8_t* row_mask, int B, int L_in, int L_out, int cin,
+                       int cout, int taps, int stride, int dil, int pad_left, int taps_major, void* stream) {
+  if (!dout || !w || !din || !gen_conv_shape_ok(B, L_in, L_out, cin, cout, taps, stride, dil))
+    return fail("gen_conv_dgrad: bad arguments (B=%d L_in=%d L_out=%d cin=%d cout=%d taps=%d)", B, L_in, L_out, cin, cout, taps);
+  gen::ConvBwdArgs a{nullptr, w, dout, din, nullptr, row_mask, B, L_in, L_out, cin, cout, taps, stride, dil, pad_left,
+                     taps_major, 0};
+  long long gx = ((long long)L_in * cin + 255) / 256;
+  const long long cap = 32LL * sm_count() / B + 1;
+  if (gx > cap) gx = cap;
+  LaunchScope scope((cudaStream_t)stream, "gen_conv_dgrad", 4.0 * B * ((double)L_out * cout + (double)L_in * cin),
+                    2.0 * B * (double)L_out * cout * cin * taps);
+  gen::conv_dgrad_kernel<<<dim3((unsigned)gx, B), 256, 0, (cudaStream_t)stream>>>(a);
+  W2S_LAUNCH_CHECK("gen_conv_dgrad");
+}
+int w2s_gen_conv_wgrad(const float* in, const float* dout, float* dw, float* dbias, double* ws, const uint8_t* row_mask, int B,
+                       int L_in, int L_out, int cin, int cout, int taps, int stride, int dil, int pad_left, int taps_major,
+                       int raw_inf_to_zero, void* stream) {
+  if (!in || !dout || !ws || (!dw && !dbias) || !gen_conv_shape_ok(B, L_in, L_out, cin, cout, taps, stride, dil))
+    return fail("gen_conv_wgrad: bad arguments (B=%d L_in=%d L_out=%d cin=%d cout=%d taps=%d)", B, L_in, L_out, cin, cout, taps);
+  const long long K = (long long)taps * cin * cout;
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(ws, 0, (size_t)(K + cout) * sizeof(double), st);
+  if (e != cudaSuccess) return cuda_fail(e, "gen_conv_wgrad memset");
+  gen::ConvBwdArgs a{in, nullptr, dout, nullptr, ws, row_mask, B, L_in, L_out, cin, cout, taps, stride, dil, pad_left, taps_major,
+                     raw_inf_to_zero};
+  const long long gx = (K + 31) / 32, tiles = ((long long)B * L_out + gen::kRedTile - 1) / gen::kRedTile;
+  // enough position tiles to fill the GPU ~8 blocks deep, each block walking several tiles (fewer fp64 atomics)
+  long long gy = (8LL * sm_count() + gx - 1) / gx;
+  if (gy > tiles) gy = tiles;
+  if (gy > 65535) gy = 65535;
+  if (gy < 1) gy = 1;
+  LaunchScope scope(st, "gen_conv_wgrad", 4.0 * B * ((double)L_out * cout + (double)L_in * cin),
+                    2.0 * B * (double)L_out * cout * cin * taps);
+  gen::conv_wgrad_kernel<<<dim3((unsigned)gx, (unsigned)gy), 256, 0, st>>>(a);
+  gen::conv_wgrad_finalize_kernel<<<ew_grid(K + cout), 256, 0, st>>>(a, dw, dbias);
+  W2S_LAUNCH_CHECK("gen_conv_wgrad");
+}
+int w2s_gen_affine_act_bwd(const float* in, const float* scale, const float* shift, const float* res, const float* dout, float* din,
+                           float* dpre, double* sums, const uint8_t* row_mask, int B, int L, int Cc, int act, int per_channel,
+                           void* stream) {
+  if (!in || !dout || B <= 0 || B > 65535 || L <= 0 || Cc < 1 || act < 0 || act > 4) return fail("gen_affine_act_bwd: bad arguments");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (sums) {
+    cudaError_t e = cudaMemsetAsync(sums, 0, (size_t)(per_channel ? 1 : B) * Cc * 2 * sizeof(double), st);
+    if (e != cudaSuccess) return cuda_fail(e, "gen_affine_act_bwd memset");
+  }
+  gen::AffineActBwdArgs a{in, scale, shift, res, dout, din, dpre, sums, row_mask, B, L, Cc, act, per_channel};
+  const long long gx = (Cc + 31) / 32, tiles = ((long long)L + gen::kRedTile - 1) / gen::kRedTile;
+  long long gy = (8LL * sm_count() + gx * B - 1) / (gx * B);
+  if (gy > tiles) gy = tiles;
+  if (gy > 65535) gy = 65535;
+  if (gy < 1) gy = 1;
+  LaunchScope scope(st, "gen_affine_act_bwd", (double)B * L * Cc * (4.0 * (2 + (res != nullptr) + (din != nullptr) + (dpre != nullptr))), 0);
+  gen::affine_act_bwd_kernel<<<dim3((unsigned)gx, (unsigned)gy, B), 256, 0, st>>>(a);
+  W2S_LAUNCH_CHECK("gen_affine_act_bwd");
+}
+int w2s_gen_norm_bwd(const float* x, const float* dpre, const double* stats, const double* sums, const float* weight, float* coef,
+                     float* dx, float* dweight, float* dbias, const uint8_t* row_mask, int B, int L, int Cc, int groups, float eps,
+                     void* stream) {
+  if (!x || !dpre || !stats || !sums || !coef || !dx || B <= 0 || B > 65535 || L <= 0 || Cc < 1 || groups < 1 || Cc % groups)
+    return fail("gen_norm_bwd: bad arguments (B=%d L=%d C=%d groups=%d)", B, L, Cc, groups);
+  cudaStream_t st = (cudaStream_t)stream;
+  gen::NormBwdArgs a{stats, sums, weight, row_mask, coef, dweight, dbias, B, Cc, L, groups, eps};
+  LaunchScope scope(st, "gen_norm_bwd", (double)B * L * Cc * 12.0, 0);
+  gen::norm_bwd_coef_kernel<<<ew_grid(Cc), 256, 0, st>>>(a);
+  long long gx = ((long long)L * Cc + 255) / 256;
+  const long long cap = 32LL * sm_count() / B + 1;
+  if (gx > cap) gx = cap;
+  gen::norm_bwd_apply_kernel<<<dim3((unsigned)gx, B), 256, 0, st>>>(x, dpre, coef, dx, row_mask, L, Cc);
+  W2S_LAUNCH_CHECK("gen_norm_bwd");
+}
+int w2s_gen_rownorm_bwd(const float* x, const float* weight, const float* bias, const float* dout, float* dx, float* dweight,
+                        float* dbias, double* ws, long long rows, int Cc, int rms, int act, float eps, void* stream) {
+  if (!x || !dout || !dx || rows <= 0 || Cc < 1 || Cc > 2048 || act < 0 || act > 4 || ((dweight || dbias) && !ws))
+    return fail("gen_rownorm_bwd: bad arguments (rows=%lld C=%d)", rows, Cc);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (ws) {
+    cudaError_t e = cudaMemsetAsync(ws, 0, (size_t)2 * Cc * sizeof(double), st);
+    if (e != cudaSuccess) return cuda_fail(e, "gen_rownorm_bwd memset");
+  }
+  gen::RowNormBwdArgs a{x, weight, bias, dout, dx, ws, rows, Cc, rms, act, eps};
+  int gx = ew_grid(rows * 32);
+  if (gx > 2 * sm_count()) gx = 2 * sm_count();  // every block adds its 2 * C column partials once
+  LaunchScope scope(st, "gen_rownorm_bwd", (double)rows * Cc * 12.0, 0);
+  gen::rownorm_bwd_kernel<<<gx, 256, 2 * Cc * sizeof(double), st>>>(a);
+  if (ws) gen::rownorm_bwd_finalize_kernel<<<ew_grid(Cc), 256, 0, st>>>(ws, dweight, dbias, Cc);
+  W2S_LAUNCH_CHECK("gen_rownorm_bwd");
+}
+int w2s_gen_attn_bwd(const float* q, const float* k, const float* v, const float* dout, float* dq, float* dk, float* dv,
+                     const uint8_t* key_mask, int N, int D, int H, int hd, int ld, float drop_p, uint64_t seed, uint32_t site,
+                     void* stream) {
+  if (!q || !k || !v || !dout || !dq || !dk || !dv || N <= 0 || D < 1 || H < 1 || hd < 1 || ld < H * hd)
+    return fail("gen_attn_bwd: bad arguments");
+  if (!(drop_p >= 0.0f && drop_p < 1.0f)) return fail("gen_attn_bwd: dropout p=%g outside [0, 1)", drop_p);
+  gen::AttnBwdArgs a{q, k, v, dout, dq, dk, dv, key_mask, N, D, H, hd, ld, drop_p, seed, site};
+  LaunchScope scope((cudaStream_t)stream, "gen_attn_bwd", (double)N * D * H * hd * 28.0, 0);
+  gen::attn_bwd_kernel<<<ew_grid((long long)N * D * H, 128), 128, 0, (cudaStream_t)stream>>>(a);
+  W2S_LAUNCH_CHECK("gen_attn_bwd");
+}
+int w2s_gen_dropout(const float* x, float* out, uint8_t* mask_out, long long n, float p, uint64_t seed, uint32_t site,
+                    void* stream) {
+  if (n <= 0 || n > 0xffffffffLL) return fail("gen_dropout: n=%lld outside [1, 2^32)", n);
+  if (!(p >= 0.0f && p < 1.0f)) return fail("gen_dropout: p=%g outside [0, 1)", p);
+  if (mask_out == nullptr && (x == nullptr || out == nullptr)) return fail("gen_dropout: null pointer");
+  LaunchScope scope((cudaStream_t)stream, "gen_dropout", (double)n * (mask_out ? 1.0 : 8.0), 0);
+  gen::dropout_kernel<<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(x, out, mask_out, n, p, seed, site);
+  W2S_LAUNCH_CHECK("gen_dropout");
 }
 
 int w2s_set_conv_impl(int impl) {

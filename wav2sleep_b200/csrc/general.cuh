@@ -14,6 +14,7 @@
 // or one warp per row, fp64 statistics.  No tensor cores, nothing fused beyond norm + activation (+ residual).
 #pragma once
 #include "common.cuh"
+#include "train_kernels.cuh"  // drop_keep: the counter-based dropout decisions of w2s_dropout
 
 namespace w2s {
 namespace gen {
@@ -195,26 +196,29 @@ __global__ void __launch_bounds__(256) rownorm_kernel(const RowNormArgs p) {
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// multi-head attention over the D tokens of each epoch, any head count / head dim; q, k, v, o: [N, D, H * hd];
-// key_mask [N, D] (1 = masked key).  One thread per (epoch, head, query).
+// multi-head attention over the D tokens of each epoch, any head count / head dim; q, k, v: rows of ld floats
+// ([N, D, ld], head h at columns h * hd ..), o: [N, D, H * hd]; key_mask [N, D] (1 = masked key).  drop_p > 0: dropout
+// on the attention weights as nn.MultiheadAttention applies it in training, keep decision drop_keep(seed, site,
+// ((n * H + h) * D + query) * D + key).  One thread per (epoch, head, query).
 // ------------------------------------------------------------------------------------------------------------
 struct AttnArgs {
   const float* q; const float* k; const float* v; float* o; const uint8_t* key_mask;
-  int N, D, H, hd;
+  int N, D, H, hd, ld; float drop_p; unsigned long long seed; unsigned site;
 };
 __global__ void __launch_bounds__(128) attn_kernel(const AttnArgs p) {
   const long long total = (long long)p.N * p.H * p.D;
   const int F = p.H * p.hd;
   const float scale = rsqrtf((float)p.hd);
+  const float keep_scale = p.drop_p > 0.0f ? 1.0f / (1.0f - p.drop_p) : 1.0f;
   for (long long it = blockIdx.x * (long long)blockDim.x + threadIdx.x; it < total; it += (long long)gridDim.x * blockDim.x) {
     const int i = (int)(it % p.D);
     const int h = (int)((it / p.D) % p.H);
     const long long n = it / ((long long)p.D * p.H);
-    const float* qi = p.q + ((size_t)n * p.D + i) * F + h * p.hd;
+    const float* qi = p.q + ((size_t)n * p.D + i) * p.ld + h * p.hd;
     float mx = -INFINITY;
     for (int j = 0; j < p.D; ++j) {
       if (p.key_mask && p.key_mask[(size_t)n * p.D + j]) continue;
-      const float* kj = p.k + ((size_t)n * p.D + j) * F + h * p.hd;
+      const float* kj = p.k + ((size_t)n * p.D + j) * p.ld + h * p.hd;
       float d = 0.0f;
       for (int c = 0; c < p.hd; ++c) d = fmaf(qi[c], kj[c], d);
       mx = fmaxf(mx, d * scale);
@@ -224,13 +228,16 @@ __global__ void __launch_bounds__(128) attn_kernel(const AttnArgs p) {
     for (int c = 0; c < p.hd; ++c) oi[c] = 0.0f;
     for (int j = 0; j < p.D; ++j) {
       if (p.key_mask && p.key_mask[(size_t)n * p.D + j]) continue;
-      const float* kj = p.k + ((size_t)n * p.D + j) * F + h * p.hd;
-      const float* vj = p.v + ((size_t)n * p.D + j) * F + h * p.hd;
+      const float* kj = p.k + ((size_t)n * p.D + j) * p.ld + h * p.hd;
+      const float* vj = p.v + ((size_t)n * p.D + j) * p.ld + h * p.hd;
       float d = 0.0f;
       for (int c = 0; c < p.hd; ++c) d = fmaf(qi[c], kj[c], d);
       const float e = expf(d * scale - mx);
       den += e;
-      for (int c = 0; c < p.hd; ++c) oi[c] = fmaf(e, vj[c], oi[c]);
+      float ew = e;  // the softmax denominator takes every key; dropout only scales / zeroes the weighted values
+      if (p.drop_p > 0.0f)
+        ew = drop_keep(p.seed, p.site, (unsigned)(((n * p.H + h) * p.D + i) * p.D + j), p.drop_p) ? e * keep_scale : 0.0f;
+      for (int c = 0; c < p.hd; ++c) oi[c] = fmaf(ew, vj[c], oi[c]);
     }
     const float inv = 1.0f / den;
     for (int c = 0; c < p.hd; ++c) oi[c] *= inv;

@@ -10,9 +10,16 @@ What is restated, with the reference lines it follows (relative to /root/referen
   SequenceCNN / DilatedConvBlock  models/wav2sleep.py:379-390 ; models/blocks.py:115-126
 
 Tensors are fp32, channels-last ``[B, L, C]``; weights stay in their PyTorch layouts (no packing).  torch is used for
-allocation and pure data movement (views, stack, index) only - every FLOP is in ``libw2s_b200.so``.  Inference only:
-BatchNorm uses its running statistics, dropout is the identity (``model.eval()`` semantics); the training path exists
-for the default model family (training.py).
+allocation and pure data movement (views, stack, index) only - every FLOP is in ``libw2s_b200.so``, except that autograd
+sums the gradients of a tensor that feeds two branches (residuals).
+
+Inference (``forward``, under ``no_grad``): BatchNorm uses its running statistics, dropout is the identity.  Training
+(``forward_train``, what ``Wav2Sleep.forward`` calls under ``train()`` with grad): every primitive below is a
+``torch.autograd.Function`` whose backward runs the kernels of ``csrc/general_bwd.cuh``, and dropout is applied where
+the reference applies it (attention weights, the FF / dropout1 / dropout2 dropouts of each mixer layer,
+DilatedConvBlock.dropout) with counter-based masks: ``dropout_seed`` (None: drawn from torch's CPU generator per step)
+and the fixed site numbers of training.py; ``dropout_mask`` returns a site's keep decisions.  Train-mode BatchNorm is
+not built (model.py raises before getting here).
 """
 from __future__ import annotations
 
@@ -21,6 +28,7 @@ from torch import Tensor, nn
 
 from . import _lib
 from .engine import _stream
+from .training import _rank
 
 ACT = {"linear": 0, "relu": 1, "leaky": 2, "gelu": 3, "silu": 4, "swish": 4}
 NORM_INSTANCE, NORM_GROUP, NORM_BATCH = 0, 1, 2
@@ -34,47 +42,257 @@ def _p(t: Tensor | None):
     return None if t is None else t.data_ptr()
 
 
+def _g(t: Tensor) -> Tensor:
+    """An incoming gradient as the kernels read it (fp32, contiguous)."""
+    return t.to(torch.float32).contiguous()
+
+
+# Every primitive is a torch.autograd.Function: its forward runs the forward kernel, its backward the backward kernels of
+# csrc/general_bwd.cuh.  Under no_grad the same forward runs and nothing is saved, so inference and training share one
+# stage code (GeneralEngine.encode / epoch_mixer / dilated_blocks / _forward).  Parameters go in as they are (detached
+# inside the forward), so their gradients reach p.grad.
+class _Conv(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, w, bias, eng, L_out, stride, dil, pad_left, mask, taps_major, raw):
+        B, L_in, cin = x.shape
+        xd, wd = _f(x), _f(w)
+        if taps_major:
+            cout, taps = wd.shape[0], wd.shape[1] // cin
+        else:
+            cout, _, taps = wd.shape
+        out = torch.zeros(B, L_out, cout, dtype=torch.float32, device=x.device)
+        _lib.check(eng.lib.w2s_gen_conv(xd.data_ptr(), wd.data_ptr(), _p(_f(bias)), out.data_ptr(), _p(mask), B, L_in, L_out,
+                                        cin, cout, taps, stride, dil, pad_left, taps_major, raw, _stream()))
+        ctx.save_for_backward(xd, wd, mask)
+        ctx.eng, ctx.has_bias = eng, bias is not None
+        ctx.geo = (B, L_in, L_out, cin, cout, taps, stride, dil, pad_left, taps_major, raw)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        xd, wd, mask = ctx.saved_tensors
+        B, L_in, L_out, cin, cout, taps, stride, dil, pad_left, taps_major, raw = ctx.geo
+        lib, g = ctx.eng.lib, _g(g)
+        dx = dw = db = None
+        if ctx.needs_input_grad[0] and not raw:
+            dx = torch.zeros_like(xd)
+            _lib.check(lib.w2s_gen_conv_dgrad(g.data_ptr(), wd.data_ptr(), dx.data_ptr(), _p(mask), B, L_in, L_out, cin, cout,
+                                              taps, stride, dil, pad_left, taps_major, _stream()))
+        want_b = ctx.has_bias and ctx.needs_input_grad[2]
+        if ctx.needs_input_grad[1] or want_b:
+            ws = torch.empty(taps * cin * cout + cout, dtype=torch.float64, device=g.device)
+            dw = torch.empty_like(wd) if ctx.needs_input_grad[1] else None
+            db = torch.empty(cout, dtype=torch.float32, device=g.device) if want_b else None
+            _lib.check(lib.w2s_gen_conv_wgrad(xd.data_ptr(), g.data_ptr(), _p(dw), _p(db), ws.data_ptr(), _p(mask), B, L_in,
+                                              L_out, cin, cout, taps, stride, dil, pad_left, taps_major, raw, _stream()))
+        return dx, dw, db, None, None, None, None, None, None, None, None
+
+
+class _AffineAct(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, scale, shift, res, eng, act, mask, per_channel):
+        B, L, Cc = x.shape
+        xd, sc, sh, rs = _f(x), _f(scale), _f(shift), _f(res)
+        out = torch.zeros_like(xd)
+        _lib.check(eng.lib.w2s_gen_affine_act(xd.data_ptr(), _p(sc), _p(sh), _p(rs), out.data_ptr(), _p(mask), B, L, Cc,
+                                              ACT[act], per_channel, _stream()))
+        ctx.save_for_backward(xd, sc, sh, rs, mask)
+        ctx.eng, ctx.act, ctx.per_channel = eng, act, per_channel
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        xd, sc, sh, rs, mask = ctx.saved_tensors
+        B, L, Cc = xd.shape
+        need_x, need_sc, need_sh, need_res = ctx.needs_input_grad[:4]
+        g = _g(g)
+        din = torch.zeros_like(xd) if need_x else None
+        dpre = torch.zeros_like(xd) if need_res else None
+        sums = None
+        if need_sc or need_sh:
+            sums = torch.empty(1 if ctx.per_channel else B, Cc, 2, dtype=torch.float64, device=g.device)
+        _lib.check(ctx.eng.lib.w2s_gen_affine_act_bwd(xd.data_ptr(), _p(sc), _p(sh), _p(rs), g.data_ptr(), _p(din), _p(dpre),
+                                                      _p(sums), _p(mask), B, L, Cc, ACT[ctx.act], ctx.per_channel, _stream()))
+        dsc = sums[..., 1].to(torch.float32).view(sc.shape) if need_sc else None
+        dsh = sums[..., 0].to(torch.float32).view(sh.shape) if need_sh else None
+        return din, dsc, dsh, dpre, None, None, None, None
+
+
+class _NormAct(torch.autograd.Function):
+    """InstanceNorm1d / GroupNorm (statistics over L, or L x channels of a group) + activation of a conv output."""
+
+    @staticmethod
+    def forward(ctx, y, weight, bias, eng, groups, mode, eps, act, mask):
+        B, L, Cc = y.shape
+        lib, dev = eng.lib, y.device
+        yd, w, b = _f(y), _f(weight), _f(bias)
+        stats = torch.zeros(B, Cc, 2, dtype=torch.float64, device=dev)
+        _lib.check(lib.w2s_gen_stats(yd.data_ptr(), stats.data_ptr(), _p(mask), B, L, Cc, _stream()))
+        scale = torch.zeros(B, Cc, dtype=torch.float32, device=dev)
+        shift = torch.zeros(B, Cc, dtype=torch.float32, device=dev)
+        _lib.check(lib.w2s_gen_norm_consts(stats.data_ptr(), _p(w), _p(b), None, None, scale.data_ptr(), shift.data_ptr(), B,
+                                           Cc, L, mode, groups, eps, _stream()))
+        out = torch.zeros_like(yd)
+        _lib.check(lib.w2s_gen_affine_act(yd.data_ptr(), scale.data_ptr(), shift.data_ptr(), None, out.data_ptr(), _p(mask),
+                                          B, L, Cc, ACT[act], 0, _stream()))
+        ctx.save_for_backward(yd, w, stats, scale, shift, mask)
+        ctx.eng, ctx.groups, ctx.eps, ctx.act = eng, groups if mode == NORM_GROUP else Cc, eps, act
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        yd, w, stats, scale, shift, mask = ctx.saved_tensors
+        B, L, Cc = yd.shape
+        lib, g, dev = ctx.eng.lib, _g(g), g.device
+        dpre = torch.zeros_like(yd)
+        sums = torch.empty(B, Cc, 2, dtype=torch.float64, device=dev)
+        _lib.check(lib.w2s_gen_affine_act_bwd(yd.data_ptr(), scale.data_ptr(), shift.data_ptr(), None, g.data_ptr(), None,
+                                              dpre.data_ptr(), sums.data_ptr(), _p(mask), B, L, Cc, ACT[ctx.act], 0, _stream()))
+        coef = torch.empty(B, Cc, 3, dtype=torch.float32, device=dev)
+        dy = torch.zeros_like(yd)
+        dw = torch.empty(Cc, dtype=torch.float32, device=dev) if ctx.needs_input_grad[1] else None
+        db = torch.empty(Cc, dtype=torch.float32, device=dev) if ctx.needs_input_grad[2] else None
+        _lib.check(lib.w2s_gen_norm_bwd(yd.data_ptr(), dpre.data_ptr(), stats.data_ptr(), sums.data_ptr(), _p(w),
+                                        coef.data_ptr(), dy.data_ptr(), _p(dw), _p(db), _p(mask), B, L, Cc, ctx.groups, ctx.eps,
+                                        _stream()))
+        return dy, dw, db, None, None, None, None, None, None
+
+
+class _RowNorm(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, weight, bias, eng, eps, act, rms):
+        Cc = x.shape[-1]
+        rows = x.numel() // Cc
+        xd, w, b = _f(x), _f(weight), _f(bias)
+        out = torch.empty_like(xd)
+        _lib.check(eng.lib.w2s_gen_rownorm(xd.data_ptr(), _p(w), _p(b), out.data_ptr(), rows, Cc, rms, ACT[act], eps,
+                                           _stream()))
+        ctx.save_for_backward(xd, w, b)
+        ctx.eng, ctx.eps, ctx.act, ctx.rms = eng, eps, act, rms
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        xd, w, b = ctx.saved_tensors
+        Cc = xd.shape[-1]
+        rows, g, dev = xd.numel() // Cc, _g(g), g.device
+        dx = torch.empty_like(xd)
+        dw = torch.empty(Cc, dtype=torch.float32, device=dev) if (w is not None and ctx.needs_input_grad[1]) else None
+        db = torch.empty(Cc, dtype=torch.float32, device=dev) if (b is not None and ctx.needs_input_grad[2]) else None
+        ws = torch.empty(2 * Cc, dtype=torch.float64, device=dev) if (dw is not None or db is not None) else None
+        _lib.check(ctx.eng.lib.w2s_gen_rownorm_bwd(xd.data_ptr(), _p(w), _p(b), g.data_ptr(), dx.data_ptr(), _p(dw), _p(db),
+                                                   _p(ws), rows, Cc, ctx.rms, ACT[ctx.act], ctx.eps, _stream()))
+        return dx, dw, db, None, None, None, None
+
+
+class _Attn(torch.autograd.Function):
+    """Attention of the fused in-projection output qkv [N * D, 3F] (q, k, v = column thirds) -> o [N * D, F]."""
+
+    @staticmethod
+    def forward(ctx, qkv, eng, km, N, D, H, p, seed, site):
+        qkv = _f(qkv)
+        F3 = qkv.shape[1]
+        Fd = F3 // 3
+        o = torch.empty(qkv.shape[0], Fd, dtype=torch.float32, device=qkv.device)
+        q = qkv.data_ptr()
+        _lib.check(eng.lib.w2s_gen_attn(q, q + 4 * Fd, q + 8 * Fd, o.data_ptr(), km.data_ptr(), N, D, H, Fd // H, F3, p, seed,
+                                        site, _stream()))
+        ctx.save_for_backward(qkv, km)
+        ctx.eng, ctx.cfg = eng, (N, D, H, p, seed, site)
+        return o
+
+    @staticmethod
+    def backward(ctx, g):
+        qkv, km = ctx.saved_tensors
+        N, D, H, p, seed, site = ctx.cfg
+        F3 = qkv.shape[1]
+        Fd = F3 // 3
+        g = _g(g)
+        d = torch.empty_like(qkv)
+        q, dq = qkv.data_ptr(), d.data_ptr()
+        _lib.check(ctx.eng.lib.w2s_gen_attn_bwd(q, q + 4 * Fd, q + 8 * Fd, g.data_ptr(), dq, dq + 4 * Fd, dq + 8 * Fd,
+                                                km.data_ptr(), N, D, H, Fd // H, F3, p, seed, site, _stream()))
+        return d, None, None, None, None, None, None, None, None
+
+
+class _Dropout(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, eng, p, seed, site):
+        xd = _f(x)
+        out = torch.empty_like(xd)
+        _lib.check(eng.lib.w2s_gen_dropout(xd.data_ptr(), out.data_ptr(), None, xd.numel(), p, seed, site, _stream()))
+        ctx.eng, ctx.cfg = eng, (p, seed, site)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        p, seed, site = ctx.cfg
+        g = _g(g)
+        dx = torch.empty_like(g)
+        _lib.check(ctx.eng.lib.w2s_gen_dropout(g.data_ptr(), dx.data_ptr(), None, g.numel(), p, seed, site, _stream()))
+        return dx, None, None, None, None
+
+
+class _Broadcast(torch.autograd.Function):
+    """A [F] parameter row repeated over n rows (register / CLS tokens); the backward is its column sum."""
+
+    @staticmethod
+    def forward(ctx, row, eng, n):
+        rd = _f(row)
+        ctx.eng = eng
+        return torch.empty(n, rd.shape[0], dtype=torch.float32, device=rd.device).copy_(rd)
+
+    @staticmethod
+    def backward(ctx, g):
+        g = _g(g)
+        n, Fd = g.shape
+        sums = torch.empty(1, Fd, 2, dtype=torch.float64, device=g.device)
+        # the per-channel sums of a linear affine_act backward: sums[c, 0] = sum over rows of g
+        _lib.check(ctx.eng.lib.w2s_gen_affine_act_bwd(g.data_ptr(), None, None, None, g.data_ptr(), None, None,
+                                                      sums.data_ptr(), None, 1, n, Fd, ACT["linear"], 1, _stream()))
+        return sums[0, :, 0].to(torch.float32), None, None
+
+
 class GeneralEngine:
     def __init__(self, model):
         self.model = model
         self.lib = _lib.load()
+        self.dropout_seed = None  # int: fixed seed for every training step (tests); None: drawn from torch's CPU generator
+        self.last_dropout_seed = 0
+        self._seed = None         # the current training forward's seed; None = no dropout (eval, or no_grad)
 
     # ------------------------------------------------------------------ kernel wrappers
     def conv(self, x: Tensor, w: Tensor, bias, L_out: int, stride=1, dil=1, pad_left=0, mask=None, taps_major=0, raw=0):
         """x [B, L_in, cin] -> [B, L_out, cout]; w [cout, cin, taps] (taps_major: [cout, taps * cin] with taps given by
         the caller through w.shape[1] // cin)."""
-        B, L_in, cin = x.shape
-        w = _f(w)
-        if taps_major:
-            cout, taps = w.shape[0], w.shape[1] // cin
-        else:
-            cout, _, taps = w.shape
-        out = torch.zeros(B, L_out, cout, dtype=torch.float32, device=x.device)
-        _lib.check(self.lib.w2s_gen_conv(x.data_ptr(), w.data_ptr(), _p(_f(bias)), out.data_ptr(), _p(mask), B, L_in, L_out,
-                                         cin, cout, taps, stride, dil, pad_left, taps_major, raw, _stream()))
-        return out
+        return _Conv.apply(x, w, bias, self, L_out, stride, dil, pad_left, mask, taps_major, raw)
 
     def linear(self, x: Tensor, lin: nn.Linear | None = None, weight=None, bias=None) -> Tensor:
         """rows [R, K] -> [R, N] = x W^T + b (a 1-tap conv over R positions)."""
         if lin is not None:
             weight, bias = lin.weight, lin.bias
         R, K = x.shape
-        return self.conv(x.view(1, R, K), _f(weight).unsqueeze(-1), bias, R).view(R, -1)
+        return self.conv(x.reshape(1, R, K), weight.unsqueeze(-1), bias, R).view(R, -1)
 
     def affine_act(self, x: Tensor, act: str, scale=None, shift=None, res=None, mask=None, per_channel=0) -> Tensor:
-        B, L, Cc = x.shape
-        out = torch.zeros_like(x)
-        _lib.check(self.lib.w2s_gen_affine_act(x.data_ptr(), _p(scale), _p(shift), _p(res), out.data_ptr(), _p(mask), B, L,
-                                               Cc, ACT[act], per_channel, _stream()))
-        return out
+        return _AffineAct.apply(x, scale, shift, res, self, act, mask, per_channel)
 
     def rownorm(self, x: Tensor, weight, bias, eps: float, act: str = "linear", rms: int = 0) -> Tensor:
-        Cc = x.shape[-1]
-        rows = x.numel() // Cc
-        out = torch.empty_like(x)
-        _lib.check(self.lib.w2s_gen_rownorm(x.data_ptr(), _p(_f(weight)), _p(_f(bias)), out.data_ptr(), rows, Cc, rms,
-                                            ACT[act], eps, _stream()))
-        return out
+        return _RowNorm.apply(x, weight, bias, self, eps, act, rms)
+
+    def dropout(self, x: Tensor, p: float, site: int) -> Tensor:
+        """nn.Dropout(p) of a training forward (identity otherwise): the counter-based masks of w2s_gen_dropout."""
+        if self._seed is None or p <= 0:
+            return x
+        return _Dropout.apply(x, self, float(p), self._seed, site)
+
+    def dropout_mask(self, n: int, site: int, p: float, seed: int, device) -> Tensor:
+        """The keep decisions (uint8 0/1) of the first n elements of a dropout site (test hook).  For the attention
+        weights of a mixer layer the element index is ((epoch * H + head) * D + query) * D + key."""
+        m = torch.empty(n, dtype=torch.uint8, device=device)
+        with torch.cuda.device(device):
+            _lib.check(self.lib.w2s_gen_dropout(None, None, m.data_ptr(), n, p, seed, site, _stream()))
+        return m
 
     def norm_act(self, y: Tensor, layer, act: str, mask=None, res=None) -> Tensor:
         """norm (by the layer's kind) -> activation of a conv output y [B, L, C]   (ConvLayer1D.forward, blocks.py:183-185)."""
@@ -87,30 +305,21 @@ class GeneralEngine:
             b = norm.bias.reshape(-1) if kind == "layer" else None
             return self.rownorm(y, w, b, norm.eps, act, rms=int(kind == "rms"))
         dev = y.device
-        if kind == "batch":  # eval mode: running statistics
+        if kind == "batch":  # eval mode: running statistics (train-mode BatchNorm is not built, see model.py)
             scale = torch.empty(1, Cc, dtype=torch.float32, device=dev)
             shift = torch.empty(1, Cc, dtype=torch.float32, device=dev)
             _lib.check(self.lib.w2s_gen_norm_consts(None, _p(_f(norm.weight)), _p(_f(norm.bias)), _f(norm.running_mean).data_ptr(),
                                                     _f(norm.running_var).data_ptr(), scale.data_ptr(), shift.data_ptr(), 1, Cc, L,
                                                     NORM_BATCH, 1, norm.eps, _stream()))
             return self.affine_act(y, act, scale, shift, mask=mask, per_channel=1)
-        stats = torch.zeros(B, Cc, 2, dtype=torch.float64, device=dev)
-        _lib.check(self.lib.w2s_gen_stats(y.data_ptr(), stats.data_ptr(), _p(mask), B, L, Cc, _stream()))
-        scale = torch.zeros(B, Cc, dtype=torch.float32, device=dev)
-        shift = torch.zeros(B, Cc, dtype=torch.float32, device=dev)
         if kind == "instance":
-            w = _f(norm.weight) if getattr(norm, "affine", False) else None
-            b = _f(norm.bias) if getattr(norm, "affine", False) else None
-            _lib.check(self.lib.w2s_gen_norm_consts(stats.data_ptr(), _p(w), _p(b), None, None, scale.data_ptr(),
-                                                    shift.data_ptr(), B, Cc, L, NORM_INSTANCE, 1, norm.eps, _stream()))
-        elif kind == "group":
+            affine = getattr(norm, "affine", False)
+            return _NormAct.apply(y, norm.weight if affine else None, norm.bias if affine else None, self, 1, NORM_INSTANCE,
+                                  norm.eps, act, mask)
+        if kind == "group":
             gn = norm.norm
-            _lib.check(self.lib.w2s_gen_norm_consts(stats.data_ptr(), _p(_f(gn.weight)), _p(_f(gn.bias)), None, None,
-                                                    scale.data_ptr(), shift.data_ptr(), B, Cc, L, NORM_GROUP, gn.num_groups,
-                                                    gn.eps, _stream()))
-        else:
-            raise NotImplementedError(f"norm {kind!r}")
-        return self.affine_act(y, act, scale, shift, mask=mask)
+            return _NormAct.apply(y, gn.weight, gn.bias, self, gn.num_groups, NORM_GROUP, gn.eps, act, mask)
+        raise NotImplementedError(f"norm {kind!r}")
 
     def conv_layer(self, a: Tensor, layer, mask=None, raw=0) -> Tensor:
         """ConvLayer1D.forward (blocks.py:173-186) on a [B, L, Cin] input."""
@@ -132,13 +341,13 @@ class GeneralEngine:
         return self.affine_act(y, blk.activation_name, res=r, mask=mask)
 
     def dilated_blocks(self, x_BSF: Tensor, blocks) -> Tensor:
-        """Sequential(DilatedConvBlock) in eval mode (blocks.py:115-126)."""
+        """Sequential(DilatedConvBlock) (blocks.py:115-126): act(dropout(layers(x)) + x)."""
         cur = x_BSF
-        for blk in blocks:
+        for bi, blk in enumerate(blocks):
             blk_in = cur
             for layer in blk.conv_layers:
                 cur = self.conv_layer(cur, layer)
-            cur = self.affine_act(cur, blk.activation_name, res=blk_in)
+            cur = self.affine_act(self.dropout(cur, blk.dropout.p, 64 + bi), blk.activation_name, res=blk_in)
         return cur
 
     # ------------------------------------------------------------------ stages
@@ -177,28 +386,27 @@ class GeneralEngine:
         N, dev = B * S, zs[0].device
         if zs[0].shape[-1] != Fd:
             raise ValueError(f"Feature dimension {zs[0].shape[-1]} does not match self.feature_dim={Fd}.")
-        reg = _f(mix.register_tokens[0, 0]).t().contiguous()  # [R + 1, F]; token 0 is the CLS token
-        toks = [reg[i].expand(B, S, Fd) for i in range(R + 1)]
+        reg = mix.register_tokens[0, 0].t()  # [R + 1, F]; token 0 is the CLS token
+        toks = [_Broadcast.apply(reg[i], self, N).view(B, S, Fd) for i in range(R + 1)]
         toks += [torch.where(m.bool()[:, None, None], torch.zeros_like(z), z) for z, m in zip(zs, masks)]
         D = len(toks)
-        x = torch.stack(toks, dim=2).reshape(N * D, Fd).contiguous()
+        x = torch.stack(toks, dim=2).reshape(N * D, Fd)
         km = torch.stack([torch.zeros_like(masks[0])] * (R + 1) + masks, dim=1)[:, None, :].expand(B, S, D)
         km = km.reshape(N * D).contiguous()
         H = mix.nhead
         act = mix.activation_name
-        for layer in mix.transformer_encoder.layers:
+        # dropout sites (as in training.py): 8 * layer + {0 attention weights, 1 dropout1, 2 FF dropout, 3 dropout2}
+        for li, layer in enumerate(mix.transformer_encoder.layers):
             def sa(h):
-                Win, bin_ = _f(layer.self_attn.in_proj_weight), _f(layer.self_attn.in_proj_bias)
-                q, k, v = (self.linear(h, weight=Win[j * Fd:(j + 1) * Fd].contiguous(), bias=bin_[j * Fd:(j + 1) * Fd].contiguous())
-                           for j in range(3))
-                o = torch.empty_like(q)
-                _lib.check(self.lib.w2s_gen_attn(q.data_ptr(), k.data_ptr(), v.data_ptr(), o.data_ptr(), km.data_ptr(), N, D, H,
-                                                 Fd // H, _stream()))
-                return self.linear(o, layer.self_attn.out_proj)
+                qkv = self.linear(h, weight=layer.self_attn.in_proj_weight, bias=layer.self_attn.in_proj_bias)  # [R, 3F]
+                p = layer.self_attn.dropout if self._seed is not None else 0.0
+                o = _Attn.apply(qkv, self, km, N, D, H, float(p), self._seed or 0, 8 * li)
+                return self.dropout(self.linear(o, layer.self_attn.out_proj), layer.dropout1.p, 8 * li + 1)
 
             def ff(h):
                 hid = self.affine_act(self.linear(h, layer.linear1).unsqueeze(0), act).squeeze(0)
-                return self.linear(hid, layer.linear2)
+                hid = self.dropout(hid, layer.dropout.p, 8 * li + 2)
+                return self.dropout(self.linear(hid, layer.linear2), layer.dropout2.p, 8 * li + 3)
 
             add = lambda a, b: self.affine_act(a.unsqueeze(0), "linear", res=b.unsqueeze(0)).squeeze(0)
             ln = lambda t, nrm: self.rownorm(t, nrm.weight, nrm.bias, nrm.eps)
@@ -211,12 +419,30 @@ class GeneralEngine:
         return x.view(N, D, Fd)[:, 0, :].contiguous().view(B, S, Fd)
 
     def sequence_mixer(self, x_BSF: Tensor) -> Tensor:
-        """SequenceCNN.forward (wav2sleep.py:379-390) + DilatedConvBlock.forward (blocks.py:115-126), eval mode."""
+        """SequenceCNN.forward (wav2sleep.py:379-390) + DilatedConvBlock.forward (blocks.py:115-126)."""
         return self.dilated_blocks(x_BSF, self.model.sequence_mixer.dilated_convs)
 
     # ------------------------------------------------------------------ model
     @torch.no_grad()
     def forward(self, x: dict[str, Tensor]) -> Tensor:
+        """Inference (eval semantics: running BatchNorm statistics, no dropout)."""
+        self._seed = None
+        return self._forward(x)
+
+    def forward_train(self, x: dict[str, Tensor]) -> Tensor:
+        """Training forward: builds the autograd graph whose backward runs the kernels of csrc/general_bwd.cuh, with
+        dropout at every site the reference applies it in training (masks drawn from ``dropout_seed``)."""
+        if self.dropout_seed is not None:
+            seed = int(self.dropout_seed)
+        else:
+            seed = int(torch.randint(0, 2 ** 62, (1,)).item()) ^ (0x5851F42D4C957F2D * (1 + _rank()) & (2 ** 62 - 1))
+        self.last_dropout_seed = self._seed = seed
+        try:
+            return self._forward(x)
+        finally:
+            self._seed = None
+
+    def _forward(self, x: dict[str, Tensor]) -> Tensor:
         m = self.model
         if not isinstance(x, dict) or len(x) == 0:
             raise ValueError("No signals provided to MultiModalAttentionEmbedder.")
@@ -242,7 +468,7 @@ class GeneralEngine:
                 elif (z.shape[0], z.shape[1]) != (B, S):
                     raise ValueError(f"{n}: batch/epoch count {tuple(z.shape[:2])} differs from {(B, S)}")
                 if m.signal_encoders.embed_signals:  # wav2sleep.py:155-159
-                    e = _f(m.signal_encoders.embedder.weight[m.signal_encoders.sig_to_embedding_idx[n]])
+                    e = m.signal_encoders.embedder.weight[m.signal_encoders.sig_to_embedding_idx[n]]
                     z = self.affine_act(z, "linear", shift=e, mask=mask, per_channel=1)
                 zs.append(z)
                 masks.append(mask)

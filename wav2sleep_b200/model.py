@@ -17,8 +17,11 @@ kernel 7) runs on the fused tcgen05 kernels (engine.py / training.py).  Every ot
 accept (SURVEY.md section 8f, row N3: causal / chunk-causal mode, norms batch / layer / rms / group / auto / none,
 activations relu / leaky / silu / linear, ``embed_signals``, ``register_tokens > 0``, ``output_norm``,
 ``use_residual=False``, other widths and feature dims) runs on the dimension-generic fp32 kernels of csrc/general.cuh
-(general.py): inference only, same results as the reference to fp32 accuracy, not tuned.  ``norm='weight'`` (a
-parametrisation with different state_dict keys) is the one option that raises ``NotImplementedError``.
+(general.py): inference and training (an autograd graph over fp32 forward / backward kernels, dropout included), same
+results as the reference to fp32 accuracy, not tuned.  ``norm='weight'`` (a parametrisation with different state_dict
+keys) is the one option that raises ``NotImplementedError``; a model with BatchNorm layers (norm='batch', SleepPPGNet)
+runs inference but raises ``NotImplementedError`` under ``train()`` with grad (train-mode batch statistics are not
+built).
 """
 from __future__ import annotations
 
@@ -370,12 +373,15 @@ class Wav2Sleep(nn.Module):
         """dict of [B, S * samples_per_epoch] fp32 (rows of -inf = missing signal) -> logits [B, S, num_classes].
 
         Under ``train()`` with grad enabled the logits carry a grad_fn whose backward runs the CUDA backward pass
-        (dropout with counter-based masks, see training.py); otherwise the fused inference kernels run."""
+        (dropout with counter-based masks, see training.py; for the non-default options the general path's autograd
+        Functions, general.py); otherwise the inference kernels run."""
         if not self.fast_path:
             if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
-                raise NotImplementedError("wav2sleep_b200: training is built for the default model family only; "
-                                          "non-default options (causal, other norms / activations / widths) run the "
-                                          "general inference kernels")
+                if any(isinstance(mod, nn.BatchNorm1d) for mod in self.modules()):
+                    raise NotImplementedError("wav2sleep_b200: training a model with BatchNorm layers (train-mode batch "
+                                              "statistics and running-statistics updates) is not built on the CUDA path; "
+                                              "eval-mode inference is")
+                return self._get_general().forward_train(x)
             return self._get_general().forward(x)
         if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             from .training import forward_with_grad

@@ -330,8 +330,8 @@ class SleepLightningModule(nn.Module):
                 if self._opt.ema is not None:
                     dist.broadcast(self._opt.ema, src=0, group=process_group)
                 self._opt._bump()
-            eng = self.model._get_train_engine()
-            eng.bucket_hooks = [self._reducer]
+            if getattr(self.model, "fast_path", False):
+                self.model._get_train_engine().bucket_hooks = [self._reducer]
 
     def fit_step(self, batch) -> Tensor:
         """One optimisation step: transforms -> forward -> loss -> backward (+ overlapped all-reduce) -> clip + AdamW."""
@@ -343,6 +343,10 @@ class SleepLightningModule(nn.Module):
         loss = self.training_step(batch)
         loss.backward()
         if self._reducer is not None:
+            if not getattr(self.model, "fast_path", False):
+                # the general path's backward is plain autograd and fires no bucket hooks: every gradient is final now
+                for name in self._reducer.segments:
+                    self._reducer(name)
             self._reducer.wait()
         self._opt.step()
         if self._sched is not None:
