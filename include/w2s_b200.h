@@ -426,6 +426,51 @@ int w2s_gen_dropout(const float* x, float* out, uint8_t* mask_out, long long n, 
                     void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
+ * Streaming step of a causal sequence mixer (ABI v6; wav2sleep_b200/streaming.py).  Every DilatedConvBlock of a causal
+ * SequenceCNN (models/blocks.py:115-126, ConvLayer1D causal :150-152, :178-182) and the classifier, for R new epochs of
+ * N streams, in eval semantics (running BatchNorm statistics, no dropout), fp32.  The history of each dilated layer is a
+ * ring in `ring`: layer l = b * n_dilations + j (dilation 2^j) keeps M_l = (k-1) * 2^j input rows of F floats per stream;
+ * the row of epoch e is in slot e mod M_l.  A stream's state is n_blocks * (k-1) * (2^n_dilations - 1) rows of F floats,
+ * its layers' rings one after the other: ring[n, off_l + slot, :] with off_l = sum of M over the layers before l.  Zero
+ * rows are the causal zero padding, so a stream restarts when the caller zeroes its rows.  Parameters are read in place.
+ * ------------------------------------------------------------------------------------------------------- */
+#define W2S_STREAM_MAX_LAYERS 32     /* n_blocks * n_dilations */
+#define W2S_STREAM_MAX_DILATIONS 16
+#define W2S_STREAM_MAX_KERNEL 16
+#define W2S_STREAM_MAX_FEATURES 256
+enum { W2S_SEQ_NORM_NONE = 0, W2S_SEQ_NORM_BATCH = 1, W2S_SEQ_NORM_LAYER = 2, W2S_SEQ_NORM_RMS = 3 };
+
+typedef struct w2s_gen_seq_stream_layer {
+  const float* w;             /* conv.weight [F, F, k] */
+  const float* bias;          /* conv.bias [F] or NULL (ConvLayer1D has one only without a norm) */
+  const float* norm_w;        /* norm weight [F] or NULL (= 1) */
+  const float* norm_b;        /* norm bias [F] or NULL (= 0) */
+  const float* running_mean;  /* W2S_SEQ_NORM_BATCH: running statistics [F] */
+  const float* running_var;
+} w2s_gen_seq_stream_layer;
+
+typedef struct w2s_gen_seq_stream_desc {
+  int32_t n_blocks;      /* num_layers */
+  int32_t n_dilations;   /* dilations 1, 2, .., 2^(n_dilations-1) */
+  int32_t kernel_size;
+  int32_t feature_dim;   /* F */
+  int32_t n_classes;
+  int32_t norm;          /* W2S_SEQ_NORM_* */
+  int32_t act;           /* W2S_ACT_* */
+  float eps;             /* of the norm */
+  w2s_gen_seq_stream_layer layer[W2S_STREAM_MAX_LAYERS];
+  const float* head_w;   /* classifier.weight [n_classes, F] */
+  const float* head_b;   /* classifier.bias [n_classes] */
+  float* ring;           /* [N, n_blocks * (k-1) * (2^n_dilations - 1), F], read and written */
+} w2s_gen_seq_stream_desc;
+
+/* x_new: [N, R, F] epoch-mixer features of epochs pos .. pos+R-1 -> logits [N, R, n_classes]; one launch, epochs in
+ * order.  Limits: F <= W2S_STREAM_MAX_FEATURES, 1 <= kernel_size <= W2S_STREAM_MAX_KERNEL, n_dilations <=
+ * W2S_STREAM_MAX_DILATIONS, n_blocks * n_dilations <= W2S_STREAM_MAX_LAYERS. */
+int w2s_gen_seq_stream_step(const w2s_gen_seq_stream_desc* d, const float* x_new, float* logits, int N, int R, long long pos,
+                            void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------
  * Measurement hooks (bench.py).  Not part of the data path.
  * ------------------------------------------------------------------------------------------------------- */
 /* Number of kernels this library has launched in this process (monotonic). */

@@ -23,7 +23,11 @@ MAX_MIXER_LAYERS = 8
 MAX_SIGNALS = 4
 MAX_SEQ_BLOCKS = 4
 MAX_DILATIONS = 8
-ABI_VERSION = 5
+STREAM_MAX_LAYERS = 32
+STREAM_MAX_DILATIONS = 16
+STREAM_MAX_KERNEL = 16
+STREAM_MAX_FEATURES = 256
+ABI_VERSION = 6
 
 PRO_NONE, PRO_NORM, PRO_NORM_RES, PRO_FIR, PRO_NORM_RES_X, PRO_DNORM = 0, 1, 2, 3, 4, 5
 EPI_STATS, EPI_BIAS_GELU, EPI_LN_GELU, EPI_LN_GELU_RES, EPI_PLAIN, EPI_ACT_BWD = 0, 1, 2, 3, 4, 5
@@ -118,6 +122,18 @@ class SeqDesc(C.Structure):
     ]
 
 
+class SeqStreamLayer(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("w", "bias", "norm_w", "norm_b", "running_mean", "running_var")]
+
+
+class SeqStreamDesc(C.Structure):
+    _fields_ = [
+        ("n_blocks", C.c_int32), ("n_dilations", C.c_int32), ("kernel_size", C.c_int32), ("feature_dim", C.c_int32),
+        ("n_classes", C.c_int32), ("norm", C.c_int32), ("act", C.c_int32), ("eps", C.c_float),
+        ("layer", SeqStreamLayer * STREAM_MAX_LAYERS), ("head_w", C.c_void_p), ("head_b", C.c_void_p), ("ring", C.c_void_p),
+    ]
+
+
 # name -> (restype, argtypes); every symbol declared in include/w2s_b200.h
 SYMBOLS = {
     "w2s_abi_version": (C.c_int, []),
@@ -191,6 +207,8 @@ SYMBOLS = {
     "w2s_gen_rownorm_bwd": (C.c_int, [C.c_void_p] * 8 + [C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p]),
     "w2s_gen_attn_bwd": (C.c_int, [C.c_void_p] * 8 + [C.c_int] * 5 + [C.c_float, C.c_uint64, C.c_uint32, C.c_void_p]),
     "w2s_gen_dropout": (C.c_int, [C.c_void_p] * 3 + [C.c_longlong, C.c_float, C.c_uint64, C.c_uint32, C.c_void_p]),
+    "w2s_gen_seq_stream_step": (C.c_int, [C.POINTER(SeqStreamDesc), C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong,
+                                          C.c_void_p]),
     "w2s_launch_count": (C.c_longlong, []),
     "w2s_profile_enable": (C.c_int, [C.c_int]),
     "w2s_profile_count": (C.c_int, []),

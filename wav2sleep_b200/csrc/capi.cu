@@ -25,6 +25,7 @@
 #include "general_bwd.cuh"
 #include "staging.cuh"
 #include "seq_mixer.cuh"
+#include "stream.cuh"
 
 using namespace w2s;
 
@@ -507,7 +508,7 @@ int check_encoder_desc(const w2s_encoder_desc* d) {
 
 extern "C" {
 
-int w2s_abi_version(void) { return 5; }
+int w2s_abi_version(void) { return 6; }
 const char* w2s_last_error(void) { return g_err.c_str(); }
 
 int w2s_conv_uses_split(int cin, int cout) { return (cin <= 16 && cout <= 16) ? 1 : 0; }
@@ -1489,6 +1490,50 @@ int w2s_gen_dropout(const float* x, float* out, uint8_t* mask_out, long long n, 
   LaunchScope scope((cudaStream_t)stream, "gen_dropout", (double)n * (mask_out ? 1.0 : 8.0), 0);
   gen::dropout_kernel<<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(x, out, mask_out, n, p, seed, site);
   W2S_LAUNCH_CHECK("gen_dropout");
+}
+
+int w2s_gen_seq_stream_step(const w2s_gen_seq_stream_desc* d, const float* x_new, float* logits, int N, int R, long long pos,
+                            void* stream) {
+  if (!d || !x_new || !logits || N <= 0 || R <= 0 || pos < 0)
+    return fail("gen_seq_stream_step: bad arguments (N=%d R=%d pos=%lld)", N, R, pos);
+  const int F = d->feature_dim, k = d->kernel_size, nb = d->n_blocks, nd = d->n_dilations;
+  if (F < 1 || F > W2S_STREAM_MAX_FEATURES)
+    return fail("gen_seq_stream_step: feature_dim %d outside [1, W2S_STREAM_MAX_FEATURES = %d]", F, W2S_STREAM_MAX_FEATURES);
+  if (k < 1 || k > W2S_STREAM_MAX_KERNEL)
+    return fail("gen_seq_stream_step: kernel_size %d outside [1, W2S_STREAM_MAX_KERNEL = %d]", k, W2S_STREAM_MAX_KERNEL);
+  if (nd < 1 || nd > W2S_STREAM_MAX_DILATIONS)
+    return fail("gen_seq_stream_step: n_dilations %d outside [1, W2S_STREAM_MAX_DILATIONS = %d]", nd, W2S_STREAM_MAX_DILATIONS);
+  if (nb < 1 || nb * nd > W2S_STREAM_MAX_LAYERS)
+    return fail("gen_seq_stream_step: n_blocks %d x n_dilations %d outside [1, W2S_STREAM_MAX_LAYERS = %d]", nb, nd,
+                W2S_STREAM_MAX_LAYERS);
+  if (d->n_classes < 1 || !d->head_w) return fail("gen_seq_stream_step: classifier missing (n_classes=%d)", d->n_classes);
+  if (d->norm < W2S_SEQ_NORM_NONE || d->norm > W2S_SEQ_NORM_RMS || d->act < 0 || d->act > 4)
+    return fail("gen_seq_stream_step: norm %d / act %d unknown", d->norm, d->act);
+  if (k > 1 && !d->ring) return fail("gen_seq_stream_step: ring state missing");
+  for (int l = 0; l < nb * nd; ++l) {
+    const w2s_gen_seq_stream_layer& L = d->layer[l];
+    if (!L.w || (d->norm == W2S_SEQ_NORM_BATCH && (!L.running_mean || !L.running_var)))
+      return fail("gen_seq_stream_step: parameters of layer %d missing", l);
+  }
+  // a tile of G * spt streams per CTA: enough CTAs to spread small N over the SMs, at most kStreamMaxAcc per thread
+  const int G = gen::kStreamThreads / F, ld = F | 1;
+  int cc = 8192 / (k * ld);
+  cc = cc < 1 ? 1 : (cc > F ? F : cc);
+  int spt = (int)(((long long)N + (long long)G * sm_count() - 1) / ((long long)G * sm_count()));
+  spt = spt < 1 ? 1 : (spt > gen::kStreamMaxAcc ? gen::kStreamMaxAcc : spt);
+  // shared memory fits at every spt: TS * F <= 8 * 256, so tile rows take <= 2048 * (k + 2) floats, and the weight chunk
+  // cc * k * (F | 1) <= 8192 floats: <= 176 KB for k <= 16
+  const size_t smem = gen::seq_stream_smem_floats(F, k, G * spt, cc) * sizeof(float);
+  cudaError_t e = cudaFuncSetAttribute(gen::seq_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return cuda_fail(e, "gen_seq_stream_step smem attribute");
+  gen::SeqStreamArgs a{*d, x_new, logits, N, R, pos, G, spt, cc};
+  const int TS = G * spt;
+  const long long grid = ((long long)N + TS - 1) / TS;
+  const double ring_bytes = 4.0 * N * R * nb * (double)k * nd * F;  // k - 1 tap rows read + 1 row written per layer
+  LaunchScope scope((cudaStream_t)stream, "gen_seq_stream_step", ring_bytes + 4.0 * N * R * (F + d->n_classes),
+                    2.0 * N * R * (double)nb * nd * F * F * k);
+  gen::seq_stream_kernel<<<(unsigned)grid, gen::kStreamThreads, smem, (cudaStream_t)stream>>>(a);
+  W2S_LAUNCH_CHECK("gen_seq_stream_step");
 }
 
 int w2s_set_conv_impl(int impl) {

@@ -370,6 +370,10 @@ class GeneralEngine:
         for blk in enc.cnn:
             a = self.conv_block(a, blk, m, raw)
             raw = 0
+        return self.epoch_features(enc, a, m, B, S), mask
+
+    def epoch_features(self, enc, a: Tensor, m: Tensor, B: int, S: int) -> Tensor:
+        """The encoder's Linear(4C -> F) + activation (+ output_norm) on the last block's output a -> z [B, S, F]."""
         Bp, L4, Cc = a.shape
         if L4 % 4 or (Bp * L4) // 4 != B * S:
             raise ValueError(f"encoder output length {L4} does not give 4 frames per epoch")
@@ -377,7 +381,7 @@ class GeneralEngine:
         z = self.affine_act(z, enc.activation_name, mask=m)
         if isinstance(enc.output_norm, nn.LayerNorm):
             z = self.rownorm(z, enc.output_norm.weight, enc.output_norm.bias, enc.output_norm.eps)
-        return z.view(B, S, -1), mask
+        return z.view(B, S, -1)
 
     def epoch_mixer(self, zs: list[Tensor], masks: list[Tensor], B: int, S: int) -> Tensor:
         """MultiModalAttentionEmbedder.forward (wav2sleep.py:301-346) -> CLS features [B, S, F]."""
