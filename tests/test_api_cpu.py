@@ -156,3 +156,19 @@ def test_encoder_pairing_rules():
     # two signals sharing ONE encoder (same weights) may be paired too
     shared = {"EOG-L": "EOG", "EOG-R": "EOG"}
     assert groups(stub(shared, {"EOG": de["EOG-L"]}, 2), sorted(xe), xe, True) == [("EOG-L", "EOG-R")]
+
+
+@pytest.mark.parametrize("mixer_layers,seq_blocks,seq_dilations,ncls,fast", [
+    (1, 1, 1, 1, True), (8, 4, 6, 8, True), (2, 2, 6, 4, True), (3, 3, 2, 2, True),
+    (2, 2, 7, 4, False), (2, 2, 8, 4, False), (1, 1, 7, 1, False),   # dilation 64 / 128: the per-layer conv cannot stage it
+    (9, 2, 6, 4, False), (2, 5, 6, 4, False), (2, 2, 6, 9, False),
+])
+def test_fast_path_routing_corners(mixer_layers, seq_blocks, seq_dilations, ncls, fast):
+    """Wav2Sleep.fast_path at the corners of its range; everything outside it runs on the general path."""
+    from wav2sleep_b200.model import MultiModalAttentionEmbedder, SequenceCNN, SignalEncoders, Wav2Sleep
+    enc = SignalEncoders(signal_map={"ECG": "ECG"}, feature_dim=128, activation="gelu", norm="instance", causal=False,
+                         chunk_causal=False)
+    mix = MultiModalAttentionEmbedder(feature_dim=128, activation="gelu", layers=mixer_layers, dim_ff=512, nhead=8)
+    seq = SequenceCNN(feature_dim=128, activation="gelu", norm="layer", num_layers=seq_blocks, kernel_size=7,
+                      num_dilations=seq_dilations)
+    assert Wav2Sleep(enc, mix, seq, ncls).fast_path is fast

@@ -277,13 +277,45 @@ def test_seq_conv_layer(cuda_device, dil, S, res):
         assert (logits - (ref @ hw.t() + hb)).abs().max().item() < 5e-3
 
 
-@pytest.mark.parametrize("B,S,n_blocks,n_dil,ncls", [(1, 1, 2, 6, 4), (3, 40, 2, 6, 5), (2, 129, 1, 2, 4), (2, 300, 2, 6, 4),
-                                                     (3, 1200, 2, 6, 4), (2, 1680, 2, 6, 5), (1, 2048, 2, 3, 4),
-                                                     (1, 2100, 2, 6, 4)])
+def _seqmixer_fwd(lib, d, x, B, S, ncls, keep):
+    """One w2s_seqmixer_head_fwd call on a workspace of NaN patterns (padding rows must be written), run twice so that
+    the second call re-uses the dirty workspace.  Returns (features, logits)."""
+    nbytes = lib.w2s_seqmixer_workspace_bytes(C.byref(d), B, S, keep)
+    work = torch.full((nbytes,), 0x7F, dtype=torch.uint8, device=x.device)
+    feat = torch.full((B, S, 128), float("nan"), dtype=torch.float16, device=x.device)
+    logits = torch.full((B, S, ncls), float("nan"), device=x.device)
+    for rep in range(2):
+        _lib.check(lib.w2s_seqmixer_head_fwd(C.byref(d), x.data_ptr(), B, S, work.data_ptr(), nbytes, keep, feat.data_ptr(),
+                                             logits.data_ptr(), G.stream()))
+    torch.cuda.synchronize()
+    return feat, logits
+
+
+# Largest night the cluster-per-night kernel takes at 7 dilations: 2 tiles of 128 rows on each of 8 CTAs, because the
+# 2 x 192 padding rows leave no room for a third tile in 232,448 B (seq_geometry_for).
+SEQ_FUSED_MAX_S7 = 2048
+
+
+@pytest.mark.parametrize("B,S,n_blocks,n_dil,ncls", [
+    (1, 1, 2, 6, 4), (3, 40, 2, 6, 5), (2, 129, 1, 2, 4), (2, 300, 2, 6, 4), (3, 1200, 2, 6, 4), (2, 1680, 2, 6, 5),
+    (1, 2048, 2, 3, 4), (1, 2100, 2, 6, 4),
+    (2, 300, 3, 6, 4), (2, 260, 4, 6, 5),           # 3 and 4 blocks (24 layers in one launch)
+    (2, 150, 2, 1, 4), (1, 70, 4, 1, 8),            # one dilation: never fused, layer-per-launch kernels
+    (2, 500, 2, 7, 4),                              # 7 dilations fused: padding 3 * 64 = 192 rows
+    (3, 40, 2, 6, 1), (2, 130, 1, 3, 8),            # 1 and 8 classes
+    (2, 5, 2, 6, 4), (3, 2, 1, 7, 5),               # nights shorter than the largest dilation
+    (1, 2048, 1, 6, 4), (1, 2049, 1, 6, 4),         # around 2048 epochs at 6 dilations ...
+    (1, 2048, 1, 7, 4), (1, 2049, 1, 7, 4),         # ... and on both sides of the fused limit at 7 dilations
+    (160, 100, 2, 6, 4),                            # more nights than clusters can be resident (148 SMs)
+    (2, 64, 1, 8, 4),                               # 8 dilations: layer-per-launch only, which cannot stage dilation 128
+])
 def test_seqmixer_stage(cuda_device, B, S, n_blocks, n_dil, ncls):
-    """w2s_seqmixer_head_fwd (SequenceCNN + classifier, models/wav2sleep.py:379-390, 66) against fp32 torch on the
-    fp16-rounded operands and inter-layer activations.  S <= 2048 runs the cluster-per-night kernel (seq_mixer.cuh: 1 CTA
-    for S <= 128 ... 8 CTAs x 256 rows), S = 2100 the layer-per-launch kernels; both must give the same numbers."""
+    """w2s_seqmixer_head_fwd (SequenceCNN + classifier, models/wav2sleep.py:379-390, 66) against an fp64 torch
+    restatement on the fp16-rounded operands and inter-layer activations.  keep = 0 runs the cluster-per-night kernel
+    where it fits (seq_mixer.cuh: 2..7 dilations, 1 CTA for S <= 128 ... 8 CTAs x 4 tiles), the layer-per-launch kernels
+    otherwise; keep = 1 (the training layout, every layer output kept) always runs the layer-per-launch kernels.  Both
+    must give the same numbers.  The tile-per-CTA conv cannot stage dilation 64 or more in shared memory: those calls
+    must fail with the layer's shape and byte count."""
     lib = _lib.load()
     torch.manual_seed(S + n_dil)
     dev = cuda_device
@@ -301,36 +333,46 @@ def test_seqmixer_stage(cuda_device, B, S, n_blocks, n_dil, ncls):
             d.w[bl][k], d.ln_w[bl][k], d.ln_b[bl][k] = pw.data_ptr(), g.data_ptr(), b.data_ptr()
     hw, hb = torch.randn(ncls, 128, device=dev) / 11, torch.randn(ncls, device=dev)
     d.head_w, d.head_b = hw.data_ptr(), hb.data_ptr()
-    nbytes = lib.w2s_seqmixer_workspace_bytes(C.byref(d), B, S, 0)
-    work = torch.full((nbytes,), 0x7F, dtype=torch.uint8, device=dev)  # garbage (NaN patterns): padding must be written
-    feat = torch.full((B, S, 128), float("nan"), dtype=torch.float16, device=dev)
-    logits = torch.full((B, S, ncls), float("nan"), device=dev)
-    for rep in range(2):  # second call re-uses the dirty workspace
-        _lib.check(lib.w2s_seqmixer_head_fwd(C.byref(d), x.data_ptr(), B, S, work.data_ptr(), nbytes, 0, feat.data_ptr(),
-                                             logits.data_ptr(), G.stream()))
-    torch.cuda.synchronize()
-    cur = x.float()
+    cur = x.double()
     i = 0
     for bl in range(n_blocks):
         blk_in = cur
         for k in range(n_dil):
-            c = G.conv_ref(cur, ws[i], stride=1, pad=3 * 2 ** k, dil=2 ** k)
+            c = torch.nn.functional.conv1d(cur.transpose(1, 2), ws[i].half().double(), padding=3 * 2 ** k,
+                                           dilation=2 ** k).transpose(1, 2)
             mu = c.mean(-1, keepdim=True)
             var = (c - mu).pow(2).mean(-1, keepdim=True)
-            a = G.gelu((c - mu) / torch.sqrt(var + 1e-5) * gs[i] + bs[i])
+            a = G.gelu((c - mu) / torch.sqrt(var + 1e-5) * gs[i].double() + bs[i].double())
             if k == n_dil - 1:
                 a = G.gelu(a + blk_in)
             last = (bl == n_blocks - 1 and k == n_dil - 1)
             final = a
-            cur = a if last else a.half().float()
+            cur = a if last else a.half().double()  # every layer but the last stores fp16
             i += 1
-    ref_logits = final @ hw.t() + hb
-    assert torch.isfinite(logits).all() and torch.isfinite(feat.float()).all()
-    e_feat = (feat.float() - final).abs().max().item()
-    e_log = (logits - ref_logits).abs().max().item()
-    print(f"seq mixer B={B} S={S}: feature max-abs {e_feat:.3e}, logits max-abs {e_log:.3e}")
-    # fp16 re-rounding of 1-ulp-different intermediates over n_blocks * n_dil layers
-    assert e_feat < 1.5e-2 and e_log < 1.5e-2
+    ref_logits = final @ hw.double().t() + hb.double()
+    # the per-layer conv stages (128 - 1) + 6 * dilation + 1 rows: dilation 64 and up exceed the shared memory of a block
+    per_layer_fits = n_dil <= 6
+    fused = 2 <= n_dil <= 7 and (n_dil < 7 or S <= SEQ_FUSED_MAX_S7)
+    out = {}
+    for kp in (0, 1):
+        if not (per_layer_fits or (kp == 0 and fused)):
+            with pytest.raises(RuntimeError, match=r"c128->128 k7 stride 1 dilation 64 needs 269328 B of shared memory"):
+                _seqmixer_fwd(lib, d, x, B, S, ncls, kp)
+            print(f"seq mixer B={B} S={S} {n_blocks}x{n_dil} keep={kp}: refused ({_lib.load().w2s_last_error().decode()})")
+            continue
+        feat, logits = _seqmixer_fwd(lib, d, x, B, S, ncls, kp)
+        assert torch.isfinite(logits).all() and torch.isfinite(feat.float()).all()
+        e_feat = (feat.double() - final).abs().max().item()
+        e_log = (logits.double() - ref_logits).abs().max().item()
+        print(f"seq mixer B={B} S={S} {n_blocks}x{n_dil} C={ncls} keep={kp}: feature max-abs {e_feat:.3e}, "
+              f"logits max-abs {e_log:.3e}")
+        # fp16 re-rounding of 1-ulp-different intermediates over n_blocks * n_dil layers
+        assert e_feat < 1.5e-2 and e_log < 1.5e-2
+        out[kp] = logits
+    if len(out) == 2:
+        e_keep = (out[1] - out[0]).abs().max().item()
+        print(f"seq mixer B={B} S={S}: keep=1 vs keep=0 logits max-abs {e_keep:.3e}")
+        assert e_keep < 1.5e-2
 
 
 @pytest.mark.parametrize("c", [32, 64, 128])

@@ -249,6 +249,31 @@ static bool conv_calls_pairable(const w2s_conv_call& a, const w2s_conv_call& b) 
          (a.row_mask != nullptr) == (b.row_mask != nullptr) && (a.bias != nullptr) == (b.bias != nullptr);
 }
 
+// Shared memory one block may opt in to on this device (232,448 B on sm_100).
+int smem_optin_bytes() {
+  static int n = 0;
+  if (n == 0) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&n, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (n <= 0) n = 232448;
+  }
+  return n;
+}
+
+// The tile-per-CTA kernel stages every input row its 128-position tile reaches, (taps - 1) * dilation of them beyond
+// the tile, so a wide dilation can need more shared memory than a block can have (k7 128 -> 128: 220,176 B at dilation
+// 32, 269,328 B at 64).  Such a call fails with its layer shape and byte count instead of the bare attribute error.
+template <int CIN, int COUT, int TAPS, int GT, int PRO, int EPI, bool DS, bool BF16OP = false>
+int run_conv_igemm(const w2s_conv_call& c, const ConvArgs& a, cudaStream_t st) {
+  const size_t smem = conv_igemm_smem_bytes<CIN, COUT, TAPS, GT, EPI, DS, BF16OP>(a);
+  if (smem > (size_t)smem_optin_bytes())
+    return fail("conv1d: c%d->%d k%d stride %d dilation %d needs %zu B of shared memory per block, over the %d B limit "
+                "of this device", c.cin, c.cout, c.taps, c.stride, c.dilation, smem, smem_optin_bytes());
+  const cudaError_t e = launch_conv_igemm<CIN, COUT, TAPS, GT, PRO, EPI, DS, BF16OP>(a, c.B, st);
+  return e == cudaSuccess ? 0 : cuda_fail(e, "conv1d launch");
+}
+
 int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* c2 = nullptr) {
   if (c2 != nullptr && !conv_calls_pairable(c, *c2)) return kNotPaired;
   if (c.B <= 0 || c.L_in <= 0 || c.L_out <= 0) return fail("conv1d: empty shape B=%d L_in=%d L_out=%d", c.B, c.L_in, c.L_out);
@@ -380,24 +405,17 @@ int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* 
   if (c2 != nullptr) return kNotPaired;  // no stream kernel for this configuration: the caller dispatches the two calls singly
   if (impl == 3) {  // bf16 operands on the tile-per-CTA kernel: un-split encoder convs without the 1x1 branch only
 #define W2S_BF16(CIN, COUT)                                                                                          \
-  if (!found && c.cin == CIN && c.cout == COUT && c.taps == 3 && c.prologue == PRO_NORM && c.epilogue == EPI_STATS && \
-      !c.has_ds) {                                                                                                   \
-    found = true;                                                                                                    \
-    e = launch_conv_igemm<CIN, COUT, 3, 3, PRO_NORM, EPI_STATS, false, true>(a, c.B, st);                            \
-  }
+  if (c.cin == CIN && c.cout == COUT && c.taps == 3 && c.prologue == PRO_NORM && c.epilogue == EPI_STATS && !c.has_ds) \
+    return run_conv_igemm<CIN, COUT, 3, 3, PRO_NORM, EPI_STATS, false, true>(c, a, st);
     W2S_BF16(32, 32)
     W2S_BF16(64, 64)
     W2S_BF16(128, 128)
 #undef W2S_BF16
-    if (!found) return fail("conv1d: bf16-operand hook is built for k3 32->32 / 64->64 / 128->128 EPI_STATS convs only");
-    return e == cudaSuccess ? 0 : cuda_fail(e, "conv_igemm (bf16 operands) launch");
+    return fail("conv1d: bf16-operand hook is built for k3 32->32 / 64->64 / 128->128 EPI_STATS convs only");
   }
-#define W2S_CASE(CIN, COUT, TAPS, GT, PRO, EPI, DS)                                                       \
-  if (!found && c.cin == CIN && c.cout == COUT && c.taps == TAPS && c.prologue == PRO && c.epilogue == EPI && \
-      (c.has_ds != 0) == DS) {                                                                            \
-    found = true;                                                                                         \
-    e = launch_conv_igemm<CIN, COUT, TAPS, GT, PRO, EPI, DS>(a, c.B, st);                                  \
-  }
+#define W2S_CASE(CIN, COUT, TAPS, GT, PRO, EPI, DS)                                                                  \
+  if (c.cin == CIN && c.cout == COUT && c.taps == TAPS && c.prologue == PRO && c.epilogue == EPI && (c.has_ds != 0) == DS) \
+    return run_conv_igemm<CIN, COUT, TAPS, GT, PRO, EPI, DS>(c, a, st);
   // encoder conv1 (block input = previous block's conv3 output + residual branch), with fused downsample
   W2S_CASE(16, 16, 3, 3, PRO_NORM_RES, EPI_STATS, true)
   W2S_CASE(16, 32, 3, 3, PRO_NORM_RES, EPI_STATS, true)
@@ -452,11 +470,8 @@ int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* 
   W2S_CASE(64, 32, 1, 1, PRO_NONE, EPI_PLAIN, false)
   W2S_CASE(64, 64, 1, 1, PRO_NONE, EPI_PLAIN, false)
 #undef W2S_CASE
-  if (!found)
-    return fail("conv1d: no kernel for cin=%d cout=%d taps=%d pro=%d epi=%d ds=%d", c.cin, c.cout, c.taps, c.prologue,
-                c.epilogue, c.has_ds);
-  if (e != cudaSuccess) return cuda_fail(e, "conv1d launch");
-  return 0;
+  return fail("conv1d: no kernel for cin=%d cout=%d taps=%d pro=%d epi=%d ds=%d", c.cin, c.cout, c.taps, c.prologue,
+              c.epilogue, c.has_ds);
 }
 
 // Rotating slot allocator for inference workspaces.

@@ -752,13 +752,19 @@ inline cudaError_t launch_conv_igemm_pair(const ConvArgs& a, const ConvArgs& a2,
   return cudaGetLastError();
 }
 
+// Dynamic shared memory of one launch_conv_igemm call.
+template <int CIN, int COUT, int TAPS, int GT, int EPI, bool HAS_DS, bool BF16OP = false>
+inline size_t conv_igemm_smem_bytes(const ConvArgs& a) {
+  constexpr bool SPLIT = ConvSplit<CIN, COUT>::value && EPI == EPI_STATS && !BF16OP;
+  return conv_smem_bytes<CIN, COUT, GT, HAS_DS, SPLIT>(1 << a.stride_log2, TAPS, a.dil);
+}
+
 // Host-side launcher.  Returns cudaError_t of the launch.
 template <int CIN, int COUT, int TAPS, int GT, int PRO, int EPI, bool HAS_DS, bool BF16OP = false>
 inline cudaError_t launch_conv_igemm(const ConvArgs& a, int B, cudaStream_t stream) {
   constexpr bool SPLIT = ConvSplit<CIN, COUT>::value && EPI == EPI_STATS && !BF16OP;
   auto kern = conv_igemm_kernel<CIN, COUT, TAPS, GT, PRO, EPI, HAS_DS, SPLIT, BF16OP>;
-  const int stride = 1 << a.stride_log2;
-  const size_t smem = conv_smem_bytes<CIN, COUT, GT, HAS_DS, SPLIT>(stride, TAPS, a.dil);
+  const size_t smem = conv_igemm_smem_bytes<CIN, COUT, TAPS, GT, EPI, HAS_DS, BF16OP>(a);
   static size_t configured = 0;  // per instantiation
   if (smem > configured) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -320,8 +320,11 @@ class SequenceCNN(nn.Module):
         self.dilated_convs = nn.Sequential(*[
             DilatedConvBlock(feature_dim=feature_dim, dropout=dropout, activation=activation, norm=norm, causal=causal,
                              kernel_size=kernel_size, num_dilations=num_dilations) for _ in range(num_layers)])
+        # num_dilations <= 6: the training forward / backward and long nights run every layer as its own tile-per-CTA
+        # conv, which stages (kernel_size - 1) * dilation rows beyond each tile in shared memory; dilation 64 (7 layers)
+        # needs 269,328 B, over the 232,448 B a block can have, so deeper stacks go to the general path
         self.fast_path = (feature_dim == 128 and kernel_size == 7 and activation == "gelu" and norm == "layer"
-                          and not causal and 1 <= num_layers <= 4 and 1 <= num_dilations <= 8)
+                          and not causal and 1 <= num_layers <= 4 and 1 <= num_dilations <= 6)
 
     def compile(self, *args, **kwargs) -> None:
         """Accepted and ignored (see SignalEncoders.compile): the CUDA path needs no tracing compiler."""
