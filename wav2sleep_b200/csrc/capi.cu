@@ -295,6 +295,13 @@ int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* 
     if (c.out_stride > 1 || c.out_offset != 0 || (c.out_rows > 0 && c.out_rows != c.L_out))
       return fail("conv1d: W2S_EPI_ACT_BWD writes dense rows only");
   }
+  if (c.epilogue == W2S_EPI_PLAIN) {  // output row o * out_stride + out_offset of a sample of out_rows rows
+    const int os = c.out_stride > 0 ? c.out_stride : 1, rows = c.out_rows > 0 ? c.out_rows : c.L_out;
+    if (c.out_offset < 0 || c.out_offset >= os || (long long)(c.L_out - 1) * os + c.out_offset >= rows)
+      return fail("conv1d: W2S_EPI_PLAIN output rows out of range: L_out=%d out_stride=%d out_offset=%d out_rows=%d "
+                  "(needs 0 <= out_offset < out_stride and (L_out - 1) * out_stride + out_offset < out_rows)",
+                  c.L_out, os, c.out_offset, rows);
+  }
   const ConvArgs a = to_args(c);
   ConvArgs a2s;
   const ConvArgs* a2 = nullptr;
@@ -1062,19 +1069,25 @@ int w2s_gemm_tn(const void* X, const void* Y, float* Cm, int M, int N, int taps,
   return e == cudaSuccess ? 0 : cuda_fail(e, "gemm_tn launch");
 }
 
+// The encoder element kernels keep one 8-channel chunk per thread for the whole grid-stride loop (C / 8 a power of two
+// dividing 256) and their per-channel constants in 128-entry shared-memory slots.
+static bool enc_channels_ok(int Cc) { return Cc == 8 || Cc == 16 || Cc == 32 || Cc == 64 || Cc == 128; }
+
 int w2s_enc_act_fwd(const void* y, const void* r, const double* stats, void* a, const uint8_t* row_mask, int B, int L,
                     int Cc, float eps, void* stream) {
-  if (!y || !stats || !a || Cc % 8) return fail("enc_act_fwd: bad arguments");
+  if (!y || !stats || !a) return fail("enc_act_fwd: bad arguments");
+  if (!enc_channels_ok(Cc)) return fail("enc_act_fwd: C=%d (built for 8, 16, 32, 64 or 128 channels)", Cc);
   EncActArgs p{(const act_t*)y, (const act_t*)r, stats, (act_t*)a, row_mask, B, L, Cc, eps};
   LaunchScope scope((cudaStream_t)stream, "enc_act_fwd", (double)B * L * Cc * (r ? 6.0 : 4.0), 0);
-  dim3 grid(ew_grid((long long)L * (Cc / 8)) / (B > 1 ? 1 : 1), B);
+  dim3 grid(ew_grid((long long)L * (Cc / 8)), B);
   enc_act_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(p);
   W2S_LAUNCH_CHECK("enc_act_fwd");
 }
 
 int w2s_enc_act_bwd(const void* dout, const void* y, const void* r, const double* stats, void* dxh, void* dr, double* sums,
                     void* a_out, const uint8_t* row_mask, int B, int L, int Cc, float eps, void* stream) {
-  if (!dout || !y || !stats || !dxh || !sums || Cc % 8 || 256 % (Cc / 8)) return fail("enc_act_bwd: bad arguments");
+  if (!dout || !y || !stats || !dxh || !sums) return fail("enc_act_bwd: bad arguments");
+  if (!enc_channels_ok(Cc)) return fail("enc_act_bwd: C=%d (built for 8, 16, 32, 64 or 128 channels)", Cc);
   if (r && !dr) return fail("enc_act_bwd: dr missing");
   EncActBwdArgs p{(const act_t*)dout, (const act_t*)y, (const act_t*)r, stats, (act_t*)dxh, (act_t*)dr, sums, row_mask,
                   B, L, Cc, eps, (act_t*)a_out};
@@ -1089,7 +1102,8 @@ int w2s_enc_act_bwd(const void* dout, const void* y, const void* r, const double
 
 int w2s_enc_norm_bwd(const void* dxh, const void* y, const double* stats, const double* sums, void* dy,
                      const uint8_t* row_mask, int B, int L, int Cc, int upsample, float eps, void* stream) {
-  if (!dxh || !y || !stats || !sums || !dy || Cc % 8) return fail("enc_norm_bwd: bad arguments");
+  if (!dxh || !y || !stats || !sums || !dy) return fail("enc_norm_bwd: bad arguments");
+  if (!enc_channels_ok(Cc)) return fail("enc_norm_bwd: C=%d (built for 8, 16, 32, 64 or 128 channels)", Cc);
   EncNormBwdArgs p{(const act_t*)dxh, (const act_t*)y, stats, sums, (act_t*)dy, row_mask, B, L, Cc, upsample, eps};
   LaunchScope scope((cudaStream_t)stream, "enc_norm_bwd", (double)B * L * Cc * 6.0, 0);
   dim3 grid(ew_grid((long long)L * (Cc / 8)), B);
@@ -1100,6 +1114,8 @@ int w2s_enc_norm_bwd(const void* dxh, const void* y, const double* stats, const 
 int w2s_first_conv_wgrad(const float* x, const void* dy1, const void* dr, float* dw1, float* dwds, const uint8_t* row_mask,
                          int B, int T, float scale, void* stream) {
   if (!x || !dy1 || !dr || !dw1 || !dwds) return fail("first_conv_wgrad: bad arguments");
+  // dr holds the T / 2 rows of the stride-2 residual branch: row l / 2 pairs with input sample l for even l
+  if (B <= 0 || T <= 0 || (T & 1)) return fail("first_conv_wgrad: B=%d T=%d (needs B > 0 and an even T > 0)", B, T);
   FirstWgradArgs p{x, (const act_t*)dy1, (const act_t*)dr, dw1, dwds, row_mask, B, T, scale};
   LaunchScope scope((cudaStream_t)stream, "first_conv_wgrad", (double)B * T * (4.0 + 32.0 + 16.0), 0);
   int gx = (T + 256 * 16 - 1) / (256 * 16);

@@ -337,7 +337,7 @@ __global__ void __launch_bounds__(256) row_ln_bwd_kernel(const RowLnArgs p) {
       xh[k] = x[k] * rstd;
       const float u = xh[k] * gv[k] + bv[k];
       float g = d[k];
-      if (p.res) { g *= gelu_grad(gelu_erf(u) + rr[k]); rr[k] = g; }  // ds
+      if (p.res) { g *= gelu_grad((p.gelu ? gelu_erf(u) : u) + rr[k]); rr[k] = g; }  // ds = dout GELU'(s)
       if (p.gelu) g *= gelu_grad(u);
       ag[k] += g * xh[k];
       ab[k] += g;
@@ -407,7 +407,7 @@ __global__ void __launch_bounds__(256) gelu_bwd_kernel(const act_t* pre, const a
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// J. column sums of a [rows, C] fp16 matrix into fp32 (bias gradients); C <= 512, C % 8 == 0
+// J. column sums of a [rows, C] fp16 matrix into fp32 (bias gradients); C <= 128, C % 8 == 0, 256 % (C / 8) == 0
 // ------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) colsum_kernel(const act_t* x, float* out, long long rows, int C, int row_stride,
                                                      int row_offset, const uint8_t* row_mask,
