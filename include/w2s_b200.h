@@ -283,10 +283,15 @@ int w2s_enc_norm_bwd(const void* dxh, const void* y, const double* stats, const 
 /* weight gradients of the Cin = 1 layers of block 0 (conv1 [16,1,3] and downsample [16,1,1]), accumulated times scale. */
 int w2s_first_conv_wgrad(const float* x, const void* dy1, const void* dr, float* dw1, float* dwds, const uint8_t* row_mask,
                          int B, int T, float scale, void* stream);
+/* data gradient of the same two layers into the raw fp32 signal (input attribution; ABI v7):
+ *   dx[b, t] = scale * (sum_c sum_k w1[c, k] dy1[b, t+1-k, c] + [t even] sum_c wds[c] dr[b, t/2, c]),
+ * out-of-range dy1 rows read as 0; dx = 0 where x is non-finite and on rows with row_mask[b] != 0.  T even. */
+int w2s_first_conv_dgrad(const float* x, const void* dy1, const void* dr, const float* w1, const float* wds,
+                         const uint8_t* row_mask, float* dx, int B, int T, float scale, void* stream);
 /* LayerNorm over 128 features per row (+GELU, + residual add + GELU): nn.LayerNorm / ConvLayerNorm (models/utils.py:9-23). */
 int w2s_row_ln_fwd(const void* x, const void* res, const float* g, const float* b, void* out, long long rows, int gelu,
                    float eps, void* stream);
-/* dg / db are accumulated times gscale (the inverse loss scale, see below). */
+/* dg / db are accumulated times gscale (the inverse loss scale, see below); both NULL: not computed (frozen parameters, ABI v7). */
 int w2s_row_ln_bwd(const void* x, const void* res, const float* g, const float* b, const void* dout, const void* dadd,
                    void* dx, void* ds, float* dg, float* db, long long rows, int gelu, float eps, float gscale,
                    void* stream);
@@ -308,7 +313,8 @@ int w2s_attn_fwd(const void* q, const void* k, const void* v, void* o, const uin
                  uint64_t seed, uint32_t site, void* stream);
 int w2s_attn_bwd(const void* q, const void* k, const void* v, const void* dout, void* dq, void* dk, void* dv,
                  const uint8_t* key_mask, int N, int D, float drop_p, uint64_t seed, uint32_t site, void* stream);
-/* token tensor [N, 1+n_sig, 128] = [cls, z_0[n], ...] (zeros + key mask for missing signals) and its backward. */
+/* token tensor [N, 1+n_sig, 128] = [cls, z_0[n], ...] (zeros + key mask for missing signals) and its backward (dcls may be
+ * NULL: the CLS gradient is not computed, ABI v7). */
 int w2s_tokens_fwd(const void* const* z, const uint8_t* const* row_mask, const float* cls, void* tokens, uint8_t* key_mask,
                    int N, int S, int n_sig, void* stream);
 int w2s_tokens_bwd(const void* dtokens, void* const* dz, const uint8_t* const* row_mask, float* dcls, int N, int S, int n_sig,
@@ -325,13 +331,16 @@ int w2s_ce_fwd_bwd(const float* logits, const long long* labels, long long N, in
  * linear in the incoming gradient, and every kernel that accumulates a PARAMETER gradient multiplies by the inverse
  * (w2s_gemm_tn scale, w2s_colsum scale, w2s_row_ln_bwd gscale, w2s_first_conv_wgrad scale, w2s_tokens_bwd cls_scale),
  * so fp32 parameter gradients come out unscaled.  Reference numerics being matched: fp32 autograd
- * (scripts/config/training/main.yaml:16 `precision: 32-true`). */
+ * (scripts/config/training/main.yaml:16 `precision: 32-true`).  dw / db may be NULL (not computed; ABI v7). */
 int w2s_head_bwd(const void* feat, const float* w, const float* dlogits, void* dfeat, float* dw, float* db, long long N, int C,
                  float dfeat_scale, void* stream);
 /* out += sum g^2 (fp64); fused global-norm clip (torch clip_grad_norm_) + AdamW step on flat fp32 buffers.
  * ema != NULL: the same pass also updates ema = ema_decay * ema + (1 - ema_decay) * p_new, the per-batch update of the
  * reference's EMACallback (trainer/callbacks.py:54-66, SURVEY 8f N4). */
 int w2s_sumsq(const float* g, long long n, double* out, void* stream);
+/* *out = max |g[i]| (fp32; the call zeroes *out first).  Picks the loss scale of a backward whose incoming gradient is
+ * not a mean cross entropy (input attribution; ABI v7). */
+int w2s_absmax(const float* g, long long n, float* out, void* stream);
 int w2s_adamw_step(float* p, const float* g, float* m, float* v, long long n, const double* gnorm_sq, float lr, float beta1,
                    float beta2, float eps, float weight_decay, float max_norm, float grad_scale, long long step, float* ema,
                    float ema_decay, void* stream);
@@ -392,6 +401,10 @@ int w2s_gen_attn(const float* q, const float* k, const float* v, float* o, const
  * are zeroed by the call itself. */
 /* din[b, li, ci] = sum over (lo, t) with lo*stride - pad_left + t*dil = li of dout[b, lo, co] * w[co, ci, t]  (gather, no
  * atomics; every case of w2s_gen_conv incl. taps_major). */
+/* eval-mode BatchNorm1d: dweight = (dscale - running_mean * dshift) / sqrt(running_var + eps), dbias = dshift, all [C]
+ * (the parameters behind w2s_gen_norm_consts' batch-mode scale / shift; either output may be NULL; ABI v7). */
+int w2s_gen_bn_eval_bwd(const float* dscale, const float* dshift, const float* running_mean, const float* running_var,
+                        float* dweight, float* dbias, int C, float eps, void* stream);
 int w2s_gen_conv_dgrad(const float* dout, const float* w, float* din, const uint8_t* row_mask, int B, int L_in, int L_out, int cin,
                        int cout, int taps, int stride, int dil, int pad_left, int taps_major, void* stream);
 /* dw[co, ci, t] = sum_{b, lo} dout * in (layout of w2s_gen_conv's w), dbias[co] = sum dout; non-finite raw samples read as 0

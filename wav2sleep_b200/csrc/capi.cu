@@ -530,7 +530,7 @@ int check_encoder_desc(const w2s_encoder_desc* d) {
 
 extern "C" {
 
-int w2s_abi_version(void) { return 6; }
+int w2s_abi_version(void) { return 7; }
 const char* w2s_last_error(void) { return g_err.c_str(); }
 
 int w2s_conv_uses_split(int cin, int cout) { return (cin <= 16 && cout <= 16) ? 1 : 0; }
@@ -1124,6 +1124,20 @@ int w2s_first_conv_wgrad(const float* x, const void* dy1, const void* dr, float*
   W2S_LAUNCH_CHECK("first_conv_wgrad");
 }
 
+int w2s_first_conv_dgrad(const float* x, const void* dy1, const void* dr, const float* w1, const float* wds,
+                         const uint8_t* row_mask, float* dx, int B, int T, float scale, void* stream) {
+  if (!x || !dy1 || !dr || !w1 || !wds || !row_mask || !dx)
+    return fail("first_conv_dgrad: NULL operand (x=%p dy1=%p dr=%p w1=%p wds=%p row_mask=%p dx=%p)", (const void*)x, dy1, dr,
+                (const void*)w1, (const void*)wds, (const void*)row_mask, (void*)dx);
+  if (B <= 0 || B > 65535 || T <= 0 || (T & 1))
+    return fail("first_conv_dgrad: B=%d T=%d (needs 0 < B <= 65535 and an even T > 0)", B, T);
+  FirstDgradArgs p{x, (const act_t*)dy1, (const act_t*)dr, w1, wds, row_mask, dx, (long long)T, scale};
+  LaunchScope scope((cudaStream_t)stream, "first_conv_dgrad", (double)B * T * (32.0 + 16.0 + 4.0 + 4.0), (double)B * T * 128.0);
+  dim3 grid((unsigned)(((long long)T + kFirstDgradThreads - 1) / kFirstDgradThreads), B);
+  first_conv_dgrad_kernel<<<grid, kFirstDgradThreads, 0, (cudaStream_t)stream>>>(p);
+  W2S_LAUNCH_CHECK("first_conv_dgrad");
+}
+
 int w2s_row_ln_fwd(const void* x, const void* res, const float* g, const float* b, void* out, long long rows, int gelu,
                    float eps, void* stream) {
   if (!x || !g || !b || !out || rows <= 0) return fail("row_ln_fwd: bad arguments");
@@ -1139,7 +1153,7 @@ int w2s_row_ln_fwd(const void* x, const void* res, const float* g, const float* 
 int w2s_row_ln_bwd(const void* x, const void* res, const float* g, const float* b, const void* dout, const void* dadd,
                    void* dx, void* ds, float* dg, float* db, long long rows, int gelu, float eps, float gscale,
                    void* stream) {
-  if (!x || !g || !b || !dout || !dx || !dg || !db || rows <= 0) return fail("row_ln_bwd: bad arguments");
+  if (!x || !g || !b || !dout || !dx || !dg != !db || rows <= 0) return fail("row_ln_bwd: bad arguments");
   RowLnArgs p;
   memset(&p, 0, sizeof(p));
   p.x = (const act_t*)x; p.res = (const act_t*)res; p.g = g; p.b = b; p.out = (act_t*)dx; p.dout = (const act_t*)dout;
@@ -1229,7 +1243,7 @@ int w2s_tokens_fwd(const void* const* z, const uint8_t* const* row_mask, const f
 }
 int w2s_tokens_bwd(const void* dtokens, void* const* dz, const uint8_t* const* row_mask, float* dcls, int N, int S, int n_sig,
                    float cls_scale, void* stream) {
-  if (!dtokens || !dz || !dcls || n_sig < 1 || n_sig > 4) return fail("tokens_bwd: bad arguments");
+  if (!dtokens || !dz || n_sig < 1 || n_sig > 4) return fail("tokens_bwd: bad arguments");
   TokenArgs p;
   memset(&p, 0, sizeof(p));
   for (int i = 0; i < n_sig; ++i) { p.dz[i] = (act_t*)dz[i]; p.row_mask[i] = row_mask ? row_mask[i] : nullptr; }
@@ -1274,7 +1288,7 @@ int w2s_ce_fwd_bwd(const float* logits, const long long* labels, long long N, in
 }
 int w2s_head_bwd(const void* feat, const float* w, const float* dlogits, void* dfeat, float* dw, float* db, long long N, int Cc,
                  float dfeat_scale, void* stream) {
-  if (!feat || !w || !dlogits || !dfeat || !dw || !db || N <= 0 || Cc < 1 || Cc > 8) return fail("head_bwd: bad arguments");
+  if (!feat || !w || !dlogits || !dfeat || N <= 0 || Cc < 1 || Cc > 8) return fail("head_bwd: bad arguments");
   HeadArgs p;
   memset(&p, 0, sizeof(p));
   p.feat = (const act_t*)feat; p.w = w; p.dlogits = dlogits; p.dfeat = (act_t*)dfeat; p.dw = dw; p.db = db; p.N = N; p.C = Cc;
@@ -1293,6 +1307,16 @@ int w2s_sumsq(const float* g, long long n, double* out, void* stream) {
   if (gx > 2 * sm_count()) gx = 2 * sm_count();
   sumsq_kernel<<<gx, 256, 0, (cudaStream_t)stream>>>(g, n, out);
   W2S_LAUNCH_CHECK("sumsq");
+}
+int w2s_absmax(const float* g, long long n, float* out, void* stream) {
+  if (!g || !out || n <= 0) return fail("absmax: bad arguments (g=%p out=%p n=%lld)", (const void*)g, (void*)out, n);
+  cudaError_t e = cudaMemsetAsync(out, 0, sizeof(float), (cudaStream_t)stream);
+  if (e != cudaSuccess) return cuda_fail(e, "absmax memset");
+  LaunchScope scope((cudaStream_t)stream, "absmax", (double)n * 4.0, 0);
+  int gx = ew_grid(n);
+  if (gx > 2 * sm_count()) gx = 2 * sm_count();
+  absmax_kernel<<<gx, 256, 0, (cudaStream_t)stream>>>(g, n, reinterpret_cast<unsigned int*>(out));
+  W2S_LAUNCH_CHECK("absmax");
 }
 int w2s_adamw_step(float* p_, const float* g, float* m, float* v, long long n, const double* gnorm_sq, float lr, float beta1,
                    float beta2, float eps, float weight_decay, float max_norm, float grad_scale, long long step, float* ema,
@@ -1512,6 +1536,15 @@ int w2s_gen_attn_bwd(const float* q, const float* k, const float* v, const float
   LaunchScope scope((cudaStream_t)stream, "gen_attn_bwd", (double)N * D * H * hd * 28.0, 0);
   gen::attn_bwd_kernel<<<ew_grid((long long)N * D * H, 128), 128, 0, (cudaStream_t)stream>>>(a);
   W2S_LAUNCH_CHECK("gen_attn_bwd");
+}
+int w2s_gen_bn_eval_bwd(const float* dscale, const float* dshift, const float* running_mean, const float* running_var,
+                        float* dweight, float* dbias, int Cc, float eps, void* stream) {
+  if (!dscale || !dshift || !running_mean || !running_var || (!dweight && !dbias) || Cc < 1)
+    return fail("gen_bn_eval_bwd: bad arguments (C=%d)", Cc);
+  LaunchScope scope((cudaStream_t)stream, "gen_bn_eval_bwd", (double)Cc * 24.0, 0);
+  gen::bn_eval_bwd_kernel<<<ew_grid(Cc), 256, 0, (cudaStream_t)stream>>>(dscale, dshift, running_mean, running_var, dweight,
+                                                                          dbias, Cc, eps);
+  W2S_LAUNCH_CHECK("gen_bn_eval_bwd");
 }
 int w2s_gen_dropout(const float* x, float* out, uint8_t* mask_out, long long n, float p, uint64_t seed, uint32_t site,
                     void* stream) {

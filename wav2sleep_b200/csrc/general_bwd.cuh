@@ -409,5 +409,17 @@ __global__ void __launch_bounds__(256) dropout_kernel(const float* x, float* out
   }
 }
 
+// Eval-mode BatchNorm1d parameters from the gradients of its per-channel affine (scale = w rstd, shift = b - mean w rstd,
+// norm_consts_kernel with NORM_BATCH_EVAL): dweight = (dscale - running_mean dshift) rstd, dbias = dshift.
+__global__ void __launch_bounds__(256) bn_eval_bwd_kernel(const float* dscale, const float* dshift, const float* running_mean,
+                                                          const float* running_var, float* dweight, float* dbias, int C,
+                                                          float eps) {
+  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < C; c += gridDim.x * blockDim.x) {
+    const double rstd = 1.0 / sqrt((double)running_var[c] + (double)eps);
+    if (dweight) dweight[c] = (float)(((double)dscale[c] - (double)running_mean[c] * (double)dshift[c]) * rstd);
+    if (dbias) dbias[c] = dshift[c];
+  }
+}
+
 }  // namespace gen
 }  // namespace w2s

@@ -253,6 +253,88 @@ __global__ void __launch_bounds__(256) first_conv_wgrad_kernel(const FirstWgradA
   else if (threadIdx.x < 64) atomicAdd(&p.dwds[threadIdx.x - 48], red[threadIdx.x] * p.scale);
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// Data gradient of block 0's two Cin = 1 layers into the raw signal (input attribution):
+//   dx[t] = scale * (sum_c sum_k W1[c,k] dy1[t+1-k, c] + [t even] sum_c Wds[c] dr[t/2, c])
+// with out-of-range dy1 rows read as 0, and dx = 0 where x is non-finite (the reference replaces those samples by a
+// constant, wav2sleep.py:150-151) and on masked rows.  One thread per sample: it reads its own 32-byte dy1 row and forms
+// the three tap projections P_k[t] = sum_c W1[c,k] dy1[t,c]; dx[t] needs P0[t+1] and P2[t-1], which come from the
+// neighbouring lanes (the two warp-edge lanes read the one row beyond the warp, an L1/L2 hit).  HBM traffic per sample:
+// 32 B dy1 + 16 B dr + 4 B x + 4 B dx.
+// ------------------------------------------------------------------------------------------------------------------
+struct FirstDgradArgs {
+  const float* x;           // [B, T]
+  const act_t* dy1;         // [B, T, 16]    gradient of conv1's pre-norm output
+  const act_t* dr;          // [B, T/2, 16]  gradient of the residual branch
+  const float* w;           // [16, 3]
+  const float* w_ds;        // [16]
+  const uint8_t* row_mask;  // [B]
+  float* dx;                // [B, T]
+  long long T;
+  float scale;              // 1 / loss scale of the incoming activation gradients
+};
+
+constexpr int kFirstDgradThreads = 256;
+
+__global__ void __launch_bounds__(kFirstDgradThreads) first_conv_dgrad_kernel(const FirstDgradArgs p) {
+  const int b = blockIdx.y;
+  const long long t = (long long)blockIdx.x * kFirstDgradThreads + threadIdx.x;
+  const size_t row = (size_t)b * p.T;
+  if (p.row_mask[b]) {  // block-uniform: a missing signal has no gradient
+    if (t < p.T) p.dx[row + t] = 0.0f;
+    return;
+  }
+  __shared__ float sw[16 * 3 + 16];
+  if (threadIdx.x < 64) sw[threadIdx.x] = threadIdx.x < 48 ? __ldg(p.w + threadIdx.x) : __ldg(p.w_ds + threadIdx.x - 48);
+  __syncthreads();
+  const int lane = threadIdx.x & 31;
+  auto load = [&](long long r, float* d) {
+    const uint4* q = reinterpret_cast<const uint4*>(p.dy1 + (row + r) * 16);
+    unpack8(__ldg(q), d);
+    unpack8(__ldg(q + 1), d + 8);
+  };
+  auto proj = [&](const float* d, int k) {
+    float s = 0.0f;
+#pragma unroll
+    for (int c = 0; c < 16; ++c) s = fmaf(sw[c * 3 + k], d[c], s);
+    return s;
+  };
+  float d[16];
+  float p0 = 0.0f, p1 = 0.0f, p2 = 0.0f;
+  if (t < p.T) {
+    load(t, d);
+    p0 = proj(d, 0);
+    p1 = proj(d, 1);
+    p2 = proj(d, 2);
+  }
+  float next0 = __shfl_down_sync(0xffffffffu, p0, 1);  // P0[t+1]
+  float prev2 = __shfl_up_sync(0xffffffffu, p2, 1);    // P2[t-1]
+  if (lane == 31) {
+    next0 = 0.0f;
+    if (t + 1 < p.T) {
+      load(t + 1, d);
+      next0 = proj(d, 0);
+    }
+  }
+  if (lane == 0) {
+    prev2 = 0.0f;
+    if (t > 0 && t - 1 < p.T) {
+      load(t - 1, d);
+      prev2 = proj(d, 2);
+    }
+  }
+  if (t >= p.T) return;
+  float g = next0 + p1 + prev2;
+  if ((t & 1) == 0) {
+    const uint4* q = reinterpret_cast<const uint4*>(p.dr + ((size_t)b * (p.T >> 1) + (t >> 1)) * 16);
+    unpack8(__ldg(q), d);
+    unpack8(__ldg(q + 1), d + 8);
+#pragma unroll
+    for (int c = 0; c < 16; ++c) g = fmaf(sw[48 + c], d[c], g);
+  }
+  p.dx[row + t] = isfinite(__ldg(p.x + row + t)) ? g * p.scale : 0.0f;
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // E/F/G. row-wise LayerNorm over 128 features (warp per row, lane = 4 features)
 //   fwd : h = LN(x) * g + b ; optional GELU ; optional (+ res -> GELU)                    [E, seq-mixer fwd]
@@ -365,7 +447,8 @@ __global__ void __launch_bounds__(256) row_ln_bwd_kernel(const RowLnArgs p) {
       *(reinterpret_cast<uint2*>(p.ds + r * 128) + lane) = w;
     }
   }
-  // dg / db: reduce the 8 warps of the block through shared memory, then one atomic per feature
+  // dg / db: reduce the 8 warps of the block through shared memory, then one atomic per feature (none when NULL)
+  if (!p.dg) return;
   __shared__ float red[8][256];
   const int w = threadIdx.x >> 5;
 #pragma unroll
@@ -636,7 +719,7 @@ __global__ void __launch_bounds__(256) tokens_bwd_kernel(const TokenArgs p) {
       *(reinterpret_cast<uint4*>(p.dz[j - 1] + n * 128) + ck) = pack8(v);
     }
   }
-  if (my_ck >= 0) {
+  if (my_ck >= 0 && p.dcls) {
 #pragma unroll
     for (int k = 0; k < 8; ++k) atomicAdd(&p.dcls[my_ck * 8 + k], cls_acc[k] * p.cls_scale);
   }
@@ -755,9 +838,11 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(const HeadArgs p) {
 #pragma unroll
   for (int k = 0; k < 8; ++k) {
     if (k < p.C) {
+      if (p.dw) {
 #pragma unroll
-      for (int q = 0; q < 4; ++q) atomicAdd(&p.dw[k * 128 + lane * 4 + q], aw[k][q]);
-      if (lane == 0) atomicAdd(&p.db[k], ab[k]);
+        for (int q = 0; q < 4; ++q) atomicAdd(&p.dw[k * 128 + lane * 4 + q], aw[k][q]);
+      }
+      if (lane == 0 && p.db) atomicAdd(&p.db[k], ab[k]);
     }
   }
 }
@@ -780,6 +865,14 @@ __global__ void __launch_bounds__(256) sumsq_kernel(const float* g, long long n,
     for (int j = 0; j < (int)(blockDim.x >> 5); ++j) t += red[j];
     atomicAdd(out, t);
   }
+}
+// out = max |g| (as the bit pattern of a non-negative float, so an integer atomicMax orders it); *out zeroed by the caller
+__global__ void __launch_bounds__(256) absmax_kernel(const float* g, long long n, unsigned int* out) {
+  float m = 0.0f;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    m = fmaxf(m, fabsf(g[i]));
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) atomicMax(out, __float_as_uint(m));
 }
 struct AdamWArgs {
   float* p; const float* g; float* m; float* v; long long n;

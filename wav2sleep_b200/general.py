@@ -13,7 +13,10 @@ Tensors are fp32, channels-last ``[B, L, C]``; weights stay in their PyTorch lay
 allocation and pure data movement (views, stack, index) only - every FLOP is in ``libw2s_b200.so``, except that autograd
 sums the gradients of a tensor that feeds two branches (residuals).
 
-Inference (``forward``, under ``no_grad``): BatchNorm uses its running statistics, dropout is the identity.  Training
+Inference (``forward``, under ``no_grad``): BatchNorm uses its running statistics, dropout is the identity.
+``forward_graph`` is the same eval-semantics forward with autograd on: what ``Wav2Sleep.forward`` runs in ``eval()`` when
+an input requires grad (attribution); the raw signal stays on the graph, its gradient is 0 at non-finite samples (the
+reference replaces them by 0, wav2sleep.py:150-151) and on missing rows.  Training
 (``forward_train``, what ``Wav2Sleep.forward`` calls under ``train()`` with grad): every primitive below is a
 ``torch.autograd.Function`` whose backward runs the kernels of ``csrc/general_bwd.cuh``, and dropout is applied where
 the reference applies it (attention weights, the FF / dropout1 / dropout2 dropouts of each mixer layer,
@@ -74,10 +77,12 @@ class _Conv(torch.autograd.Function):
         B, L_in, L_out, cin, cout, taps, stride, dil, pad_left, taps_major, raw = ctx.geo
         lib, g = ctx.eng.lib, _g(g)
         dx = dw = db = None
-        if ctx.needs_input_grad[0] and not raw:
+        if ctx.needs_input_grad[0]:
             dx = torch.zeros_like(xd)
             _lib.check(lib.w2s_gen_conv_dgrad(g.data_ptr(), wd.data_ptr(), dx.data_ptr(), _p(mask), B, L_in, L_out, cin, cout,
                                               taps, stride, dil, pad_left, taps_major, _stream()))
+            if raw:  # the forward read non-finite raw samples as 0: they have no gradient (data movement, no arithmetic)
+                dx = torch.where(torch.isfinite(xd), dx, torch.zeros_like(dx))
         want_b = ctx.has_bias and ctx.needs_input_grad[2]
         if ctx.needs_input_grad[1] or want_b:
             ws = torch.empty(taps * cin * cout + cout, dtype=torch.float64, device=g.device)
@@ -116,6 +121,37 @@ class _AffineAct(torch.autograd.Function):
         dsc = sums[..., 1].to(torch.float32).view(sc.shape) if need_sc else None
         dsh = sums[..., 0].to(torch.float32).view(sh.shape) if need_sh else None
         return din, dsc, dsh, dpre, None, None, None, None
+
+
+class _BatchNormConsts(torch.autograd.Function):
+    """Eval-mode BatchNorm1d as a per-channel affine: scale = w / sqrt(running_var + eps), shift = b - running_mean * scale
+    ([1, C] each), differentiable in w and b (the running statistics are buffers)."""
+
+    @staticmethod
+    def forward(ctx, weight, bias, eng, running_mean, running_var, eps):
+        Cc = running_mean.numel()
+        dev = running_mean.device
+        rm, rv = _f(running_mean), _f(running_var)
+        scale = torch.empty(1, Cc, dtype=torch.float32, device=dev)
+        shift = torch.empty(1, Cc, dtype=torch.float32, device=dev)
+        _lib.check(eng.lib.w2s_gen_norm_consts(None, _p(_f(weight)), _p(_f(bias)), rm.data_ptr(), rv.data_ptr(), scale.data_ptr(),
+                                               shift.data_ptr(), 1, Cc, 1, NORM_BATCH, 1, eps, _stream()))
+        ctx.save_for_backward(rm, rv)
+        ctx.eng, ctx.eps = eng, eps
+        return scale, shift
+
+    @staticmethod
+    def backward(ctx, dscale, dshift):
+        rm, rv = ctx.saved_tensors
+        Cc, dev = rm.numel(), rm.device
+        dscale = torch.zeros(Cc, dtype=torch.float32, device=dev) if dscale is None else _g(dscale)
+        dshift = torch.zeros(Cc, dtype=torch.float32, device=dev) if dshift is None else _g(dshift)
+        dw = torch.empty(Cc, dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
+        db = torch.empty(Cc, dtype=torch.float32, device=dev) if ctx.needs_input_grad[1] else None
+        if dw is not None or db is not None:
+            _lib.check(ctx.eng.lib.w2s_gen_bn_eval_bwd(dscale.data_ptr(), dshift.data_ptr(), rm.data_ptr(), rv.data_ptr(), _p(dw),
+                                                       _p(db), Cc, ctx.eps, _stream()))
+        return dw, db, None, None, None, None
 
 
 class _NormAct(torch.autograd.Function):
@@ -297,20 +333,14 @@ class GeneralEngine:
     def norm_act(self, y: Tensor, layer, act: str, mask=None, res=None) -> Tensor:
         """norm (by the layer's kind) -> activation of a conv output y [B, L, C]   (ConvLayer1D.forward, blocks.py:183-185)."""
         kind, norm = layer.norm_name, layer.norm
-        B, L, Cc = y.shape
         if kind is None:
             return self.affine_act(y, act, mask=mask)
         if kind in ("layer", "rms"):
             w = norm.weight.reshape(-1)
             b = norm.bias.reshape(-1) if kind == "layer" else None
             return self.rownorm(y, w, b, norm.eps, act, rms=int(kind == "rms"))
-        dev = y.device
         if kind == "batch":  # eval mode: running statistics (train-mode BatchNorm is not built, see model.py)
-            scale = torch.empty(1, Cc, dtype=torch.float32, device=dev)
-            shift = torch.empty(1, Cc, dtype=torch.float32, device=dev)
-            _lib.check(self.lib.w2s_gen_norm_consts(None, _p(_f(norm.weight)), _p(_f(norm.bias)), _f(norm.running_mean).data_ptr(),
-                                                    _f(norm.running_var).data_ptr(), scale.data_ptr(), shift.data_ptr(), 1, Cc, L,
-                                                    NORM_BATCH, 1, norm.eps, _stream()))
+            scale, shift = _BatchNormConsts.apply(norm.weight, norm.bias, self, norm.running_mean, norm.running_var, norm.eps)
             return self.affine_act(y, act, scale, shift, mask=mask, per_channel=1)
         if kind == "instance":
             affine = getattr(norm, "affine", False)
@@ -358,8 +388,8 @@ class GeneralEngine:
         if T % spe:
             raise ValueError(f"Input length {T} must be divisible by self.samples_per_epoch={spe}.")
         S = T // spe
-        xs = _f(x_BT)
-        mask = torch.isinf(xs[:, 0]).to(torch.uint8).contiguous()  # data-dependent control, no arithmetic
+        xs = x_BT.to(torch.float32).contiguous()  # stays on the autograd graph when the input requires grad
+        mask = torch.isinf(xs.detach()[:, 0]).to(torch.uint8).contiguous()  # data-dependent control, no arithmetic
         if enc.causal and enc.chunk_causal:  # every epoch is its own sample (wav2sleep.py:248-255)
             a = xs.view(B * S, spe, 1)
             m = mask.repeat_interleave(S).contiguous()
@@ -430,6 +460,11 @@ class GeneralEngine:
     @torch.no_grad()
     def forward(self, x: dict[str, Tensor]) -> Tensor:
         """Inference (eval semantics: running BatchNorm statistics, no dropout)."""
+        self._seed = None
+        return self._forward(x)
+
+    def forward_graph(self, x: dict[str, Tensor]) -> Tensor:
+        """The inference forward (eval semantics) with autograd on, for gradients with respect to the inputs."""
         self._seed = None
         return self._forward(x)
 

@@ -21,7 +21,7 @@ activations relu / leaky / silu / linear, ``embed_signals``, ``register_tokens >
 results as the reference to fp32 accuracy, not tuned.  ``norm='weight'`` (a parametrisation with different state_dict
 keys) is the one option that raises ``NotImplementedError``; a model with BatchNorm layers (norm='batch', SleepPPGNet)
 runs inference but raises ``NotImplementedError`` under ``train()`` with grad (train-mode batch statistics are not
-built).
+built); in ``eval()`` it is differentiable, in its inputs and its parameters.
 """
 from __future__ import annotations
 
@@ -377,16 +377,24 @@ class Wav2Sleep(nn.Module):
 
         Under ``train()`` with grad enabled the logits carry a grad_fn whose backward runs the CUDA backward pass
         (dropout with counter-based masks, see training.py; for the non-default options the general path's autograd
-        Functions, general.py); otherwise the inference kernels run."""
+        Functions, general.py).  So do they, in ``train()`` or ``eval()``, when an input tensor requires grad: then
+        ``x[name].grad`` receives d(objective)/dx (0 at non-finite samples and on missing rows), as with the reference,
+        and an ``eval()`` graph has eval semantics (no dropout, BatchNorm on its running statistics).  Otherwise the
+        inference kernels run."""
+        grad_on = torch.is_grad_enabled()
+        input_grad = grad_on and isinstance(x, dict) and any(isinstance(t, Tensor) and t.requires_grad for t in x.values())
+        train_grad = self.training and grad_on and any(p.requires_grad for p in self.parameters())
         if not self.fast_path:
-            if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+            if train_grad or (input_grad and self.training):
                 if any(isinstance(mod, nn.BatchNorm1d) for mod in self.modules()):
                     raise NotImplementedError("wav2sleep_b200: training a model with BatchNorm layers (train-mode batch "
                                               "statistics and running-statistics updates) is not built on the CUDA path; "
                                               "eval-mode inference is")
                 return self._get_general().forward_train(x)
+            if input_grad:
+                return self._get_general().forward_graph(x)
             return self._get_general().forward(x)
-        if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+        if train_grad or input_grad:
             from .training import forward_with_grad
             return forward_with_grad(self, x)
         if self.training and (self.epoch_mixer.dropout > 0 or any(b.dropout.p > 0 for b in

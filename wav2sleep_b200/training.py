@@ -20,11 +20,20 @@ runs on gradients multiplied by a power of two (``TrainEngine.loss_scale``; defa
 the loss were 4x the *sum* over epochs, which centres the activation gradients in fp16's range for any batch size), and
 every kernel that accumulates a parameter gradient multiplies by the inverse - fp32 parameter gradients are unscaled,
 exactly (powers of two), and nothing outside this file sees the scale.
+
+Input gradients (saliency, integrated gradients: ``x[name].requires_grad_()`` before the forward) come out of the same
+backward: block 0's data gradient into the raw signal is ``w2s_first_conv_dgrad``.  Their objectives are not a mean cross
+entropy - one logit or a class's summed logits give d(objective)/d(logits) of order 1, which the batch-size rule above
+would push past fp16's 65 504 - so a backward that produces input gradients without an explicit ``loss_scale`` picks
+the power of two that brings max|dlogits| into [4, 8) (one device reduction, one scalar read back).  Only the requested
+work runs: parameters with ``requires_grad=False`` get no buffer and no weight-gradient launch, and an encoder whose
+parameters are frozen and whose signal needs no gradient is not back-propagated at all.
 """
 from __future__ import annotations
 
 import contextlib
 import ctypes as C
+import math
 
 import torch
 from torch import Tensor
@@ -65,6 +74,7 @@ class TrainEngine(ForwardEngine):
         self.loss_scale = None    # power of two applied to the fp16 activation gradients; None = from B*S (see below)
         self._inv_scale = 1.0
         self.last_loss_scale = 1.0
+        self.input_grads = {}     # signal -> fp32 [B, T] d(objective)/dx of the last backward that was asked for them
 
     @staticmethod
     def auto_loss_scale(n_epochs: int) -> float:
@@ -73,6 +83,13 @@ class TrainEngine(ForwardEngine):
         middle of fp16's normal range [6e-5, 65504], whatever the batch size."""
         k = max(int(n_epochs) - 1, 0).bit_length() + 2
         return float(2 ** min(k, 24))
+
+    @staticmethod
+    def attribution_loss_scale(max_abs_dlogits: float) -> float:
+        """2^k with max|dlogits| * 2^k in [4, 8), k <= 24: the scale of a backward whose objective is not a mean cross
+        entropy (a logit, a class's summed logits), where the batch-size rule would overflow fp16."""
+        k = 3 - math.frexp(max_abs_dlogits)[1]
+        return math.ldexp(1.0, min(k, 24))
 
     def _encoder_streams(self, device, n):
         """n side streams (one per signal encoder) that have been made to wait for the current stream, or None."""
@@ -222,6 +239,8 @@ class TrainEngine(ForwardEngine):
 
     def gemm_tn(self, X, Y, Cbuf, M, N, B, LX, LY, ldc_m, ldc_n, y_stride=1, y_offset=0, row_mask=None, c_off=0, taps=1,
                 ldc_t=0, tap_stride=1):
+        if Cbuf is None:  # frozen parameter
+            return
         _lib.check(self.lib.w2s_gemm_tn(X.data_ptr(), Y.data_ptr(), Cbuf.data_ptr() + 4 * c_off, M, N, taps, tap_stride, B,
                                         LX, LY, y_stride, y_offset, ldc_m, ldc_n, ldc_t, self._inv_scale, _p(row_mask),
                                         self._wgrad_stream(X, Y, Cbuf, row_mask)))
@@ -235,18 +254,26 @@ class TrainEngine(ForwardEngine):
     def ln_bwd(self, x, g, b, dout, dg, db, rows, gelu, eps, res=None, dadd=None, want_ds=False):
         dx = torch.empty_like(x)
         ds = torch.empty_like(x) if want_ds else None
+        if (dg is None) != (db is None):  # one of the two frozen: the kernel computes both or neither
+            dg = torch.zeros_like(g) if dg is None else dg
+            db = torch.zeros_like(b) if db is None else db
         _lib.check(self.lib.w2s_row_ln_bwd(x.data_ptr(), _p(res), g.data_ptr(), b.data_ptr(), dout.data_ptr(), _p(dadd),
-                                           dx.data_ptr(), _p(ds), dg.data_ptr(), db.data_ptr(), rows, gelu, eps,
+                                           dx.data_ptr(), _p(ds), _p(dg), _p(db), rows, gelu, eps,
                                            self._inv_scale, _stream()))
         return dx, ds
 
     def colsum(self, x, out, rows, Cc, row_stride=1, row_offset=0, row_mask=None, rows_per_sample=0, out_off=0):
+        if out is None:  # frozen parameter
+            return
         _lib.check(self.lib.w2s_colsum(x.data_ptr(), out.data_ptr() + 4 * out_off, rows, Cc, row_stride, row_offset,
                                        _p(row_mask), rows_per_sample, self._inv_scale, self._wgrad_stream(x, out, row_mask)))
 
     # ------------------------------------------------------------------ gradients storage
-    def _grad(self, p: Tensor) -> Tensor:
-        """fp32 gradient buffer of a parameter, zeroed at the start of every backward, accumulated by the kernels."""
+    def _grad(self, p: Tensor) -> Tensor | None:
+        """fp32 gradient buffer of a parameter, zeroed at the start of every backward, accumulated by the kernels; None for
+        a parameter that does not require grad (its weight-gradient launches are skipped)."""
+        if not p.requires_grad:
+            return None
         g = self.grads.get(id(p))
         if g is None:
             if p.grad is not None and p.grad.dtype == torch.float32 and p.grad.is_contiguous():
@@ -426,9 +453,11 @@ class TrainEngine(ForwardEngine):
 
     # ================================================================== backward
     @torch.no_grad()
-    def backward(self, dlogits: Tensor, saved: dict | None = None) -> dict[int, Tensor]:
+    def backward(self, dlogits: Tensor, saved: dict | None = None, inputs=()) -> dict[int, Tensor]:
         """Back-propagates d(loss)/d(logits) through a saved forward (``saved``: what forward_train returned; default:
-        the most recent forward); returns {id(param): fp32 grad}.  A saved forward can be back-propagated once."""
+        the most recent forward); returns {id(param): fp32 grad} for the parameters that require grad.  ``inputs``:
+        signals whose d(loss)/dx is wanted as well, left in ``self.input_grads`` (fp32 [B, T]).  A saved forward can be
+        back-propagated once."""
         sv, lib, m = (self.saved if saved is None else saved), self.lib, self.model
         if sv is None:
             raise RuntimeError("backward called without a preceding forward_train")
@@ -439,19 +468,32 @@ class TrainEngine(ForwardEngine):
         self.grads = {}
         self.direct = set()
         self._wg = None
-        scale = float(self.loss_scale) if self.loss_scale is not None else self.auto_loss_scale(N)
-        if scale <= 0 or (scale != 2.0 ** round(__import__("math").log2(scale))):
-            raise ValueError(f"loss_scale must be a positive power of two, got {scale}")
-        self.last_loss_scale, self._inv_scale = scale, 1.0 / scale
+        inputs = set(inputs)
+        self.input_grads = {}
         with torch.cuda.device(device):
+            dlogits = dlogits.detach().to(torch.float32).contiguous()
+            if self.loss_scale is not None:
+                scale = float(self.loss_scale)
+            elif inputs:
+                amax = torch.empty(1, dtype=torch.float32, device=device)
+                _lib.check(lib.w2s_absmax(dlogits.data_ptr(), dlogits.numel(), amax.data_ptr(), _stream()))
+                amax = amax.item()
+                if amax == 0.0:  # every gradient is exactly zero: nothing to launch
+                    return self._zero_backward(sv, inputs)
+                scale = self.attribution_loss_scale(amax)
+            else:
+                scale = self.auto_loss_scale(N)
+            if scale <= 0 or (scale != 2.0 ** round(math.log2(scale))):
+                raise ValueError(f"loss_scale must be a positive power of two, got {scale}")
+            self.last_loss_scale, self._inv_scale = scale, 1.0 / scale
             st = _stream()
             G = self._grad
-            dlogits = dlogits.detach().to(torch.float32).contiguous()
+            Gv = lambda p: None if G(p) is None else G(p).view(-1)
             self._wg = self._wg_streams.setdefault(str(device), torch.cuda.Stream(device=device))
             # ---- classifier ----
             dfeat = torch.empty(N, 128, dtype=F16, device=device)
             _lib.check(lib.w2s_head_bwd(sv["feat"].data_ptr(), sv["wc"].data_ptr(), dlogits.data_ptr(), dfeat.data_ptr(),
-                                        G(m.classifier.weight).data_ptr(), G(m.classifier.bias).data_ptr(), N,
+                                        _p(G(m.classifier.weight)), _p(G(m.classifier.bias)), N,
                                         m.num_classes, scale, st))
             # ---- sequence mixer ----
             dout = dfeat
@@ -461,7 +503,7 @@ class TrainEngine(ForwardEngine):
                 ds = None
                 for k in reversed(range(nl)):
                     lr, layer = rec["layers"][k], blk.conv_layers[k]
-                    dg, db = G(layer.norm.weight).view(-1), G(layer.norm.bias).view(-1)
+                    dg, db = Gv(layer.norm.weight), Gv(layer.norm.bias)
                     last = k == nl - 1
                     if last and "t" in lr:  # dropout between the layers and the residual add
                         ds = torch.empty(N, 128, dtype=F16, device=device)
@@ -539,7 +581,7 @@ class TrainEngine(ForwardEngine):
             dzs = (C.c_void_p * len(names))(*[dz[n].data_ptr() for n in names])
             ms = (C.c_void_p * len(names))(*[sv["enc"][n]["mask"].data_ptr() for n in names])
             # register_tokens is [1, 1, 128, 1]: with no extra register tokens its gradient is the 128 CLS sums
-            _lib.check(lib.w2s_tokens_bwd(dx.data_ptr(), dzs, ms, G(mix.register_tokens).data_ptr(), N, S, len(names),
+            _lib.check(lib.w2s_tokens_bwd(dx.data_ptr(), dzs, ms, _p(G(mix.register_tokens)), N, S, len(names),
                                           self._inv_scale, st))
             # ---- encoders ----
             if self._wg is not None:  # the side stream's weight gradients are part of the "tail" bucket
@@ -559,11 +601,18 @@ class TrainEngine(ForwardEngine):
                 pending[smap[n]] = pending.get(smap[n], 0) + 1
             shared = len(set(smap[n] for n in order)) < len(order)  # a shared encoder: its passes stay in stream order
             streams = None if shared else self._encoder_streams(device, len(order))
+            main = torch.cuda.current_stream(device)
             for si, n in enumerate(order):
                 with (torch.cuda.stream(streams[si]) if streams is not None else contextlib.nullcontext()):
                     if streams is not None:
                         dz[n].record_stream(streams[si])
-                    self._encoder_backward(sv["enc"][n], dz[n], B, S)
+                    enc = sv["enc"][n]["enc"]
+                    if n in inputs or any(p.requires_grad for p in enc.parameters()):
+                        dxn = self._encoder_backward(sv["enc"][n], dz[n], B, S, want_dx=n in inputs)
+                        if dxn is not None:
+                            if streams is not None:
+                                dxn.record_stream(main)
+                            self.input_grads[n] = dxn
                     sv["enc"][n] = None  # release this encoder's activations
                     pending[smap[n]] -= 1
                     if pending[smap[n]] == 0:
@@ -579,7 +628,24 @@ class TrainEngine(ForwardEngine):
                 self.saved = None
         return self.grads
 
-    def _encoder_backward(self, e, dz, B, S):
+    def _zero_backward(self, sv, inputs):
+        """d(objective)/d(logits) is exactly zero: so is every gradient.  No kernel runs; the bucket hooks still fire."""
+        B, device = sv["B"], sv["device"]
+        self.grads = {id(p): torch.zeros_like(p, dtype=torch.float32) for p in self.model.parameters() if p.requires_grad}
+        self.input_grads = {n: torch.zeros(B, sv["enc"][n]["T"], dtype=torch.float32, device=device) for n in inputs}
+        smap = self.model.signal_encoders.signal_map
+        for bucket in ["tail"] + sorted({"encoder:" + smap[n] for n in sv["names"]}) + ["encoders"]:
+            for hook in self.bucket_hooks:
+                hook(bucket)
+        sv["consumed"] = True
+        for k in ("layers", "seq", "feat", "key_mask", "enc"):
+            sv.pop(k, None)
+        if self.saved is sv:
+            self.saved = None
+        self.last_loss_scale, self._inv_scale = 1.0, 1.0
+        return self.grads
+
+    def _encoder_backward(self, e, dz, B, S, want_dx=False):
         lib, st, G = self.lib, _stream(), self._grad
         enc, mask, tw, device = e["enc"], e["mask"], e["tw"], dz.device
         eps = enc.norm_eps
@@ -650,10 +716,20 @@ class TrainEngine(ForwardEngine):
             dn = (dxh, bk["y1"], bk["s1"], sums, 0) if fuse1 else None
             del dxh
             if i == 0:
-                _lib.check(lib.w2s_first_conv_wgrad(e["x"].data_ptr(), dy1.data_ptr(), dr.data_ptr(),
-                                                    G(blk.conv1.conv.weight).data_ptr(), G(blk.downsample.weight).data_ptr(),
-                                                    mask.data_ptr(), B, L, self._inv_scale, st))
-                break
+                dw1, dwds = G(blk.conv1.conv.weight), G(blk.downsample.weight)
+                if dw1 is not None or dwds is not None:  # the kernel computes both: a frozen one goes to scratch
+                    dw1 = torch.zeros(16, 1, 3, device=device) if dw1 is None else dw1
+                    dwds = torch.zeros(16, 1, 1, device=device) if dwds is None else dwds
+                    _lib.check(lib.w2s_first_conv_wgrad(e["x"].data_ptr(), dy1.data_ptr(), dr.data_ptr(), dw1.data_ptr(),
+                                                        dwds.data_ptr(), mask.data_ptr(), B, L, self._inv_scale, st))
+                if want_dx:
+                    dx = torch.empty(B, L, dtype=torch.float32, device=device)
+                    _lib.check(lib.w2s_first_conv_dgrad(e["x"].data_ptr(), dy1.data_ptr(), dr.data_ptr(),
+                                                        self._f32(blk.conv1.conv.weight).data_ptr(),
+                                                        self._f32(blk.downsample.weight).data_ptr(), mask.data_ptr(),
+                                                        dx.data_ptr(), B, L, self._inv_scale, st))
+                    return dx
+                return None
             pb = blocks[i - 1]
             Ci = pb["C"]
             tmp = torch.zeros(B, L, Ci, dtype=F16, device=device)
@@ -674,20 +750,26 @@ class TrainEngine(ForwardEngine):
 
 
 class _TrainFn(torch.autograd.Function):
-    """autograd bridge: ``logits = model(x)`` in train mode gets a grad_fn whose backward runs the CUDA backward."""
+    """autograd bridge: ``logits = model(x)`` gets a grad_fn whose backward runs the CUDA backward.  The signals are
+    inputs of the graph (in ``names`` order, then the parameters), so ``x[name].grad`` receives d(objective)/dx where
+    ``x[name].requires_grad``."""
 
     @staticmethod
-    def forward(ctx, engine, x, *params):
-        ctx.engine = engine
-        ctx.params = params
-        logits, ctx.saved = engine.forward_train(x, return_saved=True)  # per-graph state, like autograd's saved tensors
+    def forward(ctx, engine, names, *tensors):
+        n = len(names)
+        ctx.engine, ctx.names = engine, names
+        ctx.dtypes, ctx.params = [t.dtype for t in tensors[:n]], tensors[n:]
+        # per-graph state, like autograd's saved tensors
+        logits, ctx.saved = engine.forward_train(dict(zip(names, tensors[:n])), return_saved=True)
         return logits
 
     @staticmethod
     def backward(ctx, dlogits):
-        grads = ctx.engine.backward(dlogits, ctx.saved)
+        wanted = [name for i, name in enumerate(ctx.names) if ctx.needs_input_grad[2 + i]]
+        grads = ctx.engine.backward(dlogits, ctx.saved, inputs=wanted)
+        dx = ctx.engine.input_grads
         ctx.saved = None
-        out = []
+        out = [dx[name].to(dt) if name in dx else None for name, dt in zip(ctx.names, ctx.dtypes)]
         for p in ctx.params:
             g = grads.get(id(p))
             direct = id(p) in ctx.engine.direct  # already accumulated into p.grad by the kernels
@@ -698,4 +780,5 @@ class _TrainFn(torch.autograd.Function):
 def forward_with_grad(model, x: dict[str, Tensor]) -> Tensor:
     eng = model._get_train_engine()
     params = tuple(p for p in model.parameters() if p.requires_grad)
-    return _TrainFn.apply(eng, x, *params)
+    names = tuple(x.keys())
+    return _TrainFn.apply(eng, names, *(x[n] for n in names), *params)
