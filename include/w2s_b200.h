@@ -405,6 +405,16 @@ int w2s_gen_attn(const float* q, const float* k, const float* v, float* o, const
  * (the parameters behind w2s_gen_norm_consts' batch-mode scale / shift; either output may be NULL; ABI v7). */
 int w2s_gen_bn_eval_bwd(const float* dscale, const float* dshift, const float* running_mean, const float* running_var,
                         float* dweight, float* dbias, int C, float eps, void* stream);
+/* Train-mode BatchNorm1d statistics (ABI v8): stats[c] = fp64 (sum, sum of squares) over all rows of a [rows, C] fp32 tensor
+ * (a channels-last [B, L, C] tensor is rows = B * L; stats is then what w2s_gen_norm_consts with W2S_NORM_INSTANCE, B = 1,
+ * L = rows and w2s_gen_norm_bwd with B = 1, groups = C read).  Zeroes stats itself; refuses rows < 1 and C < 1. */
+int w2s_gen_bn_stats(const float* x, double* stats, long long rows, int C, void* stream);
+/* BatchNorm1d's running-statistics update of one training forward from those stats over n values per channel (ABI v8):
+ * *num_batches_tracked += 1 (int64, on the device); f = momentum, or 1 / num_batches_tracked when momentum < 0
+ * (momentum=None); running_mean = (1 - f) running_mean + f mean, running_var = (1 - f) running_var + f var n / (n - 1)
+ * (unbiased variance).  fp64 arithmetic (momentum is a double, as PyTorch's Python float), fp32 buffers.  Refuses n < 2, as PyTorch does. */
+int w2s_gen_bn_update_running(const double* stats, long long n, float* running_mean, float* running_var,
+                              long long* num_batches_tracked, double momentum, int C, void* stream);
 int w2s_gen_conv_dgrad(const float* dout, const float* w, float* din, const uint8_t* row_mask, int B, int L_in, int L_out, int cin,
                        int cout, int taps, int stride, int dil, int pad_left, int taps_major, void* stream);
 /* dw[co, ci, t] = sum_{b, lo} dout * in (layout of w2s_gen_conv's w), dbias[co] = sum dout; non-finite raw samples read as 0

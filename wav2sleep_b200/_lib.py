@@ -27,7 +27,7 @@ STREAM_MAX_LAYERS = 32
 STREAM_MAX_DILATIONS = 16
 STREAM_MAX_KERNEL = 16
 STREAM_MAX_FEATURES = 256
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 PRO_NONE, PRO_NORM, PRO_NORM_RES, PRO_FIR, PRO_NORM_RES_X, PRO_DNORM = 0, 1, 2, 3, 4, 5
 EPI_STATS, EPI_BIAS_GELU, EPI_LN_GELU, EPI_LN_GELU_RES, EPI_PLAIN, EPI_ACT_BWD = 0, 1, 2, 3, 4, 5
@@ -209,6 +209,9 @@ SYMBOLS = {
     "w2s_gen_rownorm_bwd": (C.c_int, [C.c_void_p] * 8 + [C.c_longlong, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p]),
     "w2s_gen_attn_bwd": (C.c_int, [C.c_void_p] * 8 + [C.c_int] * 5 + [C.c_float, C.c_uint64, C.c_uint32, C.c_void_p]),
     "w2s_gen_bn_eval_bwd": (C.c_int, [C.c_void_p] * 6 + [C.c_int, C.c_float, C.c_void_p]),
+    "w2s_gen_bn_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_void_p]),
+    "w2s_gen_bn_update_running": (C.c_int, [C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_int,
+                                            C.c_void_p]),
     "w2s_gen_dropout": (C.c_int, [C.c_void_p] * 3 + [C.c_longlong, C.c_float, C.c_uint64, C.c_uint32, C.c_void_p]),
     "w2s_gen_seq_stream_step": (C.c_int, [C.POINTER(SeqStreamDesc), C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_longlong,
                                           C.c_void_p]),

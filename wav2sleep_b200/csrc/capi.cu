@@ -530,7 +530,7 @@ int check_encoder_desc(const w2s_encoder_desc* d) {
 
 extern "C" {
 
-int w2s_abi_version(void) { return 7; }
+int w2s_abi_version(void) { return 8; }
 const char* w2s_last_error(void) { return g_err.c_str(); }
 
 int w2s_conv_uses_split(int cin, int cout) { return (cin <= 16 && cout <= 16) ? 1 : 0; }
@@ -1545,6 +1545,31 @@ int w2s_gen_bn_eval_bwd(const float* dscale, const float* dshift, const float* r
   gen::bn_eval_bwd_kernel<<<ew_grid(Cc), 256, 0, (cudaStream_t)stream>>>(dscale, dshift, running_mean, running_var, dweight,
                                                                           dbias, Cc, eps);
   W2S_LAUNCH_CHECK("gen_bn_eval_bwd");
+}
+int w2s_gen_bn_stats(const float* x, double* stats, long long rows, int Cc, void* stream) {
+  if (!x || !stats || rows < 1 || Cc < 1) return fail("gen_bn_stats: bad arguments (rows=%lld C=%d)", rows, Cc);
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(stats, 0, (size_t)Cc * 2 * sizeof(double), st);
+  if (e != cudaSuccess) return cuda_fail(e, "gen_bn_stats memset");
+  // blocks: enough row steps to keep 8 blocks on every SM, never more than there are steps
+  const int cw = Cc < gen::kBnThreads ? Cc : gen::kBnThreads;
+  const long long step = (long long)(gen::kBnThreads / cw) * gen::kBnUnroll;
+  long long g = (rows + step - 1) / step;
+  if (g > 8LL * sm_count()) g = 8LL * sm_count();
+  LaunchScope scope(st, "gen_bn_stats", (double)rows * Cc * 4.0, (double)rows * Cc * 3.0);
+  gen::bn_stats_kernel<<<(unsigned)g, gen::kBnThreads, 0, st>>>(x, stats, rows, Cc);
+  gen::bn_stats_finalize_kernel<<<ew_grid(Cc), 256, 0, st>>>(x, stats, rows, Cc);
+  W2S_LAUNCH_CHECK("gen_bn_stats");
+}
+int w2s_gen_bn_update_running(const double* stats, long long n, float* running_mean, float* running_var,
+                              long long* num_batches_tracked, double momentum, int Cc, void* stream) {
+  if (!stats || !running_mean || !running_var || !num_batches_tracked || Cc < 1)
+    return fail("gen_bn_update_running: bad arguments (C=%d)", Cc);
+  if (n < 2) return fail("gen_bn_update_running: Expected more than 1 value per channel when training, got n=%lld", n);
+  LaunchScope scope((cudaStream_t)stream, "gen_bn_running", (double)Cc * 32.0 + 16.0, 0);
+  gen::bn_update_running_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(stats, n, running_mean, running_var,
+                                                                      num_batches_tracked, momentum, Cc);
+  W2S_LAUNCH_CHECK("gen_bn_update_running");
 }
 int w2s_gen_dropout(const float* x, float* out, uint8_t* mask_out, long long n, float p, uint64_t seed, uint32_t site,
                     void* stream) {

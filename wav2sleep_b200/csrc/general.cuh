@@ -95,6 +95,94 @@ __global__ void __launch_bounds__(256) stats_kernel(const float* x, double* stat
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// train-mode BatchNorm statistics: per-channel (sum, sum of squares) over all rows of a [rows, C] tensor (fp64).
+// A channels-last [B, L, C] tensor viewed as [B * L, C] is BatchNorm's statistics group.  The block reads `span` =
+// (blockDim / C) whole rows per step (C > blockDim: one blockDim-wide channel chunk of one row), so thread t always
+// holds channel c0 + t % C and the warps walk contiguous bytes for any C.  kBnUnroll independent loads per thread
+// are in flight before they are accumulated (fp64 per thread), then the block folds its rows in shared memory and
+// adds one fp64 pair per channel to `stats` (zeroed by the caller) - one atomic per (block, channel).
+// The sums are shifted by K = x[0, c] (d = x - K and d * d are exact in fp64): for |mean| >> std, sum x^2 would round
+// at the scale of n * mean^2 in every cross-block addition, while sum d^2 rounds at the scale of n * var.
+// bn_stats_finalize_kernel turns the shifted sums back into (sum x, sum x^2) once.
+// ------------------------------------------------------------------------------------------------------------
+constexpr int kBnThreads = 256, kBnUnroll = 8;
+__global__ void __launch_bounds__(kBnThreads) bn_stats_kernel(const float* __restrict__ x, double* __restrict__ stats,
+                                                              long long rows, int C) {
+  __shared__ double r0[kBnThreads], r1[kBnThreads];
+  const int t = threadIdx.x;
+  for (int c0 = 0; c0 < C; c0 += kBnThreads) {
+    const int cw = min(C - c0, kBnThreads);   // channels of this chunk
+    const int span = kBnThreads / cw;          // rows per step
+    const int ty = t / cw, tx = t % cw;
+    const bool active = ty < span;
+    double s0 = 0.0, s1 = 0.0;
+    const long long step = (long long)span * kBnUnroll;
+    if (active) {
+      const float k = x[c0 + tx];
+      for (long long r = (long long)blockIdx.x * step + ty; r < rows; r += (long long)gridDim.x * step) {
+        float v[kBnUnroll];
+#pragma unroll
+        for (int u = 0; u < kBnUnroll; ++u) {
+          const long long ru = r + (long long)u * span;
+          v[u] = ru < rows ? x[ru * C + c0 + tx] : k;
+        }
+#pragma unroll
+        for (int u = 0; u < kBnUnroll; ++u) {
+          const double d = (double)v[u] - (double)k;
+          s0 += d;
+          s1 = fma(d, d, s1);
+        }
+      }
+    }
+    r0[t] = s0;
+    r1[t] = s1;
+    __syncthreads();
+    if (t < cw) {
+      double a0 = 0.0, a1 = 0.0;
+      for (int k = 0; k < span; ++k) {
+        a0 += r0[k * cw + t];
+        a1 += r1[k * cw + t];
+      }
+      atomicAdd(&stats[(size_t)(c0 + t) * 2], a0);
+      atomicAdd(&stats[(size_t)(c0 + t) * 2 + 1], a1);
+    }
+    __syncthreads();
+  }
+}
+// (sum d, sum d^2) with d = x - K  ->  (sum x, sum x^2) = (S1 + n K, S2 + 2 K S1 + n K^2)
+__global__ void __launch_bounds__(256) bn_stats_finalize_kernel(const float* __restrict__ x, double* __restrict__ stats,
+                                                                long long rows, int C) {
+  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < C; c += gridDim.x * blockDim.x) {
+    const double k = x[c], n = (double)rows;
+    const double s1 = stats[(size_t)c * 2], s2 = stats[(size_t)c * 2 + 1];
+    stats[(size_t)c * 2] = fma(n, k, s1);
+    stats[(size_t)c * 2 + 1] = fma(n * k, k, fma(2.0 * k, s1, s2));
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// BatchNorm1d running-statistics update of one training forward (torch.nn.functional.batch_norm, training=True):
+//   num_batches_tracked += 1;  f = momentum, or 1 / num_batches_tracked when momentum < 0 (momentum=None);
+//   running_mean = (1 - f) running_mean + f mean,  running_var = (1 - f) running_var + f var * n / (n - 1).
+// fp64 arithmetic, fp32 buffers.  One block: every thread reads the counter before thread 0 writes it back.
+// ------------------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) bn_update_running_kernel(const double* __restrict__ stats, long long n,
+                                                                float* running_mean, float* running_var,
+                                                                long long* num_batches_tracked, double momentum, int C) {
+  const long long tracked = *num_batches_tracked + 1;
+  __syncthreads();
+  if (threadIdx.x == 0) *num_batches_tracked = tracked;
+  const double f = momentum < 0.0 ? 1.0 / (double)tracked : momentum;
+  const double inv_n = 1.0 / (double)n, unbias = (double)n / (double)(n - 1);
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    const double mean = stats[(size_t)c * 2] * inv_n;
+    const double var = fmax(stats[(size_t)c * 2 + 1] * inv_n - mean * mean, 0.0);
+    running_mean[c] = (float)((1.0 - f) * (double)running_mean[c] + f * mean);
+    running_var[c] = (float)((1.0 - f) * (double)running_var[c] + f * var * unbias);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // normalisation constants: scale[b, c], shift[b, c] with y = x * scale + shift
 //   NORM_INSTANCE  : nn.InstanceNorm1d (biased variance over L, no affine)              utils.py:89-92
 //   NORM_GROUP     : nn.GroupNorm(groups) (statistics over L x C/groups, affine w, b)   utils.py:38-58

@@ -21,10 +21,14 @@ reference replaces them by 0, wav2sleep.py:150-151) and on missing rows.  Traini
 ``torch.autograd.Function`` whose backward runs the kernels of ``csrc/general_bwd.cuh``, and dropout is applied where
 the reference applies it (attention weights, the FF / dropout1 / dropout2 dropouts of each mixer layer,
 DilatedConvBlock.dropout) with counter-based masks: ``dropout_seed`` (None: drawn from torch's CPU generator per step)
-and the fixed site numbers of training.py; ``dropout_mask`` returns a site's keep decisions.  Train-mode BatchNorm is
-not built (model.py raises before getting here).
+and the fixed site numbers of training.py; ``dropout_mask`` returns a site's keep decisions.  BatchNorm in a training
+forward normalises with the batch statistics and updates the running statistics (``_BatchNormTrainAct``); SleepPPGNet
+trains through it, while model.py still refuses to train Wav2Sleep models with BatchNorm layers (their masked samples
+would need the reference's zero-filled semantics, which the row-masked kernels do not have).
 """
 from __future__ import annotations
+
+import contextlib
 
 import torch
 from torch import Tensor, nn
@@ -152,6 +156,62 @@ class _BatchNormConsts(torch.autograd.Function):
             _lib.check(ctx.eng.lib.w2s_gen_bn_eval_bwd(dscale.data_ptr(), dshift.data_ptr(), rm.data_ptr(), rv.data_ptr(), _p(dw),
                                                        _p(db), Cc, ctx.eps, _stream()))
         return dw, db, None, None, None, None
+
+
+class _BatchNormTrainAct(torch.autograd.Function):
+    """Train-mode BatchNorm1d + activation of a conv output y [B, L, C].  Viewed as [1, B * L, C], BatchNorm's statistics
+    group is an InstanceNorm's: w2s_gen_bn_stats gives the per-channel sums over every row, norm_consts (instance mode,
+    biased variance) scale = w * rstd and shift = b - mean * w * rstd, affine_act applies them, and the backward is
+    the InstanceNorm backward of that view (affine_act_bwd -> norm_bwd with groups = C).  The module's running
+    statistics are updated in place, once per forward, on the forward's stream (unbiased variance, as PyTorch)."""
+
+    @staticmethod
+    def forward(ctx, y, weight, bias, eng, norm, act):
+        B, L, Cc = y.shape
+        rows = B * L
+        if rows >= 2 ** 31:
+            raise ValueError(f"train-mode BatchNorm over {rows} rows: at most 2^31 - 1")
+        lib, dev = eng.lib, y.device
+        yd, w, b = _f(y), _f(weight), _f(bias)
+        stats = torch.empty(1, Cc, 2, dtype=torch.float64, device=dev)
+        _lib.check(lib.w2s_gen_bn_stats(yd.data_ptr(), stats.data_ptr(), rows, Cc, _stream()))
+        if norm.track_running_stats and norm.running_mean is not None:
+            for buf in (norm.running_mean, norm.running_var):
+                if buf.dtype != torch.float32 or not buf.is_contiguous():
+                    raise ValueError("BatchNorm running statistics must be contiguous fp32")
+            momentum = -1.0 if norm.momentum is None else float(norm.momentum)
+            _lib.check(lib.w2s_gen_bn_update_running(stats.data_ptr(), rows, norm.running_mean.data_ptr(),
+                                                     norm.running_var.data_ptr(), norm.num_batches_tracked.data_ptr(),
+                                                     momentum, Cc, _stream()))
+        scale = torch.empty(1, Cc, dtype=torch.float32, device=dev)
+        shift = torch.empty(1, Cc, dtype=torch.float32, device=dev)
+        _lib.check(lib.w2s_gen_norm_consts(stats.data_ptr(), _p(w), _p(b), None, None, scale.data_ptr(), shift.data_ptr(), 1,
+                                           Cc, rows, NORM_INSTANCE, 1, norm.eps, _stream()))
+        out = torch.empty_like(yd)
+        _lib.check(lib.w2s_gen_affine_act(yd.data_ptr(), scale.data_ptr(), shift.data_ptr(), None, out.data_ptr(), None, 1,
+                                          rows, Cc, ACT[act], 1, _stream()))
+        ctx.save_for_backward(yd, w, stats, scale, shift)
+        ctx.eng, ctx.eps, ctx.act = eng, norm.eps, act
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        yd, w, stats, scale, shift = ctx.saved_tensors
+        B, L, Cc = yd.shape
+        rows = B * L
+        lib, g, dev = ctx.eng.lib, _g(g), g.device
+        dpre = torch.empty_like(yd)
+        sums = torch.empty(1, Cc, 2, dtype=torch.float64, device=dev)
+        _lib.check(lib.w2s_gen_affine_act_bwd(yd.data_ptr(), scale.data_ptr(), shift.data_ptr(), None, g.data_ptr(), None,
+                                              dpre.data_ptr(), sums.data_ptr(), None, 1, rows, Cc, ACT[ctx.act], 1, _stream()))
+        coef = torch.empty(1, Cc, 3, dtype=torch.float32, device=dev)
+        dy = torch.empty_like(yd)
+        dw = torch.empty(Cc, dtype=torch.float32, device=dev) if ctx.needs_input_grad[1] else None
+        db = torch.empty(Cc, dtype=torch.float32, device=dev) if ctx.needs_input_grad[2] else None
+        _lib.check(lib.w2s_gen_norm_bwd(yd.data_ptr(), dpre.data_ptr(), stats.data_ptr(), sums.data_ptr(), _p(w),
+                                        coef.data_ptr(), dy.data_ptr(), _p(dw), _p(db), None, 1, rows, Cc, Cc, ctx.eps,
+                                        _stream()))
+        return dy, dw, db, None, None, None
 
 
 class _NormAct(torch.autograd.Function):
@@ -339,7 +399,12 @@ class GeneralEngine:
             w = norm.weight.reshape(-1)
             b = norm.bias.reshape(-1) if kind == "layer" else None
             return self.rownorm(y, w, b, norm.eps, act, rms=int(kind == "rms"))
-        if kind == "batch":  # eval mode: running statistics (train-mode BatchNorm is not built, see model.py)
+        if kind == "batch":
+            if self._seed is not None:  # a training forward: batch statistics, running-statistics update
+                if mask is not None:
+                    raise NotImplementedError("train-mode BatchNorm of masked samples is not built")
+                return _BatchNormTrainAct.apply(y, norm.weight, norm.bias, self, norm, act)
+            # eval mode: running statistics
             scale, shift = _BatchNormConsts.apply(norm.weight, norm.bias, self, norm.running_mean, norm.running_var, norm.eps)
             return self.affine_act(y, act, scale, shift, mask=mask, per_channel=1)
         if kind == "instance":
@@ -468,18 +533,25 @@ class GeneralEngine:
         self._seed = None
         return self._forward(x)
 
-    def forward_train(self, x: dict[str, Tensor]) -> Tensor:
-        """Training forward: builds the autograd graph whose backward runs the kernels of csrc/general_bwd.cuh, with
-        dropout at every site the reference applies it in training (masks drawn from ``dropout_seed``)."""
+    @contextlib.contextmanager
+    def training_forward(self):
+        """The scope of one training forward: dropout at every site the reference applies it in training, with masks
+        from ``dropout_seed`` (None: a seed drawn from torch's CPU generator, distinct per rank), and train-mode
+        BatchNorm (batch statistics, running-statistics update)."""
         if self.dropout_seed is not None:
             seed = int(self.dropout_seed)
         else:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item()) ^ (0x5851F42D4C957F2D * (1 + _rank()) & (2 ** 62 - 1))
         self.last_dropout_seed = self._seed = seed
         try:
-            return self._forward(x)
+            yield
         finally:
             self._seed = None
+
+    def forward_train(self, x: dict[str, Tensor]) -> Tensor:
+        """Training forward: builds the autograd graph whose backward runs the kernels of csrc/general_bwd.cuh."""
+        with self.training_forward():
+            return self._forward(x)
 
     def _forward(self, x: dict[str, Tensor]) -> Tensor:
         m = self.model

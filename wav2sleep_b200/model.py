@@ -19,9 +19,10 @@ activations relu / leaky / silu / linear, ``embed_signals``, ``register_tokens >
 ``use_residual=False``, other widths and feature dims) runs on the dimension-generic fp32 kernels of csrc/general.cuh
 (general.py): inference and training (an autograd graph over fp32 forward / backward kernels, dropout included), same
 results as the reference to fp32 accuracy, not tuned.  ``norm='weight'`` (a parametrisation with different state_dict
-keys) is the one option that raises ``NotImplementedError``; a model with BatchNorm layers (norm='batch', SleepPPGNet)
-runs inference but raises ``NotImplementedError`` under ``train()`` with grad (train-mode batch statistics are not
-built); in ``eval()`` it is differentiable, in its inputs and its parameters.
+keys) is the one option that raises ``NotImplementedError``; a Wav2Sleep model with BatchNorm layers (norm='batch')
+runs inference but raises ``NotImplementedError`` under ``train()`` with grad (train-mode BatchNorm is built, see
+general.py, but the reference's batch statistics include the zero-filled rows of missing signals, which the general
+path skips); in ``eval()`` it is differentiable, in its inputs and its parameters.  SleepPPGNet (ppgnet.py) trains.
 """
 from __future__ import annotations
 

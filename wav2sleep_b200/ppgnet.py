@@ -2,7 +2,9 @@
 (/root/reference/src/wav2sleep/models/ppgnet.py:19-126) whose forward runs on the general fp32 CUDA kernels
 (csrc/general.cuh through general.py): eight ``ConvBlock1D`` (batch norm, leaky ReLU) -> time-distributed
 ``Linear(1024 -> F)`` -> two ``DilatedConvBlock`` -> classifier.  Same constructor keywords, parameter names and default
-initialisation as the reference; inference only (BatchNorm uses its running statistics), not tuned.
+initialisation as the reference, not tuned.  In ``eval()``, and in ``train()`` under ``no_grad``, BatchNorm uses its
+running statistics; under ``train()`` with grad the forward builds the general path's autograd graph with train-mode
+BatchNorm (batch statistics over B x length, running-statistics update) and dropout at ``DilatedConvBlock.dropout``.
 """
 from __future__ import annotations
 
@@ -60,14 +62,15 @@ class SleepPPGNet(nn.Module):
 
     @torch.no_grad()
     def encode(self, x_BT: Tensor) -> Tensor:
-        """[N, 1228800] -> features [N, 1200, F]   (ppgnet.py:42-59)."""
+        """[N, 1228800] -> features [N, 1200, F]   (ppgnet.py:42-59), inference kernels."""
+        return self._features(x_BT)
+
+    def _features(self, x_BT: Tensor) -> Tensor:
         if x_BT.dim() != 2 or x_BT.size(1) != self.INPUT_LENGTH:
             raise ValueError(f"Input tensor had unexpected shape: {x_BT.size()}")
         if not x_BT.is_cuda:
             raise RuntimeError("wav2sleep_b200 runs on CUDA (sm_100a) only: move inputs with .to('cuda'); "
                                "there is no CPU fallback")
-        if self.training and torch.is_grad_enabled():
-            raise NotImplementedError("wav2sleep_b200: SleepPPGNet runs the general inference kernels only")
         eng = self._engine()
         B = x_BT.size(0)
         with torch.cuda.device(x_BT.device):
@@ -79,9 +82,19 @@ class SleepPPGNet(nn.Module):
             z = eng.affine_act(eng.linear(rows, self.dense.linear).view(B, 1200, -1), self.dense.activation_name)
             return eng.dilated_blocks(z, self.dilated_convs)
 
-    def forward(self, x_BT: Tensor) -> Tensor:
-        """[N, 1228800] -> logits [N, 1200, n_classes]   (ppgnet.py:61-74)."""
-        feat = self.encode(x_BT)
+    def _logits(self, feat: Tensor) -> Tensor:
         B, S, Fd = feat.shape
         with torch.cuda.device(feat.device):
             return self._engine().linear(feat.reshape(B * S, Fd), self.classifier).view(B, S, -1)
+
+    def forward(self, x_BT: Tensor) -> Tensor:
+        """[N, 1228800] -> logits [N, 1200, n_classes]   (ppgnet.py:61-74).
+
+        Under ``train()`` with grad enabled (and a parameter that requires grad) the logits carry a grad_fn whose
+        backward runs the general path's backward kernels; BatchNorm normalises with the batch statistics and updates
+        its running statistics, and ``DilatedConvBlock.dropout`` draws its masks as ``GeneralEngine.training_forward``
+        describes.  Otherwise the inference kernels run with the running statistics and no dropout."""
+        if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+            with self._engine().training_forward():
+                return self._logits(self._features(x_BT))
+        return self._logits(self.encode(x_BT))

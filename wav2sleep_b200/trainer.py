@@ -193,6 +193,7 @@ class SleepLightningModule(nn.Module):
         self.val_dataset_map: dict[int, str] = {}
         self.test_dataset_map: dict[int, str] = {}
         self._opt = self._sched = self._reducer = None
+        self._bn_buffers, self._process_group = [], None
 
     def forward(self, x: dict[str, Tensor], y: Tensor | None = None) -> Tensor:
         if not hasattr(self.model, "signal_encoders"):  # SleepPPGNet: one tensor (reference trainer/main.py:108-114)
@@ -313,15 +314,18 @@ class SleepLightningModule(nn.Module):
         self._opt = cfg["optimizer"]
         self._sched = cfg.get("lr_scheduler", {}).get("scheduler")
         if isinstance(self._opt, FusedAdamW):
-            enc = list(self.model.signal_encoders.parameters())
-            enc_ids = {id(p) for p in enc}
-            tail = [p for p in self.model.parameters() if id(p) not in enc_ids]
-            segs = {"tail": self._opt.segment(tail)}
-            for name, e in self.model.signal_encoders.encoders.items():
-                segs["encoder:" + name] = self._opt.segment(list(e.parameters()))
-            covered = sum(b - a for a, b in segs.values())
-            if covered != self._opt.flat_grad.numel():  # e.g. a parameter outside encoders / tail: one late bucket
-                segs = {"tail": segs["tail"], "encoders": self._opt.segment(enc)}
+            if hasattr(self.model, "signal_encoders"):
+                enc = list(self.model.signal_encoders.parameters())
+                enc_ids = {id(p) for p in enc}
+                tail = [p for p in self.model.parameters() if id(p) not in enc_ids]
+                segs = {"tail": self._opt.segment(tail)}
+                for name, e in self.model.signal_encoders.encoders.items():
+                    segs["encoder:" + name] = self._opt.segment(list(e.parameters()))
+                covered = sum(b - a for a, b in segs.values())
+                if covered != self._opt.flat_grad.numel():  # e.g. a parameter outside encoders / tail: one late bucket
+                    segs = {"tail": segs["tail"], "encoders": self._opt.segment(enc)}
+            else:  # SleepPPGNet: one bucket covering every parameter
+                segs = {"all": self._opt.segment(list(self.model.parameters()))}
             self._reducer = GradReducer(self._opt.flat_grad, segs, process_group)
             self._opt.grad_scale = 1.0 / self._reducer.world_size
             if self._reducer.world_size > 1:
@@ -332,12 +336,40 @@ class SleepLightningModule(nn.Module):
                 self._opt._bump()
             if getattr(self.model, "fast_path", False):
                 self.model._get_train_engine().bucket_hooks = [self._reducer]
+        # BatchNorm buffers (running mean / var, num_batches_tracked) for the rank-0 broadcast of fit_step
+        self._bn_buffers = [b for m in self.model.modules() if isinstance(m, nn.modules.batchnorm._BatchNorm)
+                            for b in (m.running_mean, m.running_var, m.num_batches_tracked) if b is not None]
+        self._process_group = process_group
+
+    def _broadcast_buffers(self) -> None:
+        """What DDP does with broadcast_buffers=True (Lightning's default) before each forward: every rank starts the step
+        from rank 0's BatchNorm running statistics and counters, in one flat collective.  Each rank still normalises
+        with its own batch statistics.  A model without BatchNorm buffers (or one process) issues nothing."""
+        if not self._bn_buffers or not (dist.is_available() and dist.is_initialized()):
+            return
+        if dist.get_world_size(self._process_group) == 1:
+            return
+        bufs = self._bn_buffers
+        f32 = [b for b in bufs if b.dtype == torch.float32]
+        i64 = [b for b in bufs if b.dtype == torch.int64]
+        # the int64 counters travel bit-exactly as pairs of fp32 words, so one fp32 buffer carries everything
+        flat = torch.cat([b.reshape(-1) for b in f32] + [b.reshape(-1).view(torch.float32) for b in i64])
+        dist.broadcast(flat, src=dist.get_global_rank(self._process_group, 0) if self._process_group is not None else 0,
+                       group=self._process_group)
+        off = 0
+        for b in f32:
+            b.copy_(flat[off:off + b.numel()].view_as(b))
+            off += b.numel()
+        for b in i64:
+            b.copy_(flat[off:off + 2 * b.numel()].view(torch.int64).view_as(b))
+            off += 2 * b.numel()
 
     def fit_step(self, batch) -> Tensor:
         """One optimisation step: transforms -> forward -> loss -> backward (+ overlapped all-reduce) -> clip + AdamW."""
         if self._opt is None:
             self.setup_training()
         self.model.train()
+        self._broadcast_buffers()
         batch = self.on_after_batch_transfer(batch, training=True)
         self._opt.zero_grad()
         loss = self.training_step(batch)
