@@ -346,27 +346,13 @@ int w2s_adamw_step(float* p, const float* g, float* m, float* v, long long n, co
                    float ema_decay, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------
- * fp32 check mode: straightforward fp32 CUDA-core restatement of every op (fp32 channels-last tensors, PyTorch weight
- * layouts, exact erf GELU, fp64 statistics).  wav2sleep_b200/check.py strings these into a forward whose logits agree
- * with the reference to <= 1e-4 (north-star fp32 gate).  A second GPU implementation for validation, never a fallback.
- * ------------------------------------------------------------------------------------------------------- */
-/* generic conv / linear: mode 0 input as is, 1 GELU(InstanceNorm(in)), 2 GELU(GELU(InstanceNorm(in)) + in_res), 3 raw
- * signal (inf -> 0); w [cout, cin, taps] (taps_major: [cout, taps*cin]); optional bias, residual `add`, output GELU. */
-int w2s_chk_conv(const float* in, const float* in_res, const double* in_stats, const float* w, const float* bias,
-                 const float* add, float* out, const uint8_t* row_mask, int B, int L_in, int L_out, int cin, int cout, int taps,
-                 int stride, int dil, int pad, int mode, int taps_major, int gelu_out, float eps, void* stream);
-int w2s_chk_stats(const float* x, double* stats, const uint8_t* row_mask, int B, int L, int C, void* stream);
-int w2s_chk_rowln(const float* x, const float* res, const float* g, const float* b, float* out, long long rows, int gelu,
-                  float eps, void* stream);
-int w2s_chk_attn(const float* q, const float* k, const float* v, float* o, const uint8_t* key_mask, int N, int D, void* stream);
-
-/* ---------------------------------------------------------------------------------------------------------
  * General fp32 path: the NON-DEFAULT model options of the reference (SURVEY 8f N3) - causal / chunk-causal encoders
  * (models/wav2sleep.py:248-255, models/blocks.py:150-152,178-182), norms batch / layer / rms / group / auto
  * (models/utils.py:77-96), activations relu / leaky / silu / linear (utils.py:61-74), any feature_dim / nhead / dim_ff,
  * register tokens, signal embeddings, output norm, causal sequence mixer.  Dimension-generic fp32 CUDA-core kernels on
  * channels-last fp32 tensors with PyTorch weight layouts; wav2sleep_b200/general.py strings them together.  The default
- * configuration never takes this path (it runs on the tcgen05 kernels above).
+ * configuration's inference and training run on the tcgen05 kernels above; its fp32 check mode
+ * (Wav2Sleep.forward_fp32_check, logits within 1e-4 of the reference) runs on these kernels.
  * ------------------------------------------------------------------------------------------------------- */
 enum { W2S_ACT_LINEAR = 0, W2S_ACT_RELU = 1, W2S_ACT_LEAKY = 2, W2S_ACT_GELU = 3, W2S_ACT_SILU = 4 };
 enum { W2S_NORM_INSTANCE = 0, W2S_NORM_GROUP = 1, W2S_NORM_BATCH_EVAL = 2 };

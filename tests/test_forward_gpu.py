@@ -202,15 +202,14 @@ def test_paired_encoder_launches_equal_single_launches(cuda_device, smap, ncls, 
 
 
 @pytest.mark.parametrize("smap,ncls,B,S,masked", [(CARDIO, 4, 2, 24, [("ABD", 0), ("ECG", 1)]), (EOG, 5, 1, 12, [])])
-def test_fp32_check_mode_within_1e4(cuda_device, smap, ncls, B, S, masked):
-    """North-star fp32 gate: the fp32 check mode (plain fp32 CUDA-core kernels, fp32 storage) reproduces the reference
-    logits to <= 1e-4 max-abs and the same argmax on every epoch."""
-    from wav2sleep_b200.check import forward_fp32
+def test_fp32_check_mode_on_general_path_within_1e4(cuda_device, smap, ncls, B, S, masked):
+    """North-star fp32 gate: the fp32 check mode (the general path's plain fp32 CUDA-core kernels, fp32 storage)
+    reproduces the reference logits to <= 1e-4 max-abs and the same argmax on every epoch."""
     model = build_default(smap, ncls, seed=0)
     x = make_inputs(smap, B, S, masked=masked, seed=21)
     ref = oracle.forward(x, model.state_dict(), oracle.OracleConfig(signal_map=smap, num_classes=ncls))
     model = model.to(cuda_device).eval()
-    out = forward_fp32(model, {k: v.to(cuda_device) for k, v in x.items()}).float().cpu()
+    out = model.forward_fp32_check({k: v.to(cuda_device) for k, v in x.items()}).float().cpu()
     err = (out - ref).abs().max().item()
     print(f"fp32 check mode max-abs {err:.3e}")
     assert out.shape == ref.shape
@@ -328,16 +327,15 @@ def test_randomised_shapes_subsets_and_masks(cuda_device):
     print(f"randomised sweep: worst max-abs {worst:.3e}")
 
 
-def test_fp32_check_mode_on_full_nights(cuda_device):
-    """The fp32 gate (1e-4) where it is hardest: whole-night InstanceNorm statistics over 1.2 M (cardio) and 6.9 M (EOG)
-    samples per channel (reference models/wav2sleep.py:256-261 non-causal path)."""
-    from wav2sleep_b200.check import forward_fp32
+def test_fp32_check_mode_on_general_path_full_nights(cuda_device):
+    """The fp32 gate (1e-4) of the general path's kernels where it is hardest: whole-night InstanceNorm statistics over
+    1.2 M (cardio) and 6.9 M (EOG) samples per channel (reference models/wav2sleep.py:256-261 non-causal path)."""
     for smap, ncls, S, cfg in ((CARDIO, 4, 1200, oracle.cardio_config()), (EOG, 5, 1680, oracle.eog_config())):
         model = build_default(smap, ncls, seed=0)
         x = make_inputs(smap, 1, S, seed=42)
         ref = oracle.forward(x, model.state_dict(), cfg)
         model = model.to(cuda_device).eval()
-        out = forward_fp32(model, {k: v.to(cuda_device) for k, v in x.items()}).float().cpu()
+        out = model.forward_fp32_check({k: v.to(cuda_device) for k, v in x.items()}).float().cpu()
         err = (out - ref).abs().max().item()
         agree = (out.argmax(-1) == ref.argmax(-1)).float().mean().item()
         print(f"fp32 check mode, full night {list(smap)}: max-abs {err:.3e} argmax agreement {agree:.5f}")

@@ -20,7 +20,6 @@
 #include "first_conv.cuh"
 #include "gemm_tn.cuh"
 #include "train_kernels.cuh"
-#include "check_fp32.cuh"
 #include "general.cuh"
 #include "general_bwd.cuh"
 #include "staging.cuh"
@@ -530,7 +529,7 @@ int check_encoder_desc(const w2s_encoder_desc* d) {
 
 extern "C" {
 
-int w2s_abi_version(void) { return 8; }
+int w2s_abi_version(void) { return 9; }
 const char* w2s_last_error(void) { return g_err.c_str(); }
 
 int w2s_conv_uses_split(int cin, int cout) { return (cin <= 16 && cout <= 16) ? 1 : 0; }
@@ -1332,44 +1331,6 @@ int w2s_adamw_step(float* p_, const float* g, float* m, float* v, long long n, c
   LaunchScope scope((cudaStream_t)stream, "adamw_step", (double)n * (ema ? 36.0 : 28.0), (double)n * 12.0);
   adamw_kernel<<<ew_grid(n), 256, 0, (cudaStream_t)stream>>>(a);
   W2S_LAUNCH_CHECK("adamw_step");
-}
-
-// ================================================================================================
-// fp32 check mode (check_fp32.cuh): kernel-level entry points, orchestrated by wav2sleep_b200/check.py
-// ================================================================================================
-int w2s_chk_conv(const float* in, const float* in_res, const double* in_stats, const float* w, const float* bias,
-                 const float* add, float* out, const uint8_t* row_mask, int B, int L_in, int L_out, int cin, int cout, int taps,
-                 int stride, int dil, int pad, int mode, int taps_major, int gelu_out, float eps, void* stream) {
-  if (!in || !w || !out || B <= 0 || L_in <= 0 || L_out <= 0 || cin < 1 || cout < 1 || cout > 256) return fail("chk_conv: bad arguments");
-  if ((mode == 1 || mode == 2) && (!in_stats || cin > 128)) return fail("chk_conv: norm prologue needs stats and cin <= 128");
-  if (mode == 2 && !in_res) return fail("chk_conv: residual input missing");
-  chk::ConvArgs a{in, in_res, in_stats, w, bias, add, out, row_mask, B, L_in, L_out, cin, cout, taps, stride, dil, pad, mode,
-                  taps_major, gelu_out, eps};
-  const int per_block = 256 / cout;
-  int gx = (L_out + per_block - 1) / per_block;
-  if (gx > 16 * sm_count()) gx = 16 * sm_count();
-  LaunchScope scope((cudaStream_t)stream, "chk_conv", 0, 2.0 * B * (double)L_out * cout * cin * taps);
-  chk::conv_kernel<<<dim3(gx < 1 ? 1 : gx, B), 256, 0, (cudaStream_t)stream>>>(a);
-  W2S_LAUNCH_CHECK("chk_conv");
-}
-int w2s_chk_stats(const float* x, double* stats, const uint8_t* row_mask, int B, int L, int Cc, void* stream) {
-  if (!x || !stats || B <= 0 || L <= 0 || Cc < 1) return fail("chk_stats: bad arguments");
-  LaunchScope scope((cudaStream_t)stream, "chk_stats", (double)B * L * Cc * 4.0, 0);
-  chk::stats_kernel<<<dim3(Cc, B), 256, 0, (cudaStream_t)stream>>>(x, stats, row_mask, L, Cc);
-  W2S_LAUNCH_CHECK("chk_stats");
-}
-int w2s_chk_rowln(const float* x, const float* res, const float* g, const float* b, float* out, long long rows, int gelu,
-                  float eps, void* stream) {
-  if (!x || !g || !b || !out || rows <= 0) return fail("chk_rowln: bad arguments");
-  LaunchScope scope((cudaStream_t)stream, "chk_rowln", (double)rows * 128 * 8.0, 0);
-  chk::rowln_kernel<<<ew_grid(rows * 32), 256, 0, (cudaStream_t)stream>>>(x, res, g, b, out, rows, gelu, eps);
-  W2S_LAUNCH_CHECK("chk_rowln");
-}
-int w2s_chk_attn(const float* q, const float* k, const float* v, float* o, const uint8_t* key_mask, int N, int D, void* stream) {
-  if (!q || !k || !v || !o || N <= 0 || D < 1 || D > 5) return fail("chk_attn: bad arguments");
-  LaunchScope scope((cudaStream_t)stream, "chk_attn", (double)N * D * 128 * 16.0, 0);
-  chk::attn_kernel<<<(N * 8 + 127) / 128, 128, 0, (cudaStream_t)stream>>>(q, k, v, o, key_mask, N, D);
-  W2S_LAUNCH_CHECK("chk_attn");
 }
 
 // ================================================================================================

@@ -431,10 +431,11 @@ class Wav2Sleep(nn.Module):
         return self._get_engine().predict_async(x, ready=ready)
 
     def forward_fp32_check(self, x: dict[str, Tensor]) -> Tensor:
-        """The same forward through the un-fused fp32 CUDA-core check kernels (check.py): slow, <= 1e-4 from the
-        reference's fp32 logits.  A validation aid, not an inference path."""
-        from .check import forward_fp32
-        return forward_fp32(self, x)
+        """The same forward through the general path's un-fused fp32 CUDA-core kernels (general.py: fp32 storage, exact
+        erf GELU, fp64 statistics), with eval semantics whatever the mode (no dropout, BatchNorm on its running
+        statistics) and under ``no_grad``: slow, <= 1e-4 from the reference's fp32 logits.  A validation aid that
+        separates the algorithm from the fast path's 16-bit storage, not an inference path."""
+        return self._get_general().forward(x)
 
 
 def build_default(signal_map: dict[str, str], num_classes: int, seed: int | None = None) -> Wav2Sleep:
