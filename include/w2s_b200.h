@@ -341,6 +341,15 @@ int w2s_sumsq(const float* g, long long n, double* out, void* stream);
 /* *out = max |g[i]| (fp32; the call zeroes *out first).  Picks the loss scale of a backward whose incoming gradient is
  * not a mean cross entropy (input attribution; ABI v7). */
 int w2s_absmax(const float* g, long long n, float* out, void* stream);
+/* Integrated gradients (ABI v10).  out [K * B, T] = the K interpolated batches out[k, b, t] = x0 + alphas[k] * (x - x0)
+ * (alphas: K device floats; x0 NULL: zero baseline).  A non-finite x[b, t] is copied unchanged onto every step, so a
+ * missing (-inf) row stays missing and w2s_gen_conv / w2s_first_conv_dgrad keep reading such samples as 0. */
+int w2s_ig_path_inputs(const float* x, const float* x0, const float* alphas, int K, int B, int T, float* out, void* stream);
+/* attr [B, T] = (first ? 0 : attr) + (x - x0) * sum_k weights[k] * grads[k, b, t] (grads [K * B, T], weights K device
+ * floats, x0 NULL: zero baseline); exactly 0 where x is non-finite.  Each step's term is added to the fp32 running sum
+ * in k order, so splitting the steps over several calls (first = 0 after the first) gives bitwise the one-call sum. */
+int w2s_ig_accumulate(const float* grads, const float* weights, int K, const float* x, const float* x0, int B, int T,
+                      float* attr, int first, void* stream);
 int w2s_adamw_step(float* p, const float* g, float* m, float* v, long long n, const double* gnorm_sq, float lr, float beta1,
                    float beta2, float eps, float weight_decay, float max_norm, float grad_scale, long long step, float* ema,
                    float ema_decay, void* stream);

@@ -27,7 +27,7 @@ STREAM_MAX_LAYERS = 32
 STREAM_MAX_DILATIONS = 16
 STREAM_MAX_KERNEL = 16
 STREAM_MAX_FEATURES = 256
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 PRO_NONE, PRO_NORM, PRO_NORM_RES, PRO_FIR, PRO_NORM_RES_X, PRO_DNORM = 0, 1, 2, 3, 4, 5
 EPI_STATS, EPI_BIAS_GELU, EPI_LN_GELU, EPI_LN_GELU_RES, EPI_PLAIN, EPI_ACT_BWD = 0, 1, 2, 3, 4, 5
@@ -190,6 +190,9 @@ SYMBOLS = {
     "w2s_head_bwd": (C.c_int, [C.c_void_p] * 6 + [C.c_longlong, C.c_int, C.c_float, C.c_void_p]),
     "w2s_sumsq": (C.c_int, [C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p]),
     "w2s_absmax": (C.c_int, [C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p]),
+    "w2s_ig_path_inputs": (C.c_int, [C.c_void_p] * 3 + [C.c_int] * 3 + [C.c_void_p, C.c_void_p]),
+    "w2s_ig_accumulate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                    C.c_int, C.c_void_p]),
     "w2s_adamw_step": (C.c_int, [C.c_void_p] * 4 + [C.c_longlong, C.c_void_p] + [C.c_float] * 7
                        + [C.c_longlong, C.c_void_p, C.c_float, C.c_void_p]),
     "w2s_gen_conv": (C.c_int, [C.c_void_p] * 5 + [C.c_int] * 11 + [C.c_void_p]),

@@ -14,6 +14,7 @@
 #include <string>
 #include <vector>
 
+#include "attribution.cuh"
 #include "conv_igemm.cuh"
 #include "conv_stream.cuh"
 #include "epoch_mixer.cuh"
@@ -529,7 +530,7 @@ int check_encoder_desc(const w2s_encoder_desc* d) {
 
 extern "C" {
 
-int w2s_abi_version(void) { return 9; }
+int w2s_abi_version(void) { return 10; }
 const char* w2s_last_error(void) { return g_err.c_str(); }
 
 int w2s_conv_uses_split(int cin, int cout) { return (cin <= 16 && cout <= 16) ? 1 : 0; }
@@ -1316,6 +1317,30 @@ int w2s_absmax(const float* g, long long n, float* out, void* stream) {
   if (gx > 2 * sm_count()) gx = 2 * sm_count();
   absmax_kernel<<<gx, 256, 0, (cudaStream_t)stream>>>(g, n, reinterpret_cast<unsigned int*>(out));
   W2S_LAUNCH_CHECK("absmax");
+}
+int w2s_ig_path_inputs(const float* x, const float* x0, const float* alphas, int K, int B, int T, float* out,
+                       void* stream) {
+  if (!x || !alphas || !out)
+    return fail("ig_path_inputs: NULL operand (x=%p alphas=%p out=%p)", (const void*)x, (const void*)alphas, (void*)out);
+  if (K < 1 || B < 1 || T < 1) return fail("ig_path_inputs: K=%d B=%d T=%d (each must be >= 1)", K, B, T);
+  const long long n = (long long)B * T;
+  LaunchScope scope((cudaStream_t)stream, "ig_path_inputs", (double)n * (x0 ? 8.0 : 4.0) + (double)n * K * 4.0, (double)n * K * 2.0);
+  ig::path_inputs_kernel<<<ew_grid(n, ig::kThreads), ig::kThreads, 0, (cudaStream_t)stream>>>(x, x0, alphas, K, n, out);
+  W2S_LAUNCH_CHECK("ig_path_inputs");
+}
+int w2s_ig_accumulate(const float* grads, const float* weights, int K, const float* x, const float* x0, int B, int T,
+                      float* attr, int first, void* stream) {
+  if (!grads || !weights || !x || !attr)
+    return fail("ig_accumulate: NULL operand (grads=%p weights=%p x=%p attr=%p)", (const void*)grads, (const void*)weights,
+                (const void*)x, (void*)attr);
+  if (K < 1 || B < 1 || T < 1 || (first != 0 && first != 1))
+    return fail("ig_accumulate: K=%d B=%d T=%d first=%d (K, B, T >= 1, first 0 or 1)", K, B, T, first);
+  const long long n = (long long)B * T;
+  LaunchScope scope((cudaStream_t)stream, "ig_accumulate", (double)n * (4.0 * K + (x0 ? 8.0 : 4.0) + (first ? 4.0 : 8.0)),
+                    (double)n * (2.0 * K + 1.0));
+  ig::accumulate_kernel<<<ew_grid(n, ig::kThreads), ig::kThreads, 0, (cudaStream_t)stream>>>(grads, weights, K, x, x0, n, attr,
+                                                                                           first);
+  W2S_LAUNCH_CHECK("ig_accumulate");
 }
 int w2s_adamw_step(float* p_, const float* g, float* m, float* v, long long n, const double* gnorm_sq, float lr, float beta1,
                    float beta2, float eps, float weight_decay, float max_norm, float grad_scale, long long step, float* ema,

@@ -5,6 +5,7 @@
 initialisation as the reference, not tuned.  In ``eval()``, and in ``train()`` under ``no_grad``, BatchNorm uses its
 running statistics; under ``train()`` with grad the forward builds the general path's autograd graph with train-mode
 BatchNorm (batch statistics over B x length, running-statistics update) and dropout at ``DilatedConvBlock.dropout``.
+In ``eval()`` an input that requires grad gets an eval-semantics graph (input gradients, attribution.py).
 """
 from __future__ import annotations
 
@@ -74,7 +75,9 @@ class SleepPPGNet(nn.Module):
         eng = self._engine()
         B = x_BT.size(0)
         with torch.cuda.device(x_BT.device):
-            a = x_BT.detach().to(torch.float32).contiguous().view(B, self.INPUT_LENGTH, 1)
+            # stays on the autograd graph when the input requires grad; block 0 reads the signal as it is (no
+            # missing-sample rule, as in the reference), so its convs run with raw = 0 in every mode
+            a = x_BT.to(torch.float32).contiguous().view(B, self.INPUT_LENGTH, 1)
             for blk in self.conv_block.model:
                 a = eng.conv_block(a, blk)
             # [B, 4800, 256] channels-last == transpose(-1, -2) of the reference tensor; reshape(-1, 1200, 1024)
@@ -90,11 +93,18 @@ class SleepPPGNet(nn.Module):
     def forward(self, x_BT: Tensor) -> Tensor:
         """[N, 1228800] -> logits [N, 1200, n_classes]   (ppgnet.py:61-74).
 
-        Under ``train()`` with grad enabled (and a parameter that requires grad) the logits carry a grad_fn whose
-        backward runs the general path's backward kernels; BatchNorm normalises with the batch statistics and updates
-        its running statistics, and ``DilatedConvBlock.dropout`` draws its masks as ``GeneralEngine.training_forward``
-        describes.  Otherwise the inference kernels run with the running statistics and no dropout."""
-        if self.training and torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+        Under ``train()`` with grad enabled (and a parameter or the input that requires grad) the logits carry a grad_fn
+        whose backward runs the general path's backward kernels; BatchNorm normalises with the batch statistics and
+        updates its running statistics, and ``DilatedConvBlock.dropout`` draws its masks as
+        ``GeneralEngine.training_forward`` describes.  In ``eval()``, an input that requires grad gets an eval-semantics
+        graph (BatchNorm on its running statistics, no dropout) whose logits are bitwise those of inference, and
+        ``x_BT.grad`` receives d(objective)/dx.  Otherwise the inference kernels run with the running statistics and no
+        dropout."""
+        grad_on = torch.is_grad_enabled()
+        input_grad = grad_on and isinstance(x_BT, Tensor) and x_BT.requires_grad
+        if self.training and grad_on and (input_grad or any(p.requires_grad for p in self.parameters())):
             with self._engine().training_forward():
                 return self._logits(self._features(x_BT))
+        if input_grad:
+            return self._logits(self._features(x_BT))
         return self._logits(self.encode(x_BT))
