@@ -762,28 +762,16 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
       const float v = xraw[j - xs0];
       return isinf(v) ? 0.0f : v;
     };
-    // 8 channels of input row u = id / CH (y [, y2]: stored conv output, r [, r2]: residual branch) -> activated fp16
-    // operand chunk(s) in the A stage
-    auto core = [&](int id, bool valid, const uint4& y, const uint4& y2, const uint4& r, const uint4& r2) {
-      const int u = id / CH;
+    auto fin = [](float v) { return isinf(v) ? 0.0f : v; };  // the reference's -inf -> 0 rule, element-wise
+    // Offset (bytes) of input row u in a chunk column of the A stage.  The row index of a thread's k-th chunk of a
+    // tile is tt / CH + k * NTT / CH, so on interior tiles every offset is a per-thread constant plus a compile-time one.
+    auto soff_of = [](int u) { return (uint32_t)((u & (STRIDE - 1)) * CH * RP + u / STRIDE) * 16; };
+    // 8 channels of one input row (y [, y2]: stored conv output, r [, r2]: residual branch; xm / x0 / xp: raw-signal
+    // samples of the block-0 fusion modes, -inf already replaced) -> activated fp16 operand chunk(s) at dst in the A stage
+    auto act = [&](bool valid, float xm, float x0, float xp, const uint4& y, const uint4& y2, const uint4& r,
+                   const uint4& r2, uint32_t dst) {
       uint4 o = make_uint4(0u, 0u, 0u, 0u), olo = make_uint4(0u, 0u, 0u, 0u);
       if (valid) {
-        float xm = 0.0f, x0 = 0.0f, xp = 0.0f;
-        auto fin = [](float v) { return isinf(v) ? 0.0f : v; };  // the reference's -inf -> 0 rule, element-wise
-        if (PRO == PRO_FIR) {
-          if (x_interior) {  // whole window staged: no per-element bounds checks
-            const float* xp3 = xraw + (i0 + u - 1 - xs0);
-            xm = fin(xp3[0]);
-            x0 = fin(xp3[1]);
-            xp = fin(xp3[2]);
-          } else {
-            xm = xat(i0 + u - 1);
-            x0 = xat(i0 + u);
-            xp = xat(i0 + u + 1);
-          }
-        } else if (PRO == PRO_NORM_RES_X) {
-          x0 = x_interior ? fin(xraw[2 * (i0 + u) - xs0]) : xat(2 * (i0 + u));
-        }
         const uint32_t yy[8] = {y.x, y.y, y.z, y.w, y2.x, y2.y, y2.z, y2.w};
         const uint32_t rr[8] = {r.x, r.y, r.z, r.w, r2.x, r2.y, r2.z, r2.w};
         auto pair = [&](const uint32_t (&w)[8], int q) -> float2 {  // channels 2q, 2q+1 of the 8 as fp32
@@ -814,9 +802,30 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
           }
         }
       }
-      const uint32_t soff = (uint32_t)((u & (STRIDE - 1)) * CH * RP + u / STRIDE) * 16;
-      sts128(adst + soff, o);
-      if (SPLIT) sts128(adst + Cfg::A_ONE + soff, olo);
+      sts128(dst, o);
+      if (SPLIT) sts128(dst + Cfg::A_ONE, olo);
+    };
+    // chunk id (input row u = id / CH) of a tile with any bounds: x samples through xat unless the window is interior
+    auto core = [&](int id, bool valid, const uint4& y, const uint4& y2, const uint4& r, const uint4& r2) {
+      const int u = id / CH;
+      float xm = 0.0f, x0 = 0.0f, xp = 0.0f;
+      if (valid) {
+        if (PRO == PRO_FIR) {
+          if (x_interior) {  // whole window staged: no per-element bounds checks
+            const float* xp3 = xraw + (i0 + u - 1 - xs0);
+            xm = fin(xp3[0]);
+            x0 = fin(xp3[1]);
+            xp = fin(xp3[2]);
+          } else {
+            xm = xat(i0 + u - 1);
+            x0 = xat(i0 + u);
+            xp = xat(i0 + u + 1);
+          }
+        } else if (PRO == PRO_NORM_RES_X) {
+          x0 = x_interior ? fin(xraw[2 * (i0 + u) - xs0]) : xat(2 * (i0 + u));
+        }
+      }
+      act(valid, xm, x0, xp, y, y2, r, r2, adst + soff_of(u));
     };
     // Hand-over: every transform thread publishes its shared-memory writes to the async proxy, then arrives
     auto hand_over = [&]() {
@@ -921,6 +930,18 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
         cur = nxt;
       }
     } else {
+    // Interior tiles: chunk k of this thread is chunk tt + k * NTT of the tile, input row u0 + k * UK.  Its raw-stage,
+    // x-window and A-stage offsets are the stage base + a per-thread constant (computed once here) + a compile-time
+    // constant, the loop over k is fully unrolled and only the last chunk is conditional (on the thread, not the tile).
+    constexpr int NK = (R * CH + NTT - 1) / NTT;  // chunks per thread and tile (the last one for some threads only)
+    constexpr int UK = NTT / CH;
+    static_assert(NTT % CH == 0 && UK % STRIDE == 0, "fixed row stride phase of a thread's chunks");
+    const int u0 = tt / CH;
+    const bool last_chunk = tt + (NK - 1) * NTT < R * CH;
+    const uint32_t raw_t = (uint32_t)tt * (8 * ESZ);
+    const uint32_t a_t = soff_of(u0);
+    constexpr int XK = (PRO == PRO_NORM_RES_X ? 2 : 1) * UK;  // x-window step between a thread's chunks
+    const int x_t = (PRO == PRO_NORM_RES_X ? 2 : 1) * u0;
     TilePos tp = pos0;
     for (int tile = tile_begin; tile < tile_end; ++tile, advance(tp)) {
       int b;
@@ -956,10 +977,36 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
         }
         core(id, valid, y, y2, r, r2);
       };
+      // chunk k of an interior tile; xq: this thread's first row in the x window (block-0 fusion modes)
+      const uint32_t raw_q = raw + raw_t, a_q = adst + a_t;
+      const float* xq = xraw + ((PRO == PRO_FIR ? i0 - 1 : 2 * i0) - xs0 + x_t);
+      auto interior_chunk = [&](int k) {
+        const uint32_t src = raw_q + (uint32_t)(k * NTT * 8 * ESZ);
+        uint4 y = make_uint4(0u, 0u, 0u, 0u), y2 = y, r = y, r2 = y;
+        if (PRO != PRO_FIR) {
+          y = lds128(src);
+          if (WIN) y2 = lds128(src + 16);
+        }
+        if (PRO == PRO_NORM_RES) {
+          r = lds128(src + Cfg::RAW_ONE);
+          if (WIN) r2 = lds128(src + Cfg::RAW_ONE + 16);
+        }
+        float xm = 0.0f, x0 = 0.0f, xp = 0.0f;
+        if (PRO == PRO_FIR) {
+          xm = fin(xq[k * XK]);
+          x0 = fin(xq[k * XK + 1]);
+          xp = fin(xq[k * XK + 2]);
+        } else if (PRO == PRO_NORM_RES_X) {
+          x0 = fin(xq[k * XK]);
+        }
+        act(true, xm, x0, xp, y, y2, r, r2, a_q + (uint32_t)(k * (UK / STRIDE) * 16));
+      };
       if (W2S_DBG(p, 32)) {
-      } else if (interior) {
-#pragma unroll 2
-        for (int id = tt; id < R * CH; id += NTT) chunk(id, true);
+      } else if (interior && (Cfg::XN == 0 || x_interior)) {
+#pragma unroll
+        for (int k = 0; k < NK; ++k) {
+          if (k < NK - 1 || last_chunk) interior_chunk(k);
+        }
       } else {
         for (int id = tt; id < R * CH; id += NTT) {
           const int i = i0 + id / CH;
