@@ -20,6 +20,7 @@ import torch
 from torch import Tensor
 
 from . import _lib
+from .engine import _f32, _stream, check_inputs
 
 __all__ = ("integrated_gradients", "gauss_legendre")
 
@@ -44,49 +45,25 @@ def _model_kind(model) -> str:
     raise TypeError(f"integrated_gradients takes a Wav2Sleep or a SleepPPGNet, got {type(model).__name__}")
 
 
-def _signals(model, kind: str, x, what: str) -> dict[str, Tensor]:
-    """The input (or baseline) as {name: [B, T]}; SleepPPGNet's single tensor is named "x"."""
+def _signals(model, kind: str, x, what: str) -> tuple[dict[str, Tensor], int, int, torch.device]:
+    """The input (or baseline) as {name: [B, T]}, with its B, S and device; SleepPPGNet's single tensor is named "x"."""
     if kind == "ppgnet":
         if not isinstance(x, Tensor):
             raise TypeError(f"{what}: SleepPPGNet takes a [B, {model.INPUT_LENGTH}] tensor, got {type(x).__name__}")
         if x.dim() != 2 or x.size(1) != model.INPUT_LENGTH:
             raise ValueError(f"{what}: expected [B, {model.INPUT_LENGTH}], got {tuple(x.shape)}")
-        xs = {"x": x}
-    else:
-        if not isinstance(x, dict) or not x:
-            raise TypeError(f"{what}: Wav2Sleep takes a non-empty {{signal: [B, T]}} dict")
-        xs = dict(x)
-        for n, t in xs.items():
-            if n not in model.signal_encoders.signal_map:
-                raise KeyError(f"{what}: signal {n!r} has no encoder (valid: {list(model.signal_encoders.signal_map)})")
-            if not isinstance(t, Tensor) or t.dim() != 2:
-                raise ValueError(f"{what}[{n!r}]: expected a [B, T] tensor")
-    for n, t in xs.items():
-        if not t.is_cuda:
+        if not x.is_cuda:
             raise RuntimeError(f"{what}: wav2sleep_b200 runs on CUDA (sm_100a) only; there is no CPU fallback")
+        if x.size(0) == 0:
+            raise ValueError(f"{what}: empty batch")
+        xs, B, S, dev = {"x": x}, x.size(0), 1200, x.device
+    else:
+        _, B, S, dev = check_inputs(model.signal_encoders, x, what)
+        xs = dict(x)
+    for n, t in xs.items():
         if not t.is_floating_point():
             raise TypeError(f"{what}[{n!r}]: expected a floating-point tensor, got {t.dtype}")
-    return xs
-
-
-def _epochs(model, kind: str, xs: dict[str, Tensor]) -> tuple[int, int]:
-    """(B, S) of the input, checked across signals."""
-    B = S = None
-    for n, t in xs.items():
-        if kind == "ppgnet":
-            s = 1200
-        else:
-            spe = model.signal_encoders.get_encoder(n).samples_per_epoch
-            if t.size(1) % spe:
-                raise ValueError(f"{n}: input length {t.size(1)} is not a multiple of {spe} samples per epoch")
-            s = t.size(1) // spe
-        if B is None:
-            B, S = t.size(0), s
-        elif (t.size(0), s) != (B, S):
-            raise ValueError(f"{n}: batch/epoch count {(t.size(0), s)} differs from {(B, S)}")
-    if B < 1 or S < 1:
-        raise ValueError(f"empty input: B={B}, S={S}")
-    return B, S
+    return xs, B, S, dev
 
 
 def parse_target(target, B: int, S: int, n_classes: int) -> Tensor:
@@ -143,23 +120,21 @@ def integrated_gradients(model, x, target, baseline=None, steps: int = 32, inter
     kind = _model_kind(model)
     steps_nodes, steps_weights = gauss_legendre(steps)
     ibs = _internal_batch(internal_batch_size)
-    xs = _signals(model, kind, x, "x")
-    B, S = _epochs(model, kind, xs)
+    xs, B, S, dev = _signals(model, kind, x, "x")
     x0s = None
     if baseline is not None:
-        x0s = _signals(model, kind, baseline, "baseline")
+        x0s, _, _, dev0 = _signals(model, kind, baseline, "baseline")
         if set(x0s) != set(xs):
             raise ValueError(f"baseline signals {sorted(x0s)} differ from the input's {sorted(xs)}")
         for n in xs:
             if x0s[n].shape != xs[n].shape:
                 raise ValueError(f"baseline[{n!r}] has shape {tuple(x0s[n].shape)}, the input {tuple(xs[n].shape)}")
+        if dev0 != dev:
+            raise ValueError("every input and baseline tensor must be on one device")
     n_classes = model.classifier.out_features
     tgt = parse_target(target, B, S, n_classes)
     if torch.is_inference_mode_enabled():
         raise RuntimeError("integrated_gradients needs autograd: call it outside torch.inference_mode()")
-    dev = next(iter(xs.values())).device
-    if any(t.device != dev for t in list(xs.values()) + list((x0s or {}).values())):
-        raise ValueError("every input and baseline tensor must be on one device")
     if B > 65535:
         raise ValueError(f"B = {B} nights: at most 65535 per call")
 
@@ -187,10 +162,8 @@ def integrated_gradients(model, x, target, baseline=None, steps: int = 32, inter
 
 
 def _run(lib, model, kind, names, xs, x0s, tgt, nodes, weights, ibs, B, S, n_classes, dev):
-    from .engine import _stream
-    f32 = lambda t: t.detach().to(torch.float32).contiguous()
-    xs = {n: f32(xs[n]) for n in names}
-    x0s = None if x0s is None else {n: f32(x0s[n]) for n in names}
+    xs = {n: _f32(xs[n]) for n in names}
+    x0s = None if x0s is None else {n: _f32(x0s[n]) for n in names}
     alphas = torch.tensor(nodes, dtype=torch.float32).to(dev)
     wts = torch.tensor(weights, dtype=torch.float32).to(dev)
     ends = torch.tensor([0.0, 1.0], dtype=torch.float32).to(dev)

@@ -14,8 +14,13 @@ from . import _lib
 from ._lib import EncoderDesc, MixerDesc, SeqDesc
 
 
-def _ptr(t: Tensor | None) -> int | None:
+def _p(t: Tensor | None) -> int | None:
     return None if t is None else t.data_ptr()
+
+
+def _f32(t: Tensor | None) -> Tensor | None:
+    """A tensor as the kernels read it: detached, fp32, contiguous (no copy when it already is)."""
+    return None if t is None else t.detach().to(torch.float32).contiguous()
 
 
 def _stream() -> int:
@@ -24,6 +29,71 @@ def _stream() -> int:
         return torch._C._cuda_getCurrentRawStream(torch._C._cuda_getDevice())
     except AttributeError:  # older / newer torch without the private accessors
         return torch.cuda.current_stream().cuda_stream
+
+
+def _argmax(lib, logits: Tensor) -> Tensor:
+    """Most likely class of every epoch of logits [B, S, C] -> int64 [B, S] (first maximum wins), on the current
+    stream of the logits' device."""
+    B, S, Cn = logits.shape
+    out = torch.empty(B, S, dtype=torch.int64, device=logits.device)
+    with torch.cuda.device(logits.device):
+        _lib.check(lib.w2s_argmax(logits.data_ptr(), B * S, Cn, out.data_ptr(), _stream()))
+    return out
+
+
+def _rank() -> int:
+    import torch.distributed as dist
+    return dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
+
+
+def _dropout_seed(fixed: int | None) -> int:
+    """The dropout seed of one training forward: ``fixed``, or (None) one drawn from torch's CPU generator and made
+    distinct per data-parallel rank."""
+    if fixed is not None:
+        return int(fixed)
+    return int(torch.randint(0, 2 ** 62, (1,)).item()) ^ (0x5851F42D4C957F2D * (1 + _rank()) & (2 ** 62 - 1))
+
+
+class UnknownSignal(KeyError, ValueError):
+    """A signal the model has no encoder for (a KeyError like a dict lookup, and a ValueError like any bad input)."""
+
+
+class NotASignalDict(ValueError, TypeError):
+    """An input that is not a non-empty ``{signal: [B, T]}`` dict."""
+
+
+def check_inputs(encoders, x, what: str = "", joint: bool = True):
+    """The host-side check of a ``Wav2Sleep`` input ``{signal: [B, T]}`` against ``encoders`` (the model's
+    ``SignalEncoders``), before any launch and without a device synchronisation -> (sorted names, B, S, device).
+    ``what`` prefixes the messages.  ``joint=False`` checks every signal on its own, for callers that encode each one
+    separately: an empty dict passes, and B, S and the device may differ between signals (those of the last one are
+    returned)."""
+    p = f"{what}: " if what else ""
+    if not isinstance(x, dict) or (joint and not x):
+        raise NotASignalDict(f"{p}No signals provided to MultiModalAttentionEmbedder: expected a non-empty "
+                             "{signal: [B, T]} dict")  # wav2sleep.py:312-313
+    smap = encoders.signal_map
+    B = S = device = None
+    for name, t in x.items():
+        if name not in smap:
+            raise UnknownSignal(f"{p}Signal {name!r} has no encoder (valid: {list(smap)})")
+        if not isinstance(t, Tensor) or t.dim() != 2:
+            raise ValueError(f"{p}{name}: expected a [B, T] tensor")
+        if not t.is_cuda:
+            raise RuntimeError(f"{p}wav2sleep_b200 runs on CUDA (sm_100a) only: move inputs with .to('cuda'); there is "
+                               "no CPU fallback")
+        spe = encoders.get_encoder(name).samples_per_epoch
+        if t.size(1) % spe:
+            raise ValueError(f"{p}{name}: Input length {t.size(1)} must be divisible by self.samples_per_epoch={spe}.")
+        b, s = t.size(0), t.size(1) // spe
+        if b == 0 or s == 0:
+            raise ValueError(f"{p}{name}: empty batch (B={b}, S={s})")
+        if joint and device is not None and t.device != device:
+            raise ValueError(f"{p}{name}: on {t.device}, other signals on {device}")
+        if joint and B is not None and (b, s) != (B, S):
+            raise ValueError(f"{p}{name}: batch/epoch count {(b, s)} differs from {(B, S)}")
+        B, S, device = b, s, t.device
+    return sorted(x), B, S, device
 
 
 class PackPlan:
@@ -283,31 +353,6 @@ class ForwardEngine:
         return buf
 
     # ------------------------------------------------------------------ forward
-    def _check_inputs(self, x):
-        if not isinstance(x, dict) or len(x) == 0:
-            raise ValueError("No signals provided to MultiModalAttentionEmbedder.")  # wav2sleep.py:312-313
-        smap = self.model.signal_encoders.signal_map
-        B = S = device = None
-        for name, t in x.items():
-            if name not in smap:
-                raise KeyError(f"Signal {name!r} has no encoder (valid: {list(smap)})")
-            if not isinstance(t, Tensor) or t.dim() != 2:
-                raise ValueError(f"{name}: expected a [B, T] tensor")
-            if not t.is_cuda:
-                raise RuntimeError("wav2sleep_b200 runs on CUDA (sm_100a) only: move inputs with .to('cuda'); "
-                                   "there is no CPU fallback")
-            spe = self.model.signal_encoders.get_encoder(name).samples_per_epoch
-            if t.size(-1) % spe:
-                raise ValueError(f"Input length {t.size(-1)} must be divisible by self.samples_per_epoch={spe}.")
-            b, s = t.size(0), t.size(-1) // spe
-            if B is None:
-                B, S, device = b, s, t.device
-            elif (b, s) != (B, S) or t.device != device:
-                raise ValueError(f"{name}: batch/epoch count {(b, s)} differs from {(B, S)}")
-        if B == 0 or S == 0:
-            raise ValueError("empty batch")
-        return B, S, device
-
     def _seq_head(self, buf, B: int, S: int, logits: Tensor, stream: "torch.cuda.Stream") -> None:
         """Sequence mixer + classifier on `stream`."""
         ws = buf["seq_ws"]
@@ -415,13 +460,10 @@ class ForwardEngine:
             logits = torch.empty(B, S, self.model.num_classes, dtype=torch.float32, device=buf["mix"].device)
             zs = (C.c_void_p * len(names))(*[buf["z"][n].data_ptr() for n in names])
             ms = (C.c_void_p * len(names))(*[buf["mask"][n].data_ptr() for n in names])
-            ts = tail.cuda_stream
-            _lib.check(lib.w2s_epoch_mixer_fwd(C.byref(self.mixer_desc), zs, ms, len(names), B, S, buf["mix"].data_ptr(), ts))
+            _lib.check(lib.w2s_epoch_mixer_fwd(C.byref(self.mixer_desc), zs, ms, len(names), B, S, buf["mix"].data_ptr(),
+                                               tail.cuda_stream))
             self._seq_head(buf, B, S, logits, tail)
-            out = logits
-            if argmax:
-                out = torch.empty(B, S, dtype=torch.int64, device=logits.device)
-                _lib.check(lib.w2s_argmax(logits.data_ptr(), B * S, self.model.num_classes, out.data_ptr(), ts))
+            out = _argmax(lib, logits) if argmax else logits  # on the tail stream: it is the current one here
             done = torch.cuda.Event()
             done.record(tail)
         buf["tail_done"] = done
@@ -431,15 +473,11 @@ class ForwardEngine:
     def forward_async(self, x: dict[str, Tensor], argmax: bool = False, ready=None) -> Pending:
         """Enqueue a forward on the engine's own streams and return at once; ``.wait()`` on the result orders the current
         stream after it.  Inputs must stay untouched until then."""
-        B, S, device = self._check_inputs(x)
+        names, B, S, device = check_inputs(self.model.signal_encoders, x)
         with torch.cuda.device(device):
             self._ensure_packed(device)
-            names = sorted(x.keys())
             buf = self._buffers(device, names, B, S, detached=True)
-            xs = {}
-            for n in names:
-                t = x[n].detach()
-                xs[n] = t if (t.dtype == torch.float32 and t.is_contiguous()) else t.to(torch.float32).contiguous()
+            xs = {n: _f32(x[n]) for n in names}
             return self._launch_async(buf, xs, names, B, S, argmax, ready)
 
     def predict_async(self, x: dict[str, Tensor], ready=None) -> Pending:
@@ -451,15 +489,11 @@ class ForwardEngine:
 
     @torch.no_grad()
     def forward(self, x: dict[str, Tensor]) -> Tensor:
-        B, S, device = self._check_inputs(x)
+        names, B, S, device = check_inputs(self.model.signal_encoders, x)  # sorted: the token order, wav2sleep.py:311
         with torch.cuda.device(device):
             self._ensure_packed(device)
-            names = sorted(x.keys())  # token order of the mixer, wav2sleep.py:311
             buf = self._buffers(device, names, B, S)
-            xs = {}
-            for n in names:
-                t = x[n].detach()
-                xs[n] = t if (t.dtype == torch.float32 and t.is_contiguous()) else t.to(torch.float32).contiguous()
+            xs = {n: _f32(x[n]) for n in names}
             in_bytes = sum(t.numel() * 4 for t in xs.values())
             if (self.use_graph and in_bytes <= self.GRAPH_MAX_INPUT_BYTES and buf.get("calls", 0) >= 1
                     and not torch.cuda.is_current_stream_capturing()):
@@ -486,9 +520,4 @@ class ForwardEngine:
 
     @torch.no_grad()
     def predict(self, x: dict[str, Tensor]) -> Tensor:
-        logits = self.forward(x)
-        B, S, Cn = logits.shape
-        out = torch.empty(B, S, dtype=torch.int64, device=logits.device)
-        with torch.cuda.device(logits.device):
-            _lib.check(self.lib.w2s_argmax(logits.data_ptr(), B * S, Cn, out.data_ptr(), _stream()))
-        return out
+        return _argmax(self.lib, self.forward(x))

@@ -34,19 +34,10 @@ import torch
 from torch import Tensor, nn
 
 from . import _lib
-from .engine import _stream
-from .training import _rank
+from .engine import _argmax, _dropout_seed, _f32, _p, _stream, check_inputs
 
 ACT = {"linear": 0, "relu": 1, "leaky": 2, "gelu": 3, "silu": 4, "swish": 4}
 NORM_INSTANCE, NORM_GROUP, NORM_BATCH = 0, 1, 2
-
-
-def _f(t: Tensor | None):
-    return None if t is None else t.detach().to(torch.float32).contiguous()
-
-
-def _p(t: Tensor | None):
-    return None if t is None else t.data_ptr()
 
 
 def _g(t: Tensor) -> Tensor:
@@ -62,14 +53,14 @@ class _Conv(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, w, bias, eng, L_out, stride, dil, pad_left, mask, taps_major, raw):
         B, L_in, cin = x.shape
-        xd, wd = _f(x), _f(w)
+        xd, wd = _f32(x), _f32(w)
         if taps_major:
             cout, taps = wd.shape[0], wd.shape[1] // cin
         else:
             cout, _, taps = wd.shape
         out = torch.zeros(B, L_out, cout, dtype=torch.float32, device=x.device)
-        _lib.check(eng.lib.w2s_gen_conv(xd.data_ptr(), wd.data_ptr(), _p(_f(bias)), out.data_ptr(), _p(mask), B, L_in, L_out,
-                                        cin, cout, taps, stride, dil, pad_left, taps_major, raw, _stream()))
+        _lib.check(eng.lib.w2s_gen_conv(xd.data_ptr(), wd.data_ptr(), _p(_f32(bias)), out.data_ptr(), _p(mask), B, L_in,
+                                        L_out, cin, cout, taps, stride, dil, pad_left, taps_major, raw, _stream()))
         ctx.save_for_backward(xd, wd, mask)
         ctx.eng, ctx.has_bias = eng, bias is not None
         ctx.geo = (B, L_in, L_out, cin, cout, taps, stride, dil, pad_left, taps_major, raw)
@@ -101,7 +92,7 @@ class _AffineAct(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, scale, shift, res, eng, act, mask, per_channel):
         B, L, Cc = x.shape
-        xd, sc, sh, rs = _f(x), _f(scale), _f(shift), _f(res)
+        xd, sc, sh, rs = _f32(x), _f32(scale), _f32(shift), _f32(res)
         out = torch.zeros_like(xd)
         _lib.check(eng.lib.w2s_gen_affine_act(xd.data_ptr(), _p(sc), _p(sh), _p(rs), out.data_ptr(), _p(mask), B, L, Cc,
                                               ACT[act], per_channel, _stream()))
@@ -135,11 +126,11 @@ class _BatchNormConsts(torch.autograd.Function):
     def forward(ctx, weight, bias, eng, running_mean, running_var, eps):
         Cc = running_mean.numel()
         dev = running_mean.device
-        rm, rv = _f(running_mean), _f(running_var)
+        rm, rv = _f32(running_mean), _f32(running_var)
         scale = torch.empty(1, Cc, dtype=torch.float32, device=dev)
         shift = torch.empty(1, Cc, dtype=torch.float32, device=dev)
-        _lib.check(eng.lib.w2s_gen_norm_consts(None, _p(_f(weight)), _p(_f(bias)), rm.data_ptr(), rv.data_ptr(), scale.data_ptr(),
-                                               shift.data_ptr(), 1, Cc, 1, NORM_BATCH, 1, eps, _stream()))
+        _lib.check(eng.lib.w2s_gen_norm_consts(None, _p(_f32(weight)), _p(_f32(bias)), rm.data_ptr(), rv.data_ptr(),
+                                               scale.data_ptr(), shift.data_ptr(), 1, Cc, 1, NORM_BATCH, 1, eps, _stream()))
         ctx.save_for_backward(rm, rv)
         ctx.eng, ctx.eps = eng, eps
         return scale, shift
@@ -172,7 +163,7 @@ class _BatchNormTrainAct(torch.autograd.Function):
         if rows >= 2 ** 31:
             raise ValueError(f"train-mode BatchNorm over {rows} rows: at most 2^31 - 1")
         lib, dev = eng.lib, y.device
-        yd, w, b = _f(y), _f(weight), _f(bias)
+        yd, w, b = _f32(y), _f32(weight), _f32(bias)
         stats = torch.empty(1, Cc, 2, dtype=torch.float64, device=dev)
         _lib.check(lib.w2s_gen_bn_stats(yd.data_ptr(), stats.data_ptr(), rows, Cc, _stream()))
         if norm.track_running_stats and norm.running_mean is not None:
@@ -221,7 +212,7 @@ class _NormAct(torch.autograd.Function):
     def forward(ctx, y, weight, bias, eng, groups, mode, eps, act, mask):
         B, L, Cc = y.shape
         lib, dev = eng.lib, y.device
-        yd, w, b = _f(y), _f(weight), _f(bias)
+        yd, w, b = _f32(y), _f32(weight), _f32(bias)
         stats = torch.zeros(B, Cc, 2, dtype=torch.float64, device=dev)
         _lib.check(lib.w2s_gen_stats(yd.data_ptr(), stats.data_ptr(), _p(mask), B, L, Cc, _stream()))
         scale = torch.zeros(B, Cc, dtype=torch.float32, device=dev)
@@ -259,7 +250,7 @@ class _RowNorm(torch.autograd.Function):
     def forward(ctx, x, weight, bias, eng, eps, act, rms):
         Cc = x.shape[-1]
         rows = x.numel() // Cc
-        xd, w, b = _f(x), _f(weight), _f(bias)
+        xd, w, b = _f32(x), _f32(weight), _f32(bias)
         out = torch.empty_like(xd)
         _lib.check(eng.lib.w2s_gen_rownorm(xd.data_ptr(), _p(w), _p(b), out.data_ptr(), rows, Cc, rms, ACT[act], eps,
                                            _stream()))
@@ -286,7 +277,7 @@ class _Attn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, qkv, eng, km, N, D, H, p, seed, site):
-        qkv = _f(qkv)
+        qkv = _f32(qkv)
         F3 = qkv.shape[1]
         Fd = F3 // 3
         o = torch.empty(qkv.shape[0], Fd, dtype=torch.float32, device=qkv.device)
@@ -314,7 +305,7 @@ class _Attn(torch.autograd.Function):
 class _Dropout(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, eng, p, seed, site):
-        xd = _f(x)
+        xd = _f32(x)
         out = torch.empty_like(xd)
         _lib.check(eng.lib.w2s_gen_dropout(xd.data_ptr(), out.data_ptr(), None, xd.numel(), p, seed, site, _stream()))
         ctx.eng, ctx.cfg = eng, (p, seed, site)
@@ -334,7 +325,7 @@ class _Broadcast(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, row, eng, n):
-        rd = _f(row)
+        rd = _f32(row)
         ctx.eng = eng
         return torch.empty(n, rd.shape[0], dtype=torch.float32, device=rd.device).copy_(rd)
 
@@ -447,11 +438,10 @@ class GeneralEngine:
 
     # ------------------------------------------------------------------ stages
     def encode(self, enc, x_BT: Tensor):
-        """SignalEncoder.forward (wav2sleep.py:235-267) -> (z [B, S, F], mask [B] uint8)."""
+        """SignalEncoder.forward (wav2sleep.py:235-267) -> (z [B, S, F], mask [B] uint8).  x_BT has passed
+        ``check_inputs``."""
         B, T = x_BT.shape
         spe = enc.samples_per_epoch
-        if T % spe:
-            raise ValueError(f"Input length {T} must be divisible by self.samples_per_epoch={spe}.")
         S = T // spe
         xs = x_BT.to(torch.float32).contiguous()  # stays on the autograd graph when the input requires grad
         mask = torch.isinf(xs.detach()[:, 0]).to(torch.uint8).contiguous()  # data-dependent control, no arithmetic
@@ -538,11 +528,7 @@ class GeneralEngine:
         """The scope of one training forward: dropout at every site the reference applies it in training, with masks
         from ``dropout_seed`` (None: a seed drawn from torch's CPU generator, distinct per rank), and train-mode
         BatchNorm (batch statistics, running-statistics update)."""
-        if self.dropout_seed is not None:
-            seed = int(self.dropout_seed)
-        else:
-            seed = int(torch.randint(0, 2 ** 62, (1,)).item()) ^ (0x5851F42D4C957F2D * (1 + _rank()) & (2 ** 62 - 1))
-        self.last_dropout_seed = self._seed = seed
+        self.last_dropout_seed = self._seed = _dropout_seed(self.dropout_seed)
         try:
             yield
         finally:
@@ -555,29 +541,11 @@ class GeneralEngine:
 
     def _forward(self, x: dict[str, Tensor]) -> Tensor:
         m = self.model
-        if not isinstance(x, dict) or len(x) == 0:
-            raise ValueError("No signals provided to MultiModalAttentionEmbedder.")
-        names = sorted(x.keys())  # token order of the mixer, wav2sleep.py:311
+        names, B, S, dev = check_inputs(m.signal_encoders, x)  # sorted: the token order, wav2sleep.py:311
         zs, masks = [], []
-        B = S = None
-        for n in names:
-            if n not in m.signal_encoders.signal_map:
-                raise KeyError(f"Signal {n!r} has no encoder (valid: {list(m.signal_encoders.signal_map)})")
-            t = x[n]
-            if not isinstance(t, Tensor) or t.dim() != 2:
-                raise ValueError(f"{n}: expected a [B, T] tensor")
-            if not t.is_cuda:
-                raise RuntimeError("wav2sleep_b200 runs on CUDA (sm_100a) only: move inputs with .to('cuda'); "
-                                   "there is no CPU fallback")
-        dev = x[names[0]].device
         with torch.cuda.device(dev):
             for n in names:
-                t = x[n]
-                z, mask = self.encode(m.signal_encoders.get_encoder(n), t)
-                if B is None:
-                    B, S = z.shape[0], z.shape[1]
-                elif (z.shape[0], z.shape[1]) != (B, S):
-                    raise ValueError(f"{n}: batch/epoch count {tuple(z.shape[:2])} differs from {(B, S)}")
+                z, mask = self.encode(m.signal_encoders.get_encoder(n), x[n])
                 if m.signal_encoders.embed_signals:  # wav2sleep.py:155-159
                     e = m.signal_encoders.embedder.weight[m.signal_encoders.sig_to_embedding_idx[n]]
                     z = self.affine_act(z, "linear", shift=e, mask=mask, per_channel=1)
@@ -589,9 +557,4 @@ class GeneralEngine:
 
     @torch.no_grad()
     def predict(self, x: dict[str, Tensor]) -> Tensor:
-        logits = self.forward(x)
-        B, S, Cn = logits.shape
-        out = torch.empty(B, S, dtype=torch.int64, device=logits.device)
-        with torch.cuda.device(logits.device):
-            _lib.check(self.lib.w2s_argmax(logits.data_ptr(), B * S, Cn, out.data_ptr(), _stream()))
-        return out
+        return _argmax(self.lib, self.forward(x))

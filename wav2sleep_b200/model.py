@@ -243,16 +243,13 @@ class SignalEncoders(nn.Module):
         plus the optional signal-source embedding.  ``Wav2Sleep.forward`` does not come through here (its fused path
         keeps the features in fp16 and hands masks over separately); this entry runs the dimension-generic fp32 CUDA
         kernels for every configuration."""
+        from .engine import check_inputs
         from .general import GeneralEngine  # deferred: loads the CUDA library
+        check_inputs(self, x, joint=False)  # each signal is encoded on its own
         if getattr(self, "_general", None) is None:
             object.__setattr__(self, "_general", GeneralEngine(None))
         eng, out = self._general, {}
         for name, x_BT in x.items():
-            if name not in self.signal_map:
-                raise KeyError(f"Signal {name!r} has no encoder (valid: {list(self.signal_map)})")
-            if not x_BT.is_cuda:
-                raise RuntimeError("wav2sleep_b200 runs on CUDA (sm_100a) only: move inputs with .to('cuda'); "
-                                   "there is no CPU fallback")
             with torch.no_grad(), torch.cuda.device(x_BT.device):
                 z, mask = eng.encode(self.get_encoder(name), x_BT)
                 if self.embed_signals:  # wav2sleep.py:155-159 (the reference adds it to the -inf rows as well)

@@ -31,8 +31,8 @@ import torch
 from torch import Tensor
 
 from . import _lib
-from .engine import _stream
-from .general import ACT, GeneralEngine, _f, _p
+from .engine import _argmax, _f32, _p, _stream, check_inputs
+from .general import ACT, GeneralEngine
 from .model import Wav2Sleep
 
 _PER_POSITION_NORMS = ("batch", "layer", "rms", None)
@@ -142,12 +142,7 @@ class StreamingSession:
 
     def predict_step(self, x: dict[str, Tensor]) -> Tensor:
         """Most likely class of each new epoch, int64 [N, R] (the argmax kernel of ``Wav2Sleep.predict``)."""
-        logits = self.step(x)
-        N, R, Cn = logits.shape
-        out = torch.empty(N, R, dtype=torch.int64, device=logits.device)
-        with torch.cuda.device(logits.device):
-            _lib.check(self.lib.w2s_argmax(logits.data_ptr(), N * R, Cn, out.data_ptr(), _stream()))
-        return out
+        return _argmax(self.lib, self.step(x))
 
     def reset(self, streams=None) -> None:
         """Zero every carried state of the given stream indices (all streams if None): they start a new night."""
@@ -173,7 +168,7 @@ class StreamingSession:
             return self.eng.encode(enc, x_NT)
         N, T = x_NT.shape
         R = T // enc.samples_per_epoch
-        xs = _f(x_NT)
+        xs = _f32(x_NT)
         mask = torch.isinf(xs[:, 0]).to(torch.uint8).contiguous()  # data-dependent control, no arithmetic
         ctx = self.context[name]
         a, raw = xs.view(N, T, 1), 1
@@ -206,11 +201,11 @@ class StreamingSession:
         N, R, Fd = feat.shape
         if N != self.n_streams or Fd != m.sequence_mixer.feature_dim:
             raise ValueError(f"features {tuple(feat.shape)} do not match [{self.n_streams}, R, {m.sequence_mixer.feature_dim}]")
-        x = _f(feat)
+        x = _f32(feat)
         keep = [x]  # every fp32 tensor the descriptor points to stays referenced until the launch is enqueued
 
         def ptr(t):
-            t = _f(t)
+            t = _f32(t)
             keep.append(t)
             return _p(t)
 
@@ -242,30 +237,12 @@ class StreamingSession:
 
     # ------------------------------------------------------------------ input checks (host side, before any launch)
     def _check(self, x) -> int:
-        encs = self.model.signal_encoders
-        if not isinstance(x, dict) or len(x) == 0:
-            raise ValueError("No signals provided to StreamingSession.step.")
-        R = None
-        for name, t in x.items():
-            if name not in encs.signal_map:
-                raise ValueError(f"Signal {name!r} has no encoder (valid: {list(encs.signal_map)})")
-            if not isinstance(t, Tensor) or t.dim() != 2:
-                raise ValueError(f"{name}: expected a [N, R * samples_per_epoch] tensor")
-            if not t.is_cuda:
-                raise RuntimeError("wav2sleep_b200 runs on CUDA (sm_100a) only: move inputs with .to('cuda'); there is no "
-                                   "CPU fallback")
-            if t.device != self.device:
-                raise RuntimeError(f"{name}: input on {t.device}, session on {self.device}")
-            if t.shape[0] != self.n_streams:
-                raise ValueError(f"{name}: {t.shape[0]} rows, the session has {self.n_streams} streams")
-            spe = encs.get_encoder(name).samples_per_epoch
-            if t.shape[1] == 0 or t.shape[1] % spe:
-                raise ValueError(f"{name}: input length {t.shape[1]} must be a positive multiple of samples_per_epoch={spe}")
-            r = t.shape[1] // spe
-            if R is not None and r != R:
-                raise ValueError(f"{name}: {r} epochs in this call, other signals have {R}")
-            R = r
-        if self.n_streams * R > 65535:
+        _, N, R, device = check_inputs(self.model.signal_encoders, x)
+        if device != self.device:
+            raise RuntimeError(f"input on {device}, session on {self.device}")
+        if N != self.n_streams:
+            raise ValueError(f"{N} rows, the session has {self.n_streams} streams")
+        if N * R > 65535:
             raise ValueError(f"{self.n_streams} streams x {R} epochs exceed the 65535 epoch rows the encoder kernels take per "
                              "call; send fewer epochs per call")
         return R

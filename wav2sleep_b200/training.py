@@ -40,18 +40,9 @@ from torch import Tensor
 
 from . import _lib
 from ._lib import PRO_DNORM, ConvCall, EPI_ACT_BWD, EPI_PLAIN, PRO_NONE
-from .engine import ForwardEngine, _stream
+from .engine import ForwardEngine, _dropout_seed, _f32, _p, _stream, check_inputs
 
 F16 = torch.float16
-
-
-def _p(t):
-    return None if t is None else C.c_void_p(t.data_ptr())
-
-
-def _rank() -> int:
-    import torch.distributed as dist
-    return dist.get_rank() if dist.is_available() and dist.is_initialized() else 0
 
 
 class TrainEngine(ForwardEngine):
@@ -290,7 +281,7 @@ class TrainEngine(ForwardEngine):
         st = _stream()
         enc = m.signal_encoders.get_encoder(n)
         pe = self.enc[m.signal_encoders.signal_map[n]]
-        xs = x_n.detach().to(torch.float32).contiguous()
+        xs = _f32(x_n)
         if side_stream is not None:
             xs.record_stream(side_stream)
         T = xs.size(1)
@@ -321,7 +312,7 @@ class TrainEngine(ForwardEngine):
         _lib.check(lib.w2s_enc_act_fwd(last["y3"].data_ptr(), last["r"].data_ptr(), last["s3"].data_ptr(),
                                        a_last.data_ptr(), mask.data_ptr(), B, L4, Cl, enc.norm_eps, st))
         z_pre = torch.zeros(B, S, 128, dtype=F16, device=device)
-        bl = self._f32(enc.linear.bias)
+        bl = _f32(enc.linear.bias)
         self.conv(a_last, e["tw"]["lin_fwd"], Cl, 128, 4, B, L4, S, z_pre, stride=4, bias=bl, row_mask=mask)
         z = torch.zeros(B, S, 128, dtype=F16, device=device)
         _lib.check(lib.w2s_gelu_fwd(z_pre.data_ptr(), z.data_ptr(), z.numel(), st))
@@ -334,19 +325,14 @@ class TrainEngine(ForwardEngine):
         """Training-mode forward.  The activations the backward needs are returned (``return_saved``: the autograd bridge
         keeps them on its ``ctx``, so several forwards may precede their backwards, like with torch autograd) and also
         remembered as ``self.saved`` for a direct ``backward(dlogits)`` call."""
-        B, S, device = self._check_inputs(x)
+        names, B, S, device = check_inputs(self.model.signal_encoders, x)
         lib, m = self.lib, self.model
         with torch.cuda.device(device):
             self._ensure_train_packed(device)
             st = _stream()
-            names = sorted(x.keys())
             N = B * S
             sv = {"B": B, "S": S, "names": names, "enc": {}, "device": device}
-            if self.dropout_seed is not None:
-                seed = int(self.dropout_seed)
-            else:
-                seed = int(torch.randint(0, 2 ** 62, (1,)).item()) ^ (0x5851F42D4C957F2D * (1 + _rank()) & (2 ** 62 - 1))
-            self.last_dropout_seed = seed
+            seed = self.last_dropout_seed = _dropout_seed(self.dropout_seed)
             p_mix = float(m.epoch_mixer.dropout) if m.training else 0.0
             sv.update(seed=seed, p_mix=p_mix)
             # ---- encoders (streaming kernels, every layer output kept), one CUDA stream each, longest first ----
@@ -366,14 +352,14 @@ class TrainEngine(ForwardEngine):
             ms = (C.c_void_p * len(names))(*[sv["enc"][n]["mask"].data_ptr() for n in names])
             tokens = torch.empty(T_tok, 128, dtype=F16, device=device)
             key_mask = torch.empty(T_tok, dtype=torch.uint8, device=device)
-            cls = self._f32(mix.register_tokens[0, 0, :, 0])
+            cls = _f32(mix.register_tokens[0, 0, :, 0])
             _lib.check(lib.w2s_tokens_fwd(zs, ms, cls.data_ptr(), tokens.data_ptr(), key_mask.data_ptr(), N, S, len(names), st))
             sv.update(D=D, key_mask=key_mask, layers=[])
             xcur = tokens
             for l, layer in enumerate(mix.transformer_encoder.layers):
                 tw = self.tw["mix"][l]
                 eps = layer.norm1.eps
-                f = self._f32
+                f = _f32
                 h1 = self.ln_fwd(xcur, f(layer.norm1.weight), f(layer.norm1.bias), T_tok, 0, eps)
                 qkv = []
                 bin_ = f(layer.self_attn.in_proj_bias)
@@ -423,7 +409,7 @@ class TrainEngine(ForwardEngine):
                     d = blk.dilations[k]
                     c = torch.empty(B, S, 128, dtype=F16, device=device)
                     self.conv(cur, self.tw["seq"][bi][k]["fwd"], 128, 128, 7, B, S, S, c, dil=d, pad=3 * d)
-                    g_, b_ = self._f32(layer.norm.weight.reshape(-1)), self._f32(layer.norm.bias.reshape(-1))
+                    g_, b_ = _f32(layer.norm.weight.reshape(-1)), _f32(layer.norm.bias.reshape(-1))
                     p_seq = float(blk.dropout.p) if m.training else 0.0
                     lrec = {"in": cur, "c": c, "g": g_, "b": b_, "eps": layer.norm.eps, "d": d}
                     if k == nl - 1 and p_seq > 0:  # gelu(dropout(layers(x)) + x), models/blocks.py:123-125
@@ -441,15 +427,11 @@ class TrainEngine(ForwardEngine):
                 blk_in = cur
             feat = blk_in
             logits = torch.empty(B, S, m.num_classes, dtype=torch.float32, device=device)
-            wc, bc = self._f32(m.classifier.weight), self._f32(m.classifier.bias)
+            wc, bc = _f32(m.classifier.weight), _f32(m.classifier.bias)
             _lib.check(lib.w2s_head_fwd(feat.data_ptr(), wc.data_ptr(), bc.data_ptr(), logits.data_ptr(), N, m.num_classes, st))
             sv.update(feat=feat, wc=wc)
             self.saved = sv
         return (logits, sv) if return_saved else logits
-
-    def _f32(self, t: Tensor) -> Tensor:
-        t = t.detach()
-        return t if (t.dtype == torch.float32 and t.is_contiguous()) else t.to(torch.float32).contiguous()
 
     # ================================================================== backward
     @torch.no_grad()
@@ -532,7 +514,7 @@ class TrainEngine(ForwardEngine):
             for l in reversed(range(len(sv["layers"]))):
                 L_, layer, tw = sv["layers"][l], mix.transformer_encoder.layers[l], self.tw["mix"][l]
                 eps = layer.norm1.eps
-                f = self._f32
+                f = _f32
                 # FFN
                 dW2, dW1 = G(layer.linear2.weight), G(layer.linear1.weight)
                 d_hact = torch.empty(4 * T_tok, 128, dtype=F16, device=device)
@@ -725,8 +707,8 @@ class TrainEngine(ForwardEngine):
                 if want_dx:
                     dx = torch.empty(B, L, dtype=torch.float32, device=device)
                     _lib.check(lib.w2s_first_conv_dgrad(e["x"].data_ptr(), dy1.data_ptr(), dr.data_ptr(),
-                                                        self._f32(blk.conv1.conv.weight).data_ptr(),
-                                                        self._f32(blk.downsample.weight).data_ptr(), mask.data_ptr(),
+                                                        _f32(blk.conv1.conv.weight).data_ptr(),
+                                                        _f32(blk.downsample.weight).data_ptr(), mask.data_ptr(),
                                                         dx.data_ptr(), B, L, self._inv_scale, st))
                     return dx
                 return None
@@ -780,5 +762,5 @@ class _TrainFn(torch.autograd.Function):
 def forward_with_grad(model, x: dict[str, Tensor]) -> Tensor:
     eng = model._get_train_engine()
     params = tuple(p for p in model.parameters() if p.requires_grad)
-    names = tuple(x.keys())
+    names = tuple(check_inputs(model.signal_encoders, x)[0])  # before x is unpacked
     return _TrainFn.apply(eng, names, *(x[n] for n in names), *params)
