@@ -263,7 +263,7 @@ int w2s_seqmixer_head_fwd(const w2s_seq_desc* d, const void* x, int B, int S, vo
  * ------------------------------------------------------------------------------------------------------- */
 /* C[m*ldc_m + n*ldc_n + t*ldc_t] += scale * sum_{b,l} X[b,l,m] * Y[b, l*y_stride + y_offset + t*tap_stride, n], t < taps
  * (weight gradients of nn.Linear (taps 1) and of all taps of an nn.Conv1d in one launch; for taps = 3, unit tap stride
- * and M, N <= 32, X and Y are read once for all taps).
+ * and M, N <= 64, X and Y are read once for all taps).
  * Built for the (M,N) pairs of the model: (16,16) (32,16) (32,32) (64,32) (64,64) (128,64) (128,128). */
 int w2s_gemm_tn(const void* X, const void* Y, float* C, int M, int N, int taps, int tap_stride, int B, int LX, int LY,
                 int y_stride, int y_offset, long long ldc_m, long long ldc_n, long long ldc_t, float scale,
@@ -338,8 +338,8 @@ int w2s_head_bwd(const void* feat, const float* w, const float* dlogits, void* d
  * ema != NULL: the same pass also updates ema = ema_decay * ema + (1 - ema_decay) * p_new, the per-batch update of the
  * reference's EMACallback (trainer/callbacks.py:54-66, SURVEY 8f N4). */
 int w2s_sumsq(const float* g, long long n, double* out, void* stream);
-/* *out = max |g[i]| (fp32; the call zeroes *out first).  Picks the loss scale of a backward whose incoming gradient is
- * not a mean cross entropy (input attribution; ABI v7). */
+/* *out = max |g[i]| (fp32; the call zeroes *out first; NaN if any g[i] is NaN).  Picks the loss scale of a backward
+ * whose incoming gradient is not a mean cross entropy (input attribution; ABI v7). */
 int w2s_absmax(const float* g, long long n, float* out, void* stream);
 /* Integrated gradients (ABI v10).  out [K * B, T] = the K interpolated batches out[k, b, t] = x0 + alphas[k] * (x - x0)
  * (alphas: K device floats; x0 NULL: zero baseline).  A non-finite x[b, t] is copied unchanged onto every step, so a

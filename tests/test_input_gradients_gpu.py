@@ -265,6 +265,21 @@ def test_zero_objective_gradient_launches_nothing(cuda_device):
     assert all(p.grad is not None and (p.grad == 0).all() for p in model.parameters())
 
 
+def test_nan_objective_gradient_propagates(cuda_device):
+    """A NaN in d(objective)/d(logits) reaches the input and parameter gradients, as with torch autograd: the max |dlogits|
+    that picks the loss scale must not drop the NaN and take the exact-zero shortcut above."""
+    model = build_default({"ECG": "ECG"}, 4, seed=0).to(cuda_device).eval()
+    x = {k: v.to(cuda_device).requires_grad_(True) for k, v in make_inputs({"ECG": "ECG"}, 2, 3, seed=1).items()}
+    logits = model(x)
+    w = torch.zeros_like(logits)
+    w[0, 1, 2] = float("nan")
+    (logits * w).sum().backward()
+    torch.cuda.synchronize()
+    assert torch.isnan(x["ECG"].grad).any()
+    no_nan = [n for n, p in model.named_parameters() if not torch.isnan(p.grad).any()]
+    assert not no_nan, no_nan
+
+
 def _profile_labels(lib, fn):
     lib.w2s_profile_enable(1)
     try:

@@ -12,6 +12,10 @@ arithmetic:
 * ``w2s_conv1d_fwd`` with ``W2S_EPI_PLAIN`` at every instance, in the output indexing each is used with;
 * ``w2s_enc_act_fwd/bwd``, ``w2s_enc_norm_bwd``, ``w2s_first_conv_wgrad``, ``w2s_row_ln_fwd/bwd``, ``w2s_gelu_fwd/bwd``,
   ``w2s_colsum`` and ``w2s_dropout``;
+* ``w2s_gemm_tn``, the weight-gradient GEMM behind almost every parameter gradient, at every call form of the training
+  step (``WG_FORMS``) and all 12 of its kernels, at tile edges, padding, masks (more than 512 nights too), prefilled C,
+  loss scales and full-night lengths, plus a replay of every call of a real backward;
+* ``w2s_sumsq``, ``w2s_absmax`` and ``w2s_adamw_step`` (200 steps against clip_grad_norm_ + AdamW + EMA in fp64);
 * the argument checks of those entry points (calls the kernels cannot run must fail with a message).
 
 References use the exact erf GELU (the reference model's ``nn.GELU()``) and ``torch.autograd`` of the forward formula.
@@ -724,6 +728,450 @@ def test_dropout(cuda_device, p, with_res, n):
     werr = _rel(out, wrong)
     print(f"  wrong reference ({what}): {werr:.2e} ({werr / DROP_TOL:.0f}x the bound)")
     assert werr >= 10 * DROP_TOL
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# e. the weight-gradient GEMM w2s_gemm_tn, at every call form of TrainEngine.backward
+# ---------------------------------------------------------------------------------------------------------------------
+# fp16 x fp16 products are exact in fp32, so the error is the fp32 accumulation alone: mma.sync chains over a CTA's rows,
+# the shared-memory k-group atomics and the fp32 global atomics across CTAs, on top of the C prefill (the kernel adds into
+# C).  Per element over sum |X| |Y| + |prefill|.  Set from the first B200 run (NVIDIA B200, 1000 W): worst 7.1e-7 (the
+# replayed calls of a backward; 3.8e-7 over the synthetic forms, 6.6e-8 at full-night lengths, where the zero-mean partial
+# sums stay far below sum |terms|), so 2e-6 (2.8x).  The closest wrong reference missed by 4.3e-4.
+WG_GEMM_TOL = 2e-6
+# C layouts: "MNT" a [M, N, taps] conv weight gradient (ldc_m = N taps, ldc_n = taps, ldc_t = 1); "MN" a row-major block
+# with ldc_m = N; "M4N" a column block of an [M, 4N] weight (ldc_m = 4N); "NM" the transposed block of linear1's weight
+# (ldc_m = 1, ldc_n = M).  The call forms of the training step, name -> [(M, N, taps, tap_stride > 1, y_stride, layout)]:
+WG_FORMS = {
+    "seq_conv": [(128, 128, 7, d > 1, 1, "MNT") for d in (1, 2)],              # sequence-mixer conv, dilation d
+    "ffn_linear2": [(128, 128, 1, False, 4, "M4N")],                           # FFN linear2, one call per j < 4
+    "ffn_linear1": [(128, 128, 1, False, 4, "NM")],                            # FFN linear1, one call per j < 4
+    "proj": [(128, 128, 1, False, 1, "MN")],                                   # out_proj, in_proj q / k / v
+    "enc_linear": [(128, cl, 1, False, 4, "M4N") for cl in (128, 64)],         # encoder Linear, one call per t < 4
+    "conv23": [(c, c, 3, False, 1, "MNT") for c in (16, 32, 64, 128)],         # encoder conv2 / conv3
+    "conv1": [(co, ci, 3, False, 1, "MNT") for co, ci in ACT_INSTANCES],       # encoder conv1 of blocks >= 1
+    "downsample": [(co, ci, 1, False, 2, "MN") for co, ci in ACT_INSTANCES],   # 1x1 stride-2 residual branch
+}
+WG_ALL_FORMS = {f for rows in WG_FORMS.values() for f in rows}
+# the 12 kernels w2s_gemm_tn is built with: (M, N, TAPS); TAPS = 3 is the fused kernel, TAPS = 1 runs one grid slice per tap
+WG_KERNELS = {(16, 16, 1), (32, 16, 1), (32, 32, 1), (64, 32, 1), (64, 64, 1), (128, 64, 1), (128, 128, 1),
+              (16, 16, 3), (32, 16, 3), (32, 32, 3), (64, 32, 3), (64, 64, 3)}
+
+
+def _tn_kernel(M, N, taps, ts, ys):
+    """The kernel w2s_gemm_tn dispatches a call to (capi.cu)."""
+    return (M, N, 3 if (taps == 3 and ts == 1 and ys == 1 and M <= 64 and N <= 64) else 1)
+
+
+def _tn_rows(M, N):
+    """X rows per tile (gemm_tn_rows)."""
+    return 512 if M + N <= 64 else 128
+
+
+def _tn_layout(M, N, taps, ldc_m, ldc_n, ldc_t):
+    if taps > 1:
+        return "MNT" if (ldc_m, ldc_n, ldc_t) == (N * taps, taps, 1) else f"other {ldc_m},{ldc_n},{ldc_t}"
+    return {(N, 1): "MN", (4 * N, 1): "M4N", (1, M): "NM"}.get((ldc_m, ldc_n), f"other {ldc_m},{ldc_n}")
+
+
+def _tn_calls(form, M, N, LX, d):
+    """The launches of one call form as TrainEngine.backward issues them -> (LY, elements of the C buffer, calls)."""
+    one = lambda ys, yo, ldc, c_off=0, taps=1, ts=1: dict(taps=taps, ts=ts, ys=ys, yo=yo, ldc=ldc, c_off=c_off)
+    if form == "seq_conv":
+        return LX, M * N * 7, [one(1, -3 * d, (N * 7, 7, 1), taps=7, ts=d)]
+    if form == "ffn_linear2":
+        return 4 * LX, M * 4 * N, [one(4, j, (4 * N, 1, 0), c_off=j * N) for j in range(4)]
+    if form == "ffn_linear1":
+        return 4 * LX, 4 * M * N, [one(4, j, (1, M, 0), c_off=j * M * N) for j in range(4)]
+    if form == "proj":
+        return LX, 3 * M * N, [one(1, 0, (N, 1, 0), c_off=j * M * N) for j in range(3)]
+    if form == "enc_linear":
+        return 4 * LX, M * 4 * N, [one(4, t, (4 * N, 1, 0), c_off=t * N) for t in range(4)]
+    if form in ("conv23", "conv1"):
+        return LX, M * N * 3, [one(1, -1, (3 * N, 3, 1), taps=3)]
+    assert form == "downsample"
+    return 2 * LX, M * N, [one(2, 0, (N, 1, 0))]
+
+
+def _tn_ref(X, Y, live, taps, ts, ys, yo, shift_last=False):
+    """fp64 sum over the live nights b and the rows l of X[b, l]^T Y[b, l ys + yo + t ts] (Y rows outside [0, LY) read
+    as zero), and of |X|^T |Y|: -> two [taps, M, N].  shift_last: a wrong reference whose last tap reads one row later."""
+    LX, M = X.shape[1:]
+    LY, N = Y.shape[1:]
+    x = X[live].to(F64).reshape(-1, M)
+    yl = Y[live]
+    ref = torch.empty(taps, M, N, dtype=F64, device="cuda")
+    absref = torch.empty_like(ref)
+    for t in range(taps):
+        rows = torch.arange(LX, device="cuda") * ys + yo + t * ts + (1 if shift_last and t == taps - 1 else 0)
+        ok = ((rows >= 0) & (rows < LY)).to(F64)[None, :, None]
+        y = (yl[:, rows.clamp(0, LY - 1)].to(F64) * ok).reshape(-1, N)
+        ref[t], absref[t] = x.t() @ y, x.abs().t() @ y.abs()
+    return ref, absref
+
+
+def _tn_index(M, N, taps, ldc, c_off):
+    """C element of every (tap, m, n) a call adds into: [taps, M, N]."""
+    ar = lambda k: torch.arange(k, device="cuda", dtype=torch.int64)
+    return c_off + ar(M)[None, :, None] * ldc[0] + ar(N)[None, None, :] * ldc[1] + ar(taps)[:, None, None] * ldc[2]
+
+
+def _tn_launch(X, Y, Cbuf, M, N, c, mask, scale):
+    B, LX, LY = X.shape[0], X.shape[1], Y.shape[1]
+    lib = _lib.load()
+    _lib.check(lib.w2s_gemm_tn(X.data_ptr(), Y.data_ptr(), Cbuf.data_ptr() + 4 * c["c_off"], M, N, c["taps"], c["ts"], B,
+                               LX, LY, c["ys"], c["yo"], *c["ldc"], scale, None if mask is None else mask.data_ptr(),
+                               G.stream()))
+    torch.cuda.synchronize()
+
+
+def _tn_err(before, after, idx, ref, absref, scale):
+    """Worst error of the elements a call adds into: after = before + scale ref, over scale sum |terms| + |before|."""
+    pre = before[idx].to(F64)
+    return _red(after[idx], pre + scale * ref, scale * absref + pre.abs())
+
+
+def _tn_check(tag, X, Y, mask, M, N, c, before, after, scale, wrong=False):
+    """Checks one launch: the elements it addresses against fp64, every other element of C bit for bit; wrong: also the
+    plausible wrong references.  -> the error."""
+    B = X.shape[0]
+    live = torch.ones(B, dtype=torch.bool, device="cuda") if mask is None else mask == 0
+    idx = _tn_index(M, N, c["taps"], c["ldc"], c["c_off"])
+    others = torch.ones_like(after, dtype=torch.bool)
+    others[idx.reshape(-1)] = False
+    assert torch.equal(after[others], before[others]), f"{tag}: C elements outside the call's slice changed"
+    if not bool(live.any()):
+        assert torch.equal(after, before), f"{tag}: every night masked, C must not change"
+        return 0.0
+    args = (c["taps"], c["ts"], c["ys"], c["yo"])
+    ref, absref = _tn_ref(X, Y, live, *args)
+    err = _tn_err(before, after, idx, ref, absref, scale)
+    assert err < WG_GEMM_TOL, (tag, err)
+    if not wrong:
+        return err
+    wrongs = [("tap shifted by one row", _tn_ref(X, Y, live, *args, shift_last=True)[0]),
+              ("y_offset off by one", _tn_ref(X, Y, live, *args[:3], c["yo"] + 1)[0])]
+    if c["ts"] > 1:
+        wrongs.append(("tap_stride 1 instead of d", _tn_ref(X, Y, live, c["taps"], 1, c["ys"], c["yo"])[0]))
+    if not bool(live.all()):
+        wrongs.append(("masked night included", _tn_ref(X, Y, torch.ones_like(live), *args)[0]))
+    if c["ldc"][:2] == (1, M):
+        wrongs.append(("C transposed", ref.transpose(1, 2)))
+    for what, w in wrongs:
+        if torch.equal(w, ref):  # e.g. the shifted tap reads only padding rows either way: no launch can tell them apart
+            print(f"  {tag}: wrong reference ({what}) equals the reference at this shape")
+            continue
+        werr = _tn_err(before, after, idx, w, absref, scale)
+        print(f"  {tag}: wrong reference ({what}) {werr:.2e} ({werr / WG_GEMM_TOL:.0f}x the bound)")
+        assert werr >= 10 * WG_GEMM_TOL, (tag, what, werr)
+    return err
+
+
+def _tn_case(form, M, N, d, B, LX, masks, scales, seed, wrong_for=None):
+    """Runs every launch of a call form over one random X, Y for each (mask, scale), each onto a random prefilled C."""
+    g = _gen(seed)
+    LY, nC, calls = _tn_calls(form, M, N, LX, d)
+    X, Y = _h((B, LX, M), g), _h((B, LY, N), g)
+    errs = []
+    for (mname, mask), scale in zip(masks, scales):
+        Cbuf = torch.randn(nC, generator=g, device="cuda") * (4 * scale)
+        for j, c in enumerate(calls):
+            before = Cbuf.clone()
+            _tn_launch(X, Y, Cbuf, M, N, c, mask, scale)
+            tag = f"gemm_tn {form} {M}x{N} d={d} B={B} L={LX} mask={mname} scale={scale:g} call {j}"
+            errs.append(_tn_check(tag, X, Y, mask, M, N, c, before, Cbuf, scale, wrong=(mname == wrong_for and j == 0)))
+    return max(errs)
+
+
+def _b3_masks():
+    m = lambda *v: torch.tensor(v, dtype=torch.uint8, device="cuda")
+    return [("none", None), ("middle", m(0, 1, 0)), ("first+last", m(1, 0, 1)), ("all", m(1, 1, 1))]
+
+
+WG_SCALES = (1.0, 2.0 ** -3, 2.0 ** -12, 2.0 ** -24)  # 1 and inverse loss scales (training.py auto_loss_scale: 2^2..2^24)
+WG_INSTANCES = ([("seq_conv", 128, 128, d) for d in (1, 2, 4, 8, 16, 32)]
+                + [(f, 128, 128, 0) for f in ("ffn_linear2", "ffn_linear1", "proj")]
+                + [("enc_linear", 128, cl, 0) for cl in (128, 64)]
+                + [("conv23", c, c, 0) for c in (16, 32, 64, 128)]
+                + [(f, co, ci, 0) for f in ("conv1", "downsample") for co, ci in ACT_INSTANCES])
+
+
+def _tn_forms_and_kernels(form, M, N, L, d):
+    """{(M, N, taps, tap_stride > 1, y_stride, layout)} and {kernel} of the launches of a call form."""
+    calls = _tn_calls(form, M, N, L, d)[2]
+    return ({(M, N, c["taps"], c["ts"] > 1, c["ys"], _tn_layout(M, N, c["taps"], *c["ldc"])) for c in calls},
+            {_tn_kernel(M, N, c["taps"], c["ts"], c["ys"]) for c in calls})
+
+
+def _tn_id(form, M, N, d, rest):
+    (k,) = _tn_forms_and_kernels(form, M, N, 1, d)[1]
+    return f"{form}-{M}x{N}" + (f"-d{d}" if form == "seq_conv" else "") + f"-kernel{k[0]}x{k[1]}x{k[2]}-{rest}"
+
+
+def _tn_lengths(form, M, N):
+    R = _tn_rows(M, N)  # one row, the tile edges, several tiles with a tail; S = 5 < 3d: padding on both sides
+    return [1, R - 1, R, R + 1, 2 * R + 37] + ([5] if form == "seq_conv" else [])
+
+
+WG_CASES = [pytest.param(f, M, N, d, L, id=_tn_id(f, M, N, d, f"L{L}"))
+            for f, M, N, d in WG_INSTANCES for L in _tn_lengths(f, M, N)]
+
+
+def test_gemm_tn_cases_cover_every_form_and_kernel():
+    forms, kernels = set(), set()
+    for p in WG_CASES:
+        f, k = _tn_forms_and_kernels(*p.values[:3], p.values[4], p.values[3])
+        assert f <= set(WG_FORMS[p.values[0]]), (p.id, f)  # the launches are the table's row
+        forms |= f
+        kernels |= k
+    assert forms == WG_ALL_FORMS, WG_ALL_FORMS - forms
+    assert kernels == WG_KERNELS, WG_KERNELS - kernels
+
+
+@pytest.mark.parametrize("form,M,N,d,L", WG_CASES)
+def test_gemm_tn_forms(cuda_device, form, M, N, d, L):
+    """Each launch of the form over 3 nights: no mask, the middle night masked, the first and last masked, all masked."""
+    err = _tn_case(form, M, N, d, 3, L, _b3_masks(), WG_SCALES, seed=M * 7 + N + L * 3 + d, wrong_for="middle")
+    print(f"gemm_tn {form} {M}x{N} d={d} L={L}: worst {err:.2e} (bound {WG_GEMM_TOL:.0e})")
+
+
+# B = 512 fills the kernel's list of live nights; with more nights it skips the tiles of masked nights one by one
+@pytest.mark.parametrize("form,M,N,L", [("conv23", 16, 16, 513), ("enc_linear", 128, 64, 129), ("conv23", 128, 128, 129)])
+@pytest.mark.parametrize("B", [512, 513, 600])
+def test_gemm_tn_many_nights(cuda_device, form, M, N, L, B):
+    g = _gen(B + M)
+    some = (torch.rand(B, generator=g, device="cuda") < 0.3).to(torch.uint8)
+    some[0] = some[-1] = 1
+    masks = [("some", some), ("all", torch.ones(B, dtype=torch.uint8, device="cuda")), ("none", None)]
+    err = _tn_case(form, M, N, 0, B, L, masks, WG_SCALES[1:], seed=B * 3 + M, wrong_for="some")
+    print(f"gemm_tn {form} {M}x{N} B={B} L={L}: worst {err:.2e} (bound {WG_GEMM_TOL:.0e})")
+
+
+# one case per family at the lengths of a B = 16 training batch of full nights (1200 epochs, 1024 ECG samples an epoch)
+WG_FULL = [("conv1", 16, 16, 0, 16, ECG_NIGHT // 2),                  # ECG block 1: 9.8 M rows, fused 16x16x3
+           ("conv23", 128, 128, 0, 16, ECG_NIGHT // 64),              # ECG block 6 conv2 / conv3
+           ("seq_conv", 128, 128, 0, 16, 1200),                       # every dilation
+           ("ffn_linear2", 128, 128, 0, 1, 16 * 1200 * 5),            # T = N D tokens, cardio
+           ("ffn_linear1", 128, 128, 0, 1, 16 * 1200 * 5)]
+
+
+@pytest.mark.parametrize("form,M,N,d,B,L", WG_FULL, ids=[f"{c[0]}-{c[1]}x{c[2]}-B{c[4]}-L{c[5]}" for c in WG_FULL])
+def test_gemm_tn_full_scale(cuda_device, form, M, N, d, B, L):
+    scale = 2.0 ** -17  # the inverse loss scale training.py picks for B x S = 19200 epochs
+    mask = None
+    if form in ("conv1", "conv23"):
+        mask = torch.zeros(B, dtype=torch.uint8, device="cuda")
+        mask[5] = 1
+    for dd in ((1, 2, 4, 8, 16, 32) if form == "seq_conv" else (d,)):
+        err = _tn_case(form, M, N, dd, B, L, [("night 5" if mask is not None else "none", mask)], [scale],
+                       seed=L + dd, wrong_for="night 5" if mask is not None else "none")
+        print(f"gemm_tn full scale {form} {M}x{N} d={dd} B={B} L={L}: worst {err:.2e} (bound {WG_GEMM_TOL:.0e})")
+        torch.cuda.empty_cache()
+
+
+@pytest.mark.parametrize("smap,n_cls,B,S,masked", [({"ABD": "ABD", "THX": "THX", "ECG": "ECG", "PPG": "PPG"}, 4, 3, 8,
+                                                     [("PPG", 1)]), ({"EOG-L": "EOG-L", "EOG-R": "EOG-R"}, 5, 2, 4, [])],
+                         ids=["cardio", "eog"])
+def test_gemm_tn_calls_of_a_backward(cuda_device, monkeypatch, smap, n_cls, B, S, masked):
+    """Every w2s_gemm_tn launch of a real training backward (dropout on), replayed against fp64 from the X, Y and
+    arguments it was given; its form must be a row of WG_FORMS, so a new call form fails here until it is tested."""
+    from conftest import make_inputs
+    from wav2sleep_b200 import build_default
+    from wav2sleep_b200.training import TrainEngine
+    orig = TrainEngine.gemm_tn
+    seen, errs = {}, []
+
+    def recorded(self, X, Y, Cbuf, M, N, B, LX, LY, ldc_m, ldc_n, y_stride=1, y_offset=0, row_mask=None, c_off=0,
+                 taps=1, ldc_t=0, tap_stride=1):
+        if Cbuf is None:
+            return orig(self, X, Y, Cbuf, M, N, B, LX, LY, ldc_m, ldc_n, y_stride, y_offset, row_mask, c_off, taps, ldc_t,
+                        tap_stride)
+        torch.cuda.synchronize()  # the launch runs on the weight-gradient side stream
+        before = Cbuf.detach().clone().view(-1)
+        orig(self, X, Y, Cbuf, M, N, B, LX, LY, ldc_m, ldc_n, y_stride, y_offset, row_mask, c_off, taps, ldc_t, tap_stride)
+        torch.cuda.synchronize()
+        form = (M, N, taps, tap_stride > 1, y_stride, _tn_layout(M, N, taps, ldc_m, ldc_n, ldc_t))
+        c = dict(taps=taps, ts=tap_stride, ys=y_stride, yo=y_offset, ldc=(ldc_m, ldc_n, ldc_t), c_off=c_off)
+        tag = f"backward call {len(errs)}: form {form} B={B} LX={LX} LY={LY} y_offset={y_offset} c_off={c_off}"
+        err = _tn_check(tag, X.reshape(B, LX, M), Y.reshape(B, LY, N), row_mask, M, N, c, before, Cbuf.view(-1),
+                        self._inv_scale)
+        errs.append(err)
+        seen[form] = seen.get(form, 0) + 1
+
+    monkeypatch.setattr(TrainEngine, "gemm_tn", recorded)
+    model = build_default(smap, n_cls, seed=0).to(cuda_device).train()  # default dropout p = 0.1 in both mixers
+    x = {k: v.to(cuda_device) for k, v in make_inputs(smap, B, S, masked=masked, seed=9).items()}
+    labels = torch.randint(0, n_cls, (B, S), generator=torch.Generator().manual_seed(9)).to(cuda_device)
+    F.cross_entropy(model(x).reshape(-1, n_cls), labels.reshape(-1)).backward()
+    torch.cuda.synchronize()
+    for form, k in sorted(seen.items()):
+        print(f"  {k:3d} x {form}")
+    print(f"{len(errs)} gemm_tn launches, worst {max(errs):.2e} (bound {WG_GEMM_TOL:.0e})")
+    assert set(seen) <= WG_ALL_FORMS, set(seen) - WG_ALL_FORMS
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# f. gradient norm, max |g| and the optimizer step: w2s_sumsq, w2s_absmax, w2s_adamw_step
+# ---------------------------------------------------------------------------------------------------------------------
+# sumsq: the squares of fp32 values are exact in fp64; fp64 sums per thread, warp shuffles, a block sum and one fp64
+# atomic per block.  Relative to sum g^2 (every term is positive).  Set from the first B200 run: worst 8.0e-16, so 2e-15
+# (2.5x).
+SUMSQ_TOL = 2e-15
+
+
+def _flat_grad_elements():
+    from wav2sleep_b200 import build_default
+    return sum(p.numel() for p in build_default({"ABD": "ABD", "THX": "THX", "ECG": "ECG", "PPG": "PPG"}, 4).parameters())
+
+
+def _reduction_sizes():
+    # one element, one block +- 2, past the 2 x SMs x 256 grid cap (the grid-stride loop runs 3 times), the flat gradient
+    return [1, 255, 257, 3 * 2 * _sms() * 256 + 77, _flat_grad_elements()]
+
+
+@pytest.mark.parametrize("which", range(5))
+def test_sumsq(cuda_device, which):
+    lib = _lib.load()
+    n = _reduction_sizes()[which]
+    g = torch.randn(n, generator=_gen(n), device="cuda") * 0.05
+    out = torch.zeros(1, dtype=F64, device="cuda")
+    _lib.check(lib.w2s_sumsq(g.data_ptr(), n, out.data_ptr(), G.stream()))
+    torch.cuda.synchronize()
+    ref = (g.to(F64) ** 2).sum()
+    err = ((out[0] - ref).abs() / ref).item()
+    print(f"sumsq n={n}: {err:.2e} (bound {SUMSQ_TOL:.0e})")
+    assert err < SUMSQ_TOL
+    if n > 2 * _sms() * 256:  # wrong: the grid-stride loop run once
+        werr = ((out[0] - (g[:2 * _sms() * 256].to(F64) ** 2).sum()).abs() / ref).item()
+        print(f"  wrong reference (grid-stride loop run once): {werr:.2e} ({werr / SUMSQ_TOL:.0f}x the bound)")
+        assert werr >= 10 * SUMSQ_TOL
+    for bad, expect in (([float("inf")], math.inf), ([float("-inf")], math.inf), ([float("nan")], None),
+                        ([float("inf"), float("nan")], None)):
+        gb = g.clone()
+        gb[0] = bad[0]
+        gb[n - 1] = bad[-1]
+        out.zero_()
+        _lib.check(lib.w2s_sumsq(gb.data_ptr(), n, out.data_ptr(), G.stream()))
+        torch.cuda.synchronize()
+        v = out.item()
+        assert (math.isnan(v) if expect is None else v == expect), (n, bad, v)
+
+
+def _absmax(lib, g):
+    out = torch.full((1,), 7.0, device="cuda")  # the call zeroes *out itself
+    _lib.check(lib.w2s_absmax(g.data_ptr(), g.numel(), out.data_ptr(), G.stream()))
+    torch.cuda.synchronize()
+    return out
+
+
+@pytest.mark.parametrize("which", range(5))
+def test_absmax(cuda_device, which):
+    """max |g| is exact: bit for bit torch's g.abs().max(), NaN if any element is NaN."""
+    lib = _lib.load()
+    n = _reduction_sizes()[which]
+    gen = _gen(n + 1)
+    base = torch.randn(n, generator=gen, device="cuda")
+    sub = torch.rand(n, generator=gen, device="cuda") * 1e-39  # subnormal magnitudes (fp32 normal range ends at 1.2e-38)
+    neg0 = torch.full((n,), -0.0, device="cuda")
+    cases = {"normal": base.clone(), "subnormal": -sub, "-0.0": neg0.clone(), "subnormal and -0.0": torch.where(
+        torch.arange(n, device="cuda") % 2 == 0, sub, neg0)}
+    cases["normal"][n // 2] = -0.0
+    cases["normal"][n - 1] = 1e-40
+    for what, v in (("+inf", float("inf")), ("-inf", float("-inf"))):
+        cases[what] = base.clone()
+        cases[what][n // 3] = v
+    for at in sorted({0, n - 1}):  # NaN at the first and at the last index, zeros elsewhere ([NaN, 0, ...])
+        cases[f"NaN at {at}, zeros"] = torch.zeros(n, device="cuda")
+        cases[f"NaN at {at}, zeros"][at] = float("nan")
+        cases[f"NaN at {at}, -inf"] = base.clone()
+        cases[f"NaN at {at}, -inf"][at] = float("nan")
+        cases[f"NaN at {at}, -inf"][n // 2] = float("-inf")
+    for what, g in cases.items():
+        got, ref = _absmax(lib, g), g.abs().max().reshape(1)
+        print(f"absmax n={n} {what}: {got.item()!r} (torch {ref.item()!r})")
+        if torch.isnan(ref).item():
+            assert torch.isnan(got).item(), (n, what, got.item())
+        else:
+            assert got.view(torch.int32).item() == ref.view(torch.int32).item(), (n, what, got.item(), ref.item())
+
+
+# adamw_step: 200 steps of fp32 state against an fp64 restatement of clip_grad_norm_ + torch.optim.AdamW + the EMA,
+# fed the same gradients and the same fp32 hyperparameters.  The fp32 rounding of p, m, v and the EMA at every step
+# accumulates over the steps.  p and the EMA are compared by their displacement from the start (max-abs error over
+# max |p_ref - p0|), where the per-step rounding of p ~ 1 (2^-24 each, ~0.01 of displacement after 200 steps) dominates:
+# worst 7.1e-4 on the first B200 run, so 2e-3 (2.8x).  m and v over their largest value: worst 1.6e-7 and 9.3e-7, so
+# 2.5e-6 (2.7x).  (An fp64 reference with beta2 = 0.999 instead of the fp32 beta2 misses v by 1.2e-5: 1 - beta2 is
+# 1.3e-5 off in fp32.)
+ADAMW_TOL = 2e-3
+ADAMW_MV_TOL = 2.5e-6
+_f32r = lambda v: float(torch.tensor(v, dtype=torch.float32))  # a hyperparameter as the kernel receives it
+
+
+def _adamw_ref(p, g, m, v, ema, t, lr, b1, b2, eps, wd, max_norm, grad_scale, decay):
+    g = g * grad_scale
+    if max_norm > 0:
+        g = g * min(1.0, max_norm / (g.norm().item() + 1e-6))  # torch.nn.utils.clip_grad_norm_
+    p = p * (1 - lr * wd)
+    m = b1 * m + (1 - b1) * g
+    v = b2 * v + (1 - b2) * g * g
+    p = p - lr / (1 - b1 ** t) * m / ((v / (1 - b2 ** t)).sqrt() + eps)
+    if ema is not None:
+        ema = decay * ema + (1 - decay) * p
+    return p, m, v, ema
+
+
+@pytest.mark.parametrize("mode", ["clip_ema", "grad_scale_clip_ema", "no_clip"])
+def test_adamw_step_200_steps(cuda_device, mode):
+    lib = _lib.load()
+    n, steps = 100_003, 200
+    lr, b1, b2, eps, wd, max_norm, decay = (_f32r(v) for v in (1e-3, 0.9, 0.999, 1e-8, 1e-2, 1.0, 0.99))
+    grad_scale = 2.0 ** -7 if mode == "grad_scale_clip_ema" else 1.0
+    clip = mode != "no_clip"
+    gen = _gen(len(mode))
+    p0 = torch.randn(n, generator=gen, device="cuda")
+    p, m, v = p0.clone(), torch.zeros(n, device="cuda"), torch.zeros(n, device="cuda")
+    ema = p0.clone() if clip else None
+    rp, rm, rv, rema = p0.to(F64), torch.zeros(n, dtype=F64, device="cuda"), torch.zeros(n, dtype=F64, device="cuda"), \
+        (p0.to(F64) if clip else None)
+    wp = p0.to(F64)  # wrong reference: clipping ignored (clip modes) / no bias correction
+    wm, wv = torch.zeros_like(rm), torch.zeros_like(rv)
+    nsq = torch.zeros(1, dtype=F64, device="cuda")
+    clipped = 0
+    for t in range(1, steps + 1):
+        # |g| ~ 316 x the step's scale: clipping to 1.0 is active on two steps of three
+        s = (0.02 if t % 3 else 0.001) / grad_scale
+        g = torch.randn(n, generator=gen, device="cuda") * s
+        clipped += int((g.to(F64) * grad_scale).norm().item() > max_norm)
+        gn = None  # no_clip: gnorm_sq NULL, with max_norm still set, turns clipping off
+        if clip:
+            nsq.zero_()
+            _lib.check(lib.w2s_sumsq(g.data_ptr(), n, nsq.data_ptr(), G.stream()))
+            gn = nsq.data_ptr()
+        _lib.check(lib.w2s_adamw_step(p.data_ptr(), g.data_ptr(), m.data_ptr(), v.data_ptr(), n, gn, lr, b1, b2, eps, wd,
+                                      max_norm, grad_scale, t, None if ema is None else ema.data_ptr(),
+                                      decay, G.stream()))
+        g64 = g.to(F64)
+        rp, rm, rv, rema = _adamw_ref(rp, g64, rm, rv, rema, t, lr, b1, b2, eps, wd, max_norm if clip else 0.0,
+                                      grad_scale, decay)
+        if clip:
+            wp, wm, wv, _ = _adamw_ref(wp, g64, wm, wv, None, t, lr, b1, b2, eps, wd, 0.0, grad_scale, decay)
+        else:  # bias corrections 1 - beta^t dropped (t = 1e9)
+            wp, wm, wv, _ = _adamw_ref(wp, g64, wm, wv, None, 10 ** 9, lr, b1, b2, eps, wd, 0.0, grad_scale, decay)
+    torch.cuda.synchronize()
+    if clip:
+        assert 0 < clipped < steps, clipped
+    disp = (rp - p0.to(F64)).abs().max()
+    errs = {"p": ((p.to(F64) - rp).abs().max() / disp).item(), "m": _rel(m, rm), "v": _rel(v, rv)}
+    if ema is not None:
+        errs["ema"] = ((ema.to(F64) - rema).abs().max() / (rema - p0.to(F64)).abs().max()).item()
+    print(f"adamw {mode}" + (f" ({clipped} of {steps} steps clipped)" if clip else "") + ": "
+          + ", ".join(f"{k} {e:.2e}" for k, e in errs.items()) + f" (bounds p, ema {ADAMW_TOL:.0e} / m, v {ADAMW_MV_TOL:.1e})")
+    for k, e in errs.items():
+        assert e < (ADAMW_MV_TOL if k in ("m", "v") else ADAMW_TOL), (mode, k, e)
+    werr = ((p.to(F64) - wp).abs().max() / disp).item()
+    what = "clipping ignored" if clip else "no bias correction"
+    print(f"  wrong reference ({what}): {werr:.2e} ({werr / ADAMW_TOL:.0f}x the bound)")
+    assert werr >= 10 * ADAMW_TOL
 
 
 # ---------------------------------------------------------------------------------------------------------------------

@@ -866,13 +866,15 @@ __global__ void __launch_bounds__(256) sumsq_kernel(const float* g, long long n,
     atomicAdd(out, t);
   }
 }
-// out = max |g| (as the bit pattern of a non-negative float, so an integer atomicMax orders it); *out zeroed by the caller
+// out = max |g|; *out zeroed by the caller.  The reduction runs on the bit patterns of |g|: an unsigned max orders every
+// non-negative float (subnormals and +inf included) and sorts NaN above +inf, so a NaN anywhere makes the result NaN
+// (fmaxf would drop it and could report 0 for [NaN, 0, ...]).
 __global__ void __launch_bounds__(256) absmax_kernel(const float* g, long long n, unsigned int* out) {
-  float m = 0.0f;
+  unsigned int m = 0u;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
-    m = fmaxf(m, fabsf(g[i]));
-  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-  if ((threadIdx.x & 31) == 0) atomicMax(out, __float_as_uint(m));
+    m = max(m, __float_as_uint(fabsf(g[i])));
+  for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) atomicMax(out, m);
 }
 struct AdamWArgs {
   float* p; const float* g; float* m; float* v; long long n;
