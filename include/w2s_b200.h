@@ -86,7 +86,7 @@ typedef struct w2s_conv_call {
   const void* w;          /* packed fp16 */
   const void* w_ds;       /* packed fp16 1x1          (has_ds) */
   void* out;              /* fp16 [B, L_out, cout] */
-  void* out_ds;           /* fp16 [B, L_out/2, cout]  (has_ds) */
+  void* out_ds;           /* fp16 [B, L_out/2, cout]  (has_ds; row j: 1x1 branch of row 2j, L_out/2 rounded down) */
   double* out_stats;      /* [B, cout, 2], pre-zeroed (W2S_EPI_STATS) */
   const uint8_t* row_mask;/* [B] or NULL */
   const float* bias;      /* [cout] (W2S_EPI_BIAS_GELU) */
@@ -102,7 +102,8 @@ typedef struct w2s_conv_call {
    * rows (0, 0, 0 = dense: stride 1, offset 0, out_rows = L_out); res uses the same indexing. */
   int32_t out_stride, out_offset, out_rows;
   /* block-0 fusion (W2S_PRO_FIR: the input is conv1(x) recomputed from the raw signal; W2S_PRO_NORM_RES_X: the residual
-   * branch is w_first_ds * x[2i]); x_raw fp32 [B, T_raw], w_first fp32 [16,3], w_first_ds fp32 [16]. */
+   * branch is w_first_ds * x[2i]); x_raw fp32 [B, T_raw] with T_raw a multiple of 4, w_first fp32 [16,3],
+   * w_first_ds fp32 [16]. */
   const float* x_raw;
   const float* w_first;
   const float* w_first_ds;
@@ -135,6 +136,9 @@ typedef struct w2s_conv_call {
 } w2s_conv_call;
 
 int w2s_conv1d_fwd(const w2s_conv_call* call, void* stream);
+/* Two calls of identical shape and configuration in ONE launch (w2s_encoder_fwd_pair's stream / Linear kernels).
+ * Fails, launching nothing, if the pair has no paired kernel. */
+int w2s_conv1d_fwd_pair(const w2s_conv_call* c0, const w2s_conv_call* c1, void* stream);  /* ABI v11 */
 /* ---------------------------------------------------------------------------------------------------------
  * Input staging (SURVEY 8f N1).  Replaces ParquetDataset._zscore_normalize (data/dataset.py:76-87) and the -inf fill
  * of missing signals (:170-173) for a batch of raw nights already copied to the device:

@@ -75,162 +75,6 @@ def test_first_conv(cuda_device, B, T):
     assert torch.allclose(s1[live][..., 1], (ref * ref).sum(1), rtol=1e-4, atol=1e-2)
 
 
-ENC_CASES = [
-    # cin, cout, stride, has_ds, L
-    (16, 16, 1, 0, 2500), (32, 32, 1, 0, 1100), (64, 64, 1, 0, 700), (128, 128, 1, 0, 300),
-    (16, 16, 2, 0, 4096), (32, 32, 2, 0, 1030), (64, 64, 2, 0, 512), (128, 128, 2, 0, 258),
-    (16, 16, 1, 1, 2048), (16, 32, 1, 1, 1000), (32, 32, 1, 1, 600), (32, 64, 1, 1, 512),
-    (64, 64, 1, 1, 256), (64, 128, 1, 1, 384), (128, 128, 1, 1, 130),
-]
-
-
-@pytest.fixture(params=[0, 1], ids=["stream", "tile"])
-def conv_impl(request):
-    """Run with the persistent streaming kernel (default) and with the tile-per-CTA kernel."""
-    lib = _lib.load()
-    lib.w2s_set_conv_impl(request.param)
-    yield request.param
-    lib.w2s_set_conv_impl(0)
-
-
-@pytest.mark.parametrize("cin,cout,stride,has_ds,L", ENC_CASES)
-def test_encoder_conv_layer(cuda_device, conv_impl, cin, cout, stride, has_ds, L):
-    """EPI_STATS conv kernels: prologue norm+GELU(+res), k3 conv (tcgen05), fp16 store, sums, fused 1x1."""
-    torch.manual_seed(cin * 1000 + cout + stride)
-    B = 2
-    dev = cuda_device
-    y = (torch.randn(B, L, cin, device=dev) * 1.5 + 0.3).half()
-    r = torch.randn(B, L, cin, device=dev).half() if has_ds else None
-    w = torch.randn(cout, cin, 3, device=dev) / (3 * cin) ** 0.5
-    wd = torch.randn(cout, cin, 1, device=dev) / cin ** 0.5 if has_ds else None
-    L_out = (L + 2 - 3) // stride + 1
-    out = torch.full((B, L_out, cout), float("nan"), dtype=torch.float16, device=dev)
-    out_ds = torch.full((B, L_out // 2, cout), float("nan"), dtype=torch.float16, device=dev) if has_ds else None
-    stats = torch.zeros(B, cout, 2, device=dev, dtype=torch.float64)
-    split = G.uses_split(cin, cout)
-    assert split == (1 if max(cin, cout) <= 16 else 0)
-    G.run_conv(cin=cin, cout=cout, taps=3, stride=stride, dilation=1, pad=1,
-               prologue=_lib.PRO_NORM_RES if has_ds else _lib.PRO_NORM, epilogue=_lib.EPI_STATS, has_ds=has_ds,
-               B=B, L_in=L, L_out=L_out, **{"in": y}, in_res=r, in_stats=G.sums(y), w=G.pack_conv(w, split=split),
-               w_ds=G.pack_conv(wd, split=split) if has_ds else None, out=out, out_ds=out_ds, out_stats=stats,
-               in_eps=1e-2)
-    stats = stats.float()
-    a = G.prologue_ref(y, r)
-    ref = G.conv_ref(a, w, stride=stride, split=split)
-    assert ref.shape == out.shape
-    assert not torch.isnan(out.float()).any()
-    # split layers: only the fp16 rounding of the stored output remains (2^-11 relative to each element)
-    assert rel_err(out, ref) < (1e-3 if split else 4e-3)
-    assert torch.allclose(stats[..., 0], ref.sum(1), rtol=2e-3, atol=0.05 * L ** 0.5)
-    assert torch.allclose(stats[..., 1], (ref * ref).sum(1), rtol=2e-3, atol=1e-2)
-    if has_ds:
-        refd = G.conv_ref(a, wd, stride=2, pad=0, split=split)
-        assert refd.shape == out_ds.shape
-        assert rel_err(out_ds, refd) < 4e-3
-
-
-@pytest.mark.parametrize("cin,cout,stride,has_ds,B,L", [
-    (16, 16, 1, 0, 5, 40000), (16, 16, 2, 0, 3, 70000), (16, 32, 1, 1, 4, 33000), (32, 32, 2, 0, 7, 9000),
-    (64, 64, 1, 0, 9, 5000), (128, 128, 2, 0, 6, 3000), (128, 128, 1, 1, 5, 2000), (64, 128, 1, 1, 20, 1000),
-])
-def test_encoder_conv_many_tiles_with_mask(cuda_device, conv_impl, cin, cout, stride, has_ds, B, L):
-    """Persistent CTAs walk tile ranges that cross sample boundaries; one sample in the middle is masked out."""
-    torch.manual_seed(B * L + cin)
-    dev = cuda_device
-    y = (torch.randn(B, L, cin, device=dev) + 0.2).half()
-    r = torch.randn(B, L, cin, device=dev).half() if has_ds else None
-    w = torch.randn(cout, cin, 3, device=dev) / (3 * cin) ** 0.5
-    wd = torch.randn(cout, cin, 1, device=dev) / cin ** 0.5 if has_ds else None
-    L_out = (L - 1) // stride + 1
-    out = torch.zeros(B, L_out, cout, dtype=torch.float16, device=dev)
-    out_ds = torch.zeros(B, L_out // 2, cout, dtype=torch.float16, device=dev) if has_ds else None
-    stats = torch.zeros(B, cout, 2, device=dev, dtype=torch.float64)
-    mask = torch.zeros(B, dtype=torch.uint8, device=dev)
-    mask[B // 2] = 1
-    split = G.uses_split(cin, cout)
-    G.run_conv(cin=cin, cout=cout, taps=3, stride=stride, dilation=1, pad=1,
-               prologue=_lib.PRO_NORM_RES if has_ds else _lib.PRO_NORM, epilogue=_lib.EPI_STATS, has_ds=has_ds,
-               B=B, L_in=L, L_out=L_out, **{"in": y}, in_res=r, in_stats=G.sums(y), w=G.pack_conv(w, split=split),
-               w_ds=G.pack_conv(wd, split=split) if has_ds else None, out=out, out_ds=out_ds, out_stats=stats,
-               row_mask=mask, in_eps=1e-2)
-    live = [b for b in range(B) if b != B // 2]
-    a = G.prologue_ref(y, r)
-    ref = G.conv_ref(a, w, stride=stride, split=split)
-    assert out[B // 2].abs().max().item() == 0 and stats[B // 2].abs().max().item() == 0
-    assert rel_err(out[live], ref[live]) < (1e-3 if split else 4e-3)
-    st = stats.float()
-    assert torch.allclose(st[live][..., 0], ref[live].sum(1), rtol=2e-3, atol=0.05 * L ** 0.5)
-    assert torch.allclose(st[live][..., 1], (ref[live] * ref[live]).sum(1), rtol=2e-3, atol=1e-2)
-    if has_ds:
-        refd = G.conv_ref(a, wd, stride=2, pad=0, split=split)
-        assert out_ds[B // 2].abs().max().item() == 0
-        assert rel_err(out_ds[live], refd[live]) < (1e-3 if split else 4e-3)
-
-
-@pytest.mark.parametrize("cin,cout,stride,has_ds,in_wide,out_wide,block", [
-    (16, 16, 1, 0, 1, 1, 1), (16, 16, 2, 0, 1, 1, 1), (16, 32, 1, 1, 1, 0, 2), (16, 32, 1, 1, 1, 1, 2), (32, 32, 1, 0, 1, 1, 2), (32, 32, 2, 0, 1, 1, 3),
-    (32, 32, 1, 1, 1, 1, 3), (32, 64, 1, 1, 1, 0, 4), (32, 64, 1, 1, 1, 1, 4), (64, 64, 1, 0, 1, 1, 4), (64, 64, 2, 0, 1, 1, 5),
-    (64, 64, 1, 1, 1, 1, 5), (64, 128, 1, 1, 1, 0, 6)])
-def test_encoder_conv_wide_storage(cuda_device, cin, cout, stride, has_ds, in_wide, out_wide, block):
-    """Wide-storage variants of the streaming kernels (fp32 input / output tensors) incl. the split-operand 64-channel
-    kernels of deep encoders (wide_blocks = 6); several tiles per sample, one masked sample."""
-    lib = _lib.load()
-    torch.manual_seed(cin * 100 + cout + stride + block)
-    dev, B, L = cuda_device, 3, 3000
-    wide_blocks = (6 if cout == 64 else 4) if out_wide else (2 if cout == 32 else 4)
-    split = lib.w2s_encoder_conv_split(wide_blocks, block, cin, cout)
-    assert split == (1 if (max(cin, cout) <= 16 or (out_wide and max(cin, cout) <= 64)) else 0)
-    y = torch.randn(B, L, cin, device=dev) * 1.5 + 0.3
-    r = torch.randn(B, L, cin, device=dev) if has_ds else None
-    w = torch.randn(cout, cin, 3, device=dev) / (3 * cin) ** 0.5
-    wd = torch.randn(cout, cin, 1, device=dev) / cin ** 0.5 if has_ds else None
-    L_out = (L - 1) // stride + 1
-    odt = torch.float32 if out_wide else torch.float16
-    out = torch.zeros(B, L_out, cout, dtype=odt, device=dev)
-    out_ds = torch.zeros(B, L_out // 2, cout, dtype=odt, device=dev) if has_ds else None
-    stats = torch.zeros(B, cout, 2, device=dev, dtype=torch.float64)
-    mask = torch.tensor([0, 1, 0], dtype=torch.uint8, device=dev)
-    yd = y.double()
-    in_stats = torch.stack([yd.sum(1), (yd * yd).sum(1)], dim=-1).contiguous()
-    G.run_conv(cin=cin, cout=cout, taps=3, stride=stride, dilation=1, pad=1,
-               prologue=_lib.PRO_NORM_RES if has_ds else _lib.PRO_NORM, epilogue=_lib.EPI_STATS, has_ds=has_ds,
-               B=B, L_in=L, L_out=L_out, **{"in": y}, in_res=r, in_stats=in_stats, w=G.pack_conv(w, split=split),
-               w_ds=G.pack_conv(wd, split=split) if has_ds else None, out=out, out_ds=out_ds, out_stats=stats,
-               row_mask=mask, in_eps=1e-2, in_wide=in_wide, out_wide=out_wide,
-               force_split=1 if (split and not G.uses_split(cin, cout)) else 0)
-    mu = y.mean(1, keepdim=True)
-    var = (y * y).mean(1, keepdim=True) - mu * mu
-    a = G.gelu((y - mu) / torch.sqrt(var.clamp_min(0) + 1e-2))
-    if has_ds:
-        a = G.gelu(a + r)
-    ref = G.conv_ref(a, w, stride=stride, split=split)
-    live = [0, 2]
-    assert out[1].abs().max().item() == 0 and stats[1].abs().max().item() == 0
-    assert rel_err(out[live], ref[live]) < (1e-3 if split else 4e-3)
-    st = stats.float()
-    assert torch.allclose(st[live][..., 0], ref[live].sum(1), rtol=2e-3, atol=0.05 * L ** 0.5)
-    assert torch.allclose(st[live][..., 1], (ref[live] * ref[live]).sum(1), rtol=2e-3, atol=1e-2)
-    if has_ds:
-        refd = G.conv_ref(a, wd, stride=2, pad=0, split=split)
-        assert out_ds[1].abs().max().item() == 0
-        assert rel_err(out_ds[live], refd[live]) < (1e-3 if split else 4e-3)
-
-
-def test_encoder_conv_row_mask_skips_sample(cuda_device):
-    dev = cuda_device
-    B, L, c = 3, 1024, 16
-    y = torch.randn(B, L, c, device=dev).half()
-    w = torch.randn(c, c, 3, device=dev) / 7
-    out = torch.zeros(B, L, c, dtype=torch.float16, device=dev)
-    stats = torch.zeros(B, c, 2, device=dev, dtype=torch.float64)
-    mask = torch.tensor([0, 1, 0], dtype=torch.uint8, device=dev)
-    G.run_conv(cin=c, cout=c, taps=3, stride=1, dilation=1, pad=1, prologue=_lib.PRO_NORM, epilogue=_lib.EPI_STATS,
-               has_ds=0, B=B, L_in=L, L_out=L, **{"in": y}, in_stats=G.sums(y), w=G.pack_conv(w, split=1), out=out,
-               out_stats=stats, row_mask=mask, in_eps=1e-2)
-    assert out[1].abs().max().item() == 0 and stats[1].abs().max().item() == 0
-    assert out[0].abs().max().item() > 0 and out[2].abs().max().item() > 0
-
-
 @pytest.mark.parametrize("cin,S", [(64, 37), (128, 130), (128, 16)])
 def test_encoder_linear(cuda_device, cin, S):
     """Linear(4C -> 128) + bias + GELU as a 4-tap stride-4 conv (reference models/wav2sleep.py:261-265)."""

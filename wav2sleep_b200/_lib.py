@@ -27,7 +27,7 @@ STREAM_MAX_LAYERS = 32
 STREAM_MAX_DILATIONS = 16
 STREAM_MAX_KERNEL = 16
 STREAM_MAX_FEATURES = 256
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 PRO_NONE, PRO_NORM, PRO_NORM_RES, PRO_FIR, PRO_NORM_RES_X, PRO_DNORM = 0, 1, 2, 3, 4, 5
 EPI_STATS, EPI_BIAS_GELU, EPI_LN_GELU, EPI_LN_GELU_RES, EPI_PLAIN, EPI_ACT_BWD = 0, 1, 2, 3, 4, 5
@@ -146,6 +146,7 @@ SYMBOLS = {
     "w2s_pack_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "w2s_pack_linear_frag": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "w2s_conv1d_fwd": (C.c_int, [C.POINTER(ConvCall), C.c_void_p]),
+    "w2s_conv1d_fwd_pair": (C.c_int, [C.POINTER(ConvCall), C.POINTER(ConvCall), C.c_void_p]),
     "w2s_set_conv_impl": (C.c_int, [C.c_int]),
     "w2s_encoder_workspace_bytes": (C.c_size_t, [C.POINTER(EncoderDesc), C.c_int, C.c_int64, C.c_int]),
     "w2s_encoder_layout": (C.c_int, [C.POINTER(EncoderDesc), C.c_int, C.c_int64, C.POINTER(C.c_int64)]),

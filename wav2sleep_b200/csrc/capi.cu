@@ -289,6 +289,14 @@ int conv_dispatch(const w2s_conv_call& c, cudaStream_t st, const w2s_conv_call* 
     if (!c.in_res || !c.in_stats || !c.dn_sums || !c.dn_out) return fail("conv1d: W2S_PRO_DNORM needs in_res (y), in_stats, dn_sums, dn_out");
     if (c.dn_upsample && (c.L_in & 1)) return fail("conv1d: W2S_PRO_DNORM upsample needs an even L_in");
   }
+  // the block-0 fusion kernels stage each night's raw-signal window with 16-byte bulk copies from x_raw + b * T_raw
+  // (both calls of a pair: conv_calls_pairable compares T_raw but not the pointers)
+  for (const w2s_conv_call* q : {&c, c2}) {
+    if (q == nullptr || (q->prologue != W2S_PRO_FIR && q->prologue != W2S_PRO_NORM_RES_X)) continue;
+    if (q->x_raw == nullptr || q->T_raw <= 0 || (q->T_raw & 3))
+      return fail("conv1d: W2S_PRO_FIR / W2S_PRO_NORM_RES_X need x_raw and a T_raw that is a multiple of 4 (got x_raw=%p "
+                  "T_raw=%d, L_in=%d)", (const void*)q->x_raw, q->T_raw, q->L_in);
+  }
   if (c.epilogue == W2S_EPI_ACT_BWD) {
     if (!c.act_y || !c.act_stats || !c.out_stats || (c.act_r && !c.act_dr))
       return fail("conv1d: W2S_EPI_ACT_BWD needs act_y, act_stats, out_stats (and act_dr with act_r)");
@@ -530,7 +538,7 @@ int check_encoder_desc(const w2s_encoder_desc* d) {
 
 extern "C" {
 
-int w2s_abi_version(void) { return 10; }
+int w2s_abi_version(void) { return 11; }
 const char* w2s_last_error(void) { return g_err.c_str(); }
 
 int w2s_conv_uses_split(int cin, int cout) { return (cin <= 16 && cout <= 16) ? 1 : 0; }
@@ -610,6 +618,16 @@ int w2s_debug_timestamps(uint64_t* out16, uint64_t* cta1024) {
 int w2s_conv1d_fwd(const w2s_conv_call* call, void* stream) {
   if (call == nullptr) return fail("conv1d: null call");
   return conv_dispatch(*call, (cudaStream_t)stream);
+}
+
+int w2s_conv1d_fwd_pair(const w2s_conv_call* c0, const w2s_conv_call* c1, void* stream) {
+  if (c0 == nullptr || c1 == nullptr) return fail("conv1d pair: null call");
+  const int rc = conv_dispatch(*c0, (cudaStream_t)stream, c1);
+  if (rc == kNotPaired)
+    return fail("conv1d pair: no paired kernel for c%d->%d k%d s%d pro%d epi%d ds%d in_wide=%d out_wide=%d split=%d B=%d "
+                "L_in=%d (or the two calls differ in shape or configuration)", c0->cin, c0->cout, c0->taps, c0->stride,
+                c0->prologue, c0->epilogue, c0->has_ds, c0->in_wide, c0->out_wide, c0->force_split, c0->B, c0->L_in);
+  return rc;
 }
 
 size_t w2s_encoder_workspace_bytes(const w2s_encoder_desc* d, int B, int64_t T, int keep) {

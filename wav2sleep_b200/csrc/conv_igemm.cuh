@@ -495,7 +495,7 @@ W2S_DEVINL void conv_igemm_body(const ConvArgs& p, const int b) {
         float v[16];
         tmem_ld16(tmem_base + t_lane + 128 + j * COUT + cg * 16, v);
         const int o = o0 + j * 128 + quad * 32 + lane;
-        if (o < p.L_out && (o & 1) == 0) {
+        if (o < (p.L_out & ~1) && (o & 1) == 0) {  // out_ds has L_out / 2 rows (rounded down)
           store_h16(dsb + (size_t)(o >> 1) * COUT + cg * 16, v);
         }
       }

@@ -564,7 +564,7 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
                 const int r = 2 * (it * RPI + crow);
                 const int o = obase + r;
                 const uint4 val = lds128(stg + r * SEGB + ((cchunk ^ swz(r)) * 16));
-                if (o < p.L_out)
+                if (o < (p.L_out & ~1))  // out_ds has L_out / 2 rows (rounded down)
                   *reinterpret_cast<uint4*>(dsb + ((size_t)(o >> 1) * COUT + sg * SEG + cchunk * 8) * 2) = val;
               }
               __syncwarp();
@@ -676,7 +676,7 @@ conv_stream_kernel(const ConvArgs pa, const ConvGroup2 pb, int tiles_per_sample,
             float v[16];
             if (EPI_SPLIT > 1 && ((cg * MT + j) % EPI_SPLIT) != epi_half) continue;
             tmem_ld16(d_base + (MT + j) * COUT + cg * 16, v);
-            if (o < p.L_out && (o & 1) == 0) {
+            if (o < (p.L_out & ~1) && (o & 1) == 0) {  // out_ds has L_out / 2 rows (rounded down)
               store16<WOUT>(dsb, (size_t)(o >> 1) * COUT + cg * 16, v);
             }
           }
